@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - S-CGIB pre-training throughput (graphs/s) on N B200s + roofline + CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--k 1] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--k 1] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): pre-training graphs/s, PCQM4Mv2-shape synthetic molecules, GIN-4x64 (models.py:57-58),
 k_transition=1, fp32.  A "step" is one full pre-training step on one mini-batch per GPU:
@@ -12,6 +12,9 @@ on-GPU k-hop ego-net extraction + noise draw + forward + backward + gradient all
           D2H of the losses inside the timed region.
   --impl reference : the reference's CPU path (oracle restatement, loop-for-loop; DGL cannot be installed
           here) on the host cores, B=128 mini-batches (the reference's default --batch_size).
+  --dump-outputs DIR : after the timed steps, what the timed path computed in its last step (losses or scores, parameters
+          after the optimiser step, gradients, BatchNorm running statistics) as DIR/<name>.npy in float32.  Inputs, weights
+          and noise are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -40,6 +43,14 @@ def peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy (float32) per device tensor."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 class NvmlClockSampler:
@@ -291,7 +302,7 @@ def run_finetune(args, emit):
     nb = 3
     host = [synth_batch(50 + i, B, args.shape).pin_memory() for i in range(nb)]
     resident = [h.to(dev) for h in host]
-    targets = (torch.rand(B, 10, device=dev) < 0.1).float()
+    targets = (torch.rand(B, 10, generator=torch.Generator().manual_seed(2)) < 0.1).float().to(dev)
     state = {"n": 0}
 
     def run_steps(src, steps, read):
@@ -315,7 +326,7 @@ def run_finetune(args, emit):
                 handle = eng.prefetch_batch(src[(i + 1) % nb], args.k)
             if read:
                 state["scores"] = scores.cpu()
-        state["b"] = b
+        state["b"], state["last_scores"] = b, scores
 
     def timed(src, steps, read):
         torch.cuda.synchronize()
@@ -329,6 +340,9 @@ def run_finetune(args, emit):
     sampler.start()
     ms = timed(resident, args.steps, False)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"scores": state["last_scores"], "params": eng.params, "grads": eng.grads,
+                                         "head_params": head.params, "head_grads": head.grads})
     run_steps(host, 3, True)
     ms_e2e = timed(host, args.steps, True)
     prof = {}
@@ -420,6 +434,7 @@ def run_encoder_variant(args, emit):
             opt.step()
             if read:
                 state["loss"] = loss.detach().item()
+        state["last_loss"] = loss
         state["shape"] = (bg.num_nodes(), bg.num_edges(), int(ego.sub_indptr.numel() - 1), int(ego.sub_indices.numel()))
 
     def timed(src, steps, read):
@@ -434,6 +449,13 @@ def run_encoder_variant(args, emit):
     sampler.start()
     ms = timed(resident, args.steps, False)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        flat = lambda ts: torch.cat([t.detach().float().reshape(-1) for t in ts])
+        dump_outputs(args.dump_outputs, {
+            "loss": state["last_loss"].reshape(1),
+            "params": flat(dm.parameters()),
+            "grads": flat(p.grad if p.grad is not None else torch.zeros_like(p) for p in dm.parameters()),
+            "bn_running": flat(v for n, v in dm.state_dict().items() if n.endswith(("running_mean", "running_var")))})
     run_steps(host, 3, True)
     ms_e2e = timed(host, args.steps, True)
     N, E, Ns, Es = state["shape"]
@@ -474,7 +496,11 @@ def main():
                     help="fp32 = the headline (reference precision); bf16 = bf16 activations + single-pass bf16 tensor-core MLPs in the GIN encoders")
     ap.add_argument("--encoder", default="GIN", choices=["GIN", "GraphSAGE", "GCN"],
                     help="GIN = the headline (fused tensor-core engine); GraphSAGE / GCN = the operator-composed variants (1 GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     # stdout carries exactly ONE JSON line: anything libraries print (e.g. the NCCL version banner) goes to stderr
     real_stdout = os.dup(1)
     os.dup2(2, 1)
@@ -611,6 +637,9 @@ def main():
         sampler.start()
     ms = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:          # the e2e / dropin / profiling passes below keep training this engine
+        dump_outputs(args.dump_outputs, {"losses": eng.losses, "params": eng.params, "grads": eng.grads,
+                                         "bn_running": eng.bn_running})
     step_e2e(3)
     ms_e2e = timed(step_e2e, args.steps)
     step_ids(3)
