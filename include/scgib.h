@@ -314,6 +314,16 @@ SCGIB_API int scgib_recon_adj_h_f32(const float* Z, const int32_t* indptr, const
                                     void* stream);
 SCGIB_API int scgib_contrastive_h_f32(const float* core, const float* readout, int32_t B, int32_t hidden, float scale, float* loss,
                                       float* g_core, float* g_readout, void* workspace, size_t workspace_bytes, void* stream);
+/* loss_recon of --recons_type logM (models.py:770-782 with the k-step log transition matrices of util.py:60-91):
+ *   loss = (1/k) sum_g sum_{i=1..k} || Z_g Z_g^T - logM_{g,i} ||_F^2 / n_g^2,   Z [N][hidden], hidden 64 or 128,
+ * computed per graph (graph_ptr [B+1]) on the symmetric CSR without any dense n x n matrix.  gZ (optional) = scale * d loss / d Z.
+ * status = device int32[1]: set to 0, then to 1 when a k-hop ball exceeds SCGIB_EGO_CAP nodes (its terms are then dropped).
+ * workspace >= scgib_recon_logm_workspace_bytes(B, N, k), 256-byte aligned; Z / gZ 16-byte aligned.
+ * Codes: hidden not 64 / 128 -> SCGIB_E_SHAPE; k outside [1, 8], B < 1 or N < 2 -> SCGIB_E_RANGE. */
+SCGIB_API size_t scgib_recon_logm_workspace_bytes(int32_t B, int32_t N, int32_t k);
+SCGIB_API int scgib_recon_logm_h_f32(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices,
+                                     int32_t B, int32_t N, int32_t hidden, int32_t k, float scale, float* loss, float* gZ,
+                                     int32_t* status, void* workspace, size_t workspace_bytes, void* stream);
 
 /* out[s] = sum_{rows in segment s} f(in[row])  (dgl.sum_nodes, models.py:716,725,733,684);
  * f = relu(BN(.)) when bn = {mean,rstd,gamma,beta} is given, identity otherwise. */
@@ -343,6 +353,14 @@ SCGIB_API int scgib_core_gate_fwd_f32(const float* Hfeat, const int32_t* graph_p
                                       const float* wc2, const float* bc2, const float* gate_u, const float* feat_u,
                                       float* noisy, float* lam, float* graph_readout, float* core_readout, float* kl,
                                       void* workspace, size_t workspace_bytes, void* stream);
+/* model.eval() instance of scgib_core_gate_fwd_f32: compressor.1 normalises q with its running statistics
+ * running = {mean[H], var[H]} (nn.BatchNorm1d in eval mode) instead of the per-graph batch statistics, and nothing is kept
+ * for a backward or for scgib_core_gate_ema_f32 (forward only).  Same codes as scgib_core_gate_fwd_f32. */
+SCGIB_API int scgib_core_gate_eval_fwd_f32(const float* Hfeat, const int32_t* graph_ptr, int32_t B, int32_t N, int32_t hidden,
+                                           const float* Wc1, const float* bc1, const float* gamma_c, const float* beta_c,
+                                           const float* wc2, const float* bc2, const float* running, const float* gate_u,
+                                           const float* feat_u, float* noisy, float* lam, float* graph_readout,
+                                           float* core_readout, float* kl, void* workspace, size_t workspace_bytes, void* stream);
 /* running = {mean[H], var[H]} of compressor.1 after the B per-graph BatchNorm calls of the forward that filled `workspace`. */
 SCGIB_API int scgib_core_gate_ema_f32(int32_t B, int32_t N, int32_t hidden, float* running, void* workspace,
                                       size_t workspace_bytes, void* stream);

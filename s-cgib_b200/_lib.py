@@ -94,11 +94,16 @@ _SIGNATURES = {
                                       c_size_t, c_void_p]),
     "scgib_contrastive_h_f32": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                         c_void_p]),
+    "scgib_recon_logm_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "scgib_recon_logm_h_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_float, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "scgib_segment_sum_f32": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
     "scgib_core_gate_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
     "scgib_core_gate_fwd_f32": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32] + [c_void_p] * 13 + [c_void_p, c_size_t, c_void_p]),
     "scgib_core_gate_bwd_f32": (c_int, [c_void_p, c_int32, c_int32, c_int32] + [c_void_p] * 8 + [c_float] + [c_void_p] * 7 +
                                 [c_void_p, c_size_t, c_void_p]),
+    "scgib_core_gate_eval_fwd_f32": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32] + [c_void_p] * 14 +
+                                     [c_void_p, c_size_t, c_void_p]),
     "scgib_core_gate_ema_f32": (c_int, [c_int32, c_int32, c_int32, c_void_p, c_void_p, c_size_t, c_void_p]),
     "scgib_core_cand_attn_fwd_f32": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "scgib_core_cand_attn_bwd_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p,

@@ -432,7 +432,7 @@ static int forward_impl(const ScgibDims* d, const float* params, float* bn_runni
   const int logm = b->recon_logm_steps;
   if (!features_only && logm > 0) {
     PROF("logm_fwd", launch_logm_fwd(w.Z, b->graph_ptr, b->indptr, b->indices, b->B, b->N, logm, w.logm_walks, w.logm_gram,
-                                     w.logm_pair, w.logm_loss, (int32_t*)(w.counters + 32), s));
+                                     w.logm_pair, w.logm_loss, (int32_t*)(w.counters + 32), HID, s));
   } else if (!features_only) {
     const int grid = recon_fwd_grid();
     ReconFwdArgs a{w.Z, b->indptr, b->indices, b->N, w.rpart};
@@ -528,7 +528,7 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
     }
     if (logm) {
       PROF("logm_bwd", launch_logm_bwd(w.Z, b->graph_ptr, b->indptr, b->indices, b->B, b->N, b->recon_logm_steps, w.logm_walks,
-                                       s_rec, w.gZ, (int32_t*)(w.counters + 32), s));
+                                       s_rec, w.gZ, (int32_t*)(w.counters + 32), HID, s));
     } else if (!con_tc) {
       PROF("recon_bwd", launch_recon_bwd(ra, HID, s));
     }
@@ -1055,6 +1055,42 @@ extern "C" SCGIB_API int scgib_contrastive_h_f32(const float* core, const float*
   return contrastive_impl(core, readout, B, hidden, scale, loss, g_core, g_readout, workspace, workspace_bytes, stream_);
 }
 
+// ---- --recons_type logM as an operator (logm_kernels.cu): hidden 64 or 128
+namespace scgib {
+struct LogmOpWs { float *walks, *gram, *pair, *loss; size_t bytes; };
+static LogmOpWs logm_op_carve(int B, int N, int k, void* base) {
+  LogmOpWs w;
+  char* p = (char*)base;
+  size_t o = 0;
+  auto take = [&](size_t nfloats) { float* r = (float*)(p + o); o += al(nfloats * sizeof(float)); return r; };
+  w.walks = take((size_t)k * N); w.gram = take(B); w.pair = take(N); w.loss = take(4);
+  w.bytes = o;
+  return w;
+}
+}  // namespace scgib
+
+extern "C" SCGIB_API size_t scgib_recon_logm_workspace_bytes(int32_t B, int32_t N, int32_t k) {
+  if (B < 1 || N < 2 || k < 1 || k > logm_max_steps()) return 0;
+  return logm_op_carve(B, N, k, nullptr).bytes;
+}
+
+extern "C" SCGIB_API int scgib_recon_logm_h_f32(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices,
+                                                int32_t B, int32_t N, int32_t hidden, int32_t k, float scale, float* loss, float* gZ,
+                                                int32_t* status, void* workspace, size_t workspace_bytes, void* stream_) {
+  if (!Z || !graph_ptr || !indptr || !indices || !loss || !status || !workspace) return SCGIB_E_NULL;
+  if (hidden != 64 && hidden != 128) return SCGIB_E_SHAPE;
+  if (k < 1 || k > logm_max_steps() || B < 1 || N < 2) return SCGIB_E_RANGE;
+  if (((uintptr_t)workspace & 255u) || ((uintptr_t)Z & 15u) || ((uintptr_t)gZ & 15u)) return SCGIB_E_ALIGN;
+  const LogmOpWs w = logm_op_carve(B, N, k, workspace);
+  if (workspace_bytes < w.bytes) return SCGIB_E_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream_;
+  cudaMemsetAsync(status, 0, sizeof(int32_t), s);
+  launch_logm_fwd(Z, graph_ptr, indptr, indices, B, N, k, w.walks, w.gram, w.pair, w.loss, status, hidden, s);
+  cudaMemcpyAsync(loss, w.loss, sizeof(float), cudaMemcpyDeviceToDevice, s);
+  if (gZ) launch_logm_bwd(Z, graph_ptr, indptr, indices, B, N, k, w.walks, scale, gZ, status, hidden, s);
+  return (int)cudaGetLastError();
+}
+
 extern "C" SCGIB_API int scgib_segment_sum_f32(const float* in, const int32_t* seg_ptr, int32_t S, const float* bn, float* out, void* stream) {
   if (!in || !seg_ptr || !out) return SCGIB_E_NULL;
   if (S < 1) return SCGIB_E_RANGE;
@@ -1095,17 +1131,21 @@ extern "C" SCGIB_API size_t scgib_core_gate_workspace_bytes(int32_t hidden, int3
   return gate_op_carve(hidden, B, N, nullptr).bytes;
 }
 
-extern "C" SCGIB_API int scgib_core_gate_fwd_f32(const float* Hfeat, const int32_t* graph_ptr, int32_t B, int32_t N, int32_t hidden,
-                                       const float* Wc1, const float* bc1, const float* gamma_c, const float* beta_c,
-                                       const float* wc2, const float* bc2, const float* gate_u, const float* feat_u, float* noisy,
-                                       float* lam, float* graph_readout, float* core_readout, float* kl, void* workspace,
-                                       size_t workspace_bytes, void* stream_) {
+// running == nullptr: training-mode BatchNorm (per-graph batch statistics, kept in cstat for scgib_core_gate_ema_f32);
+// otherwise model.eval(): q is normalised with running = {mean, var} and cstat is not written
+static int core_gate_fwd_impl(const float* Hfeat, const int32_t* graph_ptr, int32_t B, int32_t N, int32_t hidden, const float* Wc1,
+                              const float* bc1, const float* gamma_c, const float* beta_c, const float* wc2, const float* bc2,
+                              const float* running, const float* gate_u, const float* feat_u, float* noisy, float* lam,
+                              float* graph_readout, float* core_readout, float* kl, void* workspace, size_t workspace_bytes,
+                              void* stream_) {
   if (!Hfeat || !graph_ptr || !Wc1 || !bc1 || !gamma_c || !beta_c || !wc2 || !bc2 || !gate_u || !feat_u || !noisy || !graph_readout ||
       !core_readout || !workspace)
     return SCGIB_E_NULL;
   if (!hidden_ok(hidden)) return SCGIB_E_SHAPE;
   if (B < 1 || N < 2) return SCGIB_E_RANGE;
-  if (((uintptr_t)workspace & 255u) || ((uintptr_t)Hfeat & 15u) || ((uintptr_t)feat_u & 15u) || ((uintptr_t)noisy & 15u)) return SCGIB_E_ALIGN;
+  if (((uintptr_t)workspace & 255u) || ((uintptr_t)Hfeat & 15u) || ((uintptr_t)feat_u & 15u) || ((uintptr_t)noisy & 15u) ||
+      ((uintptr_t)running & 15u))
+    return SCGIB_E_ALIGN;
   const GateOpWs w = gate_op_carve(hidden, B, N, workspace);
   if (workspace_bytes < w.bytes) return SCGIB_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream_;
@@ -1119,11 +1159,33 @@ extern "C" SCGIB_API int scgib_core_gate_fwd_f32(const float* Hfeat, const int32
   a.graph_ptr = graph_ptr; a.B = B; a.N = N; a.H = w.Hc; a.q = w.q;
   a.gamma_c = gamma_c; a.beta_c = beta_c; a.wc2 = wc2; a.bc2 = bc2; a.gate_u = gate_u; a.feat_u = feat_u; a.logit = w.logit0;
   a.noisy = noisy; a.lam = w.lam; a.alpha = w.alpha0; a.readout = graph_readout; a.core = core_readout; a.gstat = w.gstat;
-  a.eval_running = nullptr; a.cstat = w.cstat; a.kl = w.kl;      // per-graph batch statistics of q: scgib_core_gate_ema_f32
+  a.eval_running = running;
+  a.cstat = running ? nullptr : w.cstat;      // per-graph batch statistics of q: scgib_core_gate_ema_f32
+  a.kl = w.kl;
   launch_graph_gate_fwd(a, H, s);
   if (lam) cudaMemcpyAsync(lam, w.lam, (size_t)N * sizeof(float), cudaMemcpyDeviceToDevice, s);
   if (kl) cudaMemcpyAsync(kl, w.kl, sizeof(float), cudaMemcpyDeviceToDevice, s);
   return (int)cudaGetLastError();
+}
+
+extern "C" SCGIB_API int scgib_core_gate_fwd_f32(const float* Hfeat, const int32_t* graph_ptr, int32_t B, int32_t N, int32_t hidden,
+                                       const float* Wc1, const float* bc1, const float* gamma_c, const float* beta_c,
+                                       const float* wc2, const float* bc2, const float* gate_u, const float* feat_u, float* noisy,
+                                       float* lam, float* graph_readout, float* core_readout, float* kl, void* workspace,
+                                       size_t workspace_bytes, void* stream_) {
+  return core_gate_fwd_impl(Hfeat, graph_ptr, B, N, hidden, Wc1, bc1, gamma_c, beta_c, wc2, bc2, nullptr, gate_u, feat_u, noisy, lam,
+                            graph_readout, core_readout, kl, workspace, workspace_bytes, stream_);
+}
+
+extern "C" SCGIB_API int scgib_core_gate_eval_fwd_f32(const float* Hfeat, const int32_t* graph_ptr, int32_t B, int32_t N,
+                                                      int32_t hidden, const float* Wc1, const float* bc1, const float* gamma_c,
+                                                      const float* beta_c, const float* wc2, const float* bc2, const float* running,
+                                                      const float* gate_u, const float* feat_u, float* noisy, float* lam,
+                                                      float* graph_readout, float* core_readout, float* kl, void* workspace,
+                                                      size_t workspace_bytes, void* stream_) {
+  if (!running) return SCGIB_E_NULL;
+  return core_gate_fwd_impl(Hfeat, graph_ptr, B, N, hidden, Wc1, bc1, gamma_c, beta_c, wc2, bc2, running, gate_u, feat_u, noisy, lam,
+                            graph_readout, core_readout, kl, workspace, workspace_bytes, stream_);
 }
 
 // compressor.1's running statistics after the B per-graph BatchNorm calls of the forward that filled `workspace`

@@ -364,10 +364,11 @@ int finetune_max_classes();
 // ---------------------------------------------------------------- logm_kernels.cu
 // `--recons_type logM` (models.py:770-782 with util.py:60-91): per-graph Gram term + sparse k-hop pair term, no dense n x n.
 // walks [k][N], gram [B], pair [N] are workspace; loss_out[0] = the loss; bwd OVERWRITES gZ with scale * d loss / d Z.
+// Z is [N][hidden], hidden 64 or 128.
 int logm_max_steps();
 void launch_logm_fwd(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
-                     int k, float* walks, float* gram, float* pair, float* loss_out, int32_t* status, cudaStream_t s);
+                     int k, float* walks, float* gram, float* pair, float* loss_out, int32_t* status, int hidden, cudaStream_t s);
 void launch_logm_bwd(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
-                     int k, const float* walks, float scale, float* gZ, int32_t* status, cudaStream_t s);
+                     int k, const float* walks, float scale, float* gZ, int32_t* status, int hidden, cudaStream_t s);
 
 }  // namespace scgib

@@ -6,7 +6,7 @@
 //   L_{g,i}[r][c] = max( log( (A_g^i)[r][c] / colsum_c(A_g^i) ) - log(1/n_g), 0 )       (nan / -inf -> 0)
 //
 // || Z Z^T - L ||^2 = || Z^T Z ||_F^2 - 2 sum_{rc} (z_r . z_c) L_rc + sum_{rc} L_rc^2, and L_{g,i} is SPARSE: (A^i)[r][c] is the
-// number of i-step walks r -> c, non-zero only inside the i-hop ball of r.  So the loss is a per-graph 64 x 64 Gram term
+// number of i-step walks r -> c, non-zero only inside the i-hop ball of r.  So the loss is a per-graph H x H Gram term (H = 64 or 128)
 // plus a sum over the (seed, ball node) pairs of the k-hop ego-nets - the same warp-per-seed machinery as the ego-net
 // extraction, with a walk-count dynamic programme on the ball.  A is symmetric, so colsum_c(A^i) = rowsum_c(A^i) = the
 // number of i-step walks starting at c (`walks`), and L_i[c][r] follows from the same count as L_i[r][c].
@@ -42,38 +42,50 @@ logm_walks_kernel(const int32_t* __restrict__ graph_ptr, const int32_t* __restri
   }
 }
 
-// per graph: G = Z_g^T Z_g in shared memory (thread (ty, tx) owns a 4 x 4 block)
+// per graph: G = Z_g^T Z_g in shared memory (thread (ty, tx) owns an H/16 x H/16 block)
+template <int H>
 __device__ __forceinline__ void graph_gram(const float* __restrict__ Z, int v0, int v1, float* sG) {
+  constexpr int TM = H / 16;
   const int ty = threadIdx.x >> 4, tx = threadIdx.x & 15;
-  float acc[4][4];
+  float acc[TM][TM];
 #pragma unroll
-  for (int i = 0; i < 4; ++i)
+  for (int i = 0; i < TM; ++i)
 #pragma unroll
-    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+    for (int j = 0; j < TM; ++j) acc[i][j] = 0.f;
   for (int r = v0; r < v1; ++r) {
-    const float4 a = ldg4(Z + (size_t)r * HID + ty * 4), b = ldg4(Z + (size_t)r * HID + tx * 4);
-    const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {b.x, b.y, b.z, b.w};
+    float av[TM], bv[TM];
 #pragma unroll
-    for (int i = 0; i < 4; ++i)
+    for (int q = 0; q < TM; q += 4) {
+      const float4 a = ldg4(Z + (size_t)r * H + ty * TM + q), b = ldg4(Z + (size_t)r * H + tx * TM + q);
+      av[q] = a.x; av[q + 1] = a.y; av[q + 2] = a.z; av[q + 3] = a.w;
+      bv[q] = b.x; bv[q + 1] = b.y; bv[q + 2] = b.z; bv[q + 3] = b.w;
+    }
 #pragma unroll
-      for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
+    for (int i = 0; i < TM; ++i)
+#pragma unroll
+      for (int j = 0; j < TM; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
   }
 #pragma unroll
-  for (int i = 0; i < 4; ++i)
+  for (int i = 0; i < TM; ++i)
 #pragma unroll
-    for (int j = 0; j < 4; ++j) sG[(ty * 4 + i) * HID + tx * 4 + j] = acc[i][j];
+    for (int j = 0; j < TM; ++j) sG[(ty * TM + i) * H + tx * TM + j] = acc[i][j];
 }
 
+// the H x H Gram matrix lives in dynamic shared memory: 16 KB at H = 64, 64 KB (opt-in) at H = 128
+template <int H>
+constexpr int gram_smem_bytes() { return H * H * (int)sizeof(float); }
+
+template <int H>
 __global__ void __launch_bounds__(kThreads)
 logm_gram_fwd_kernel(const float* __restrict__ Z, const int32_t* __restrict__ graph_ptr, float* __restrict__ gram) {
-  __shared__ float sG[HID * HID];
+  extern __shared__ float sG[];
   __shared__ float s_red[kThreads / 32];
   const int g = blockIdx.x;
   const int v0 = graph_ptr[g], v1 = graph_ptr[g + 1];
-  graph_gram(Z, v0, v1, sG);
+  graph_gram<H>(Z, v0, v1, sG);
   __syncthreads();
   float s = 0.f;
-  for (int i = threadIdx.x; i < HID * HID; i += kThreads) s = fmaf(sG[i], sG[i], s);
+  for (int i = threadIdx.x; i < H * H; i += kThreads) s = fmaf(sG[i], sG[i], s);
   s = warp_sum(s);
   if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = s;
   __syncthreads();
@@ -86,22 +98,23 @@ logm_gram_fwd_kernel(const float* __restrict__ Z, const int32_t* __restrict__ gr
 }
 
 // gZ_g = scale * (4 / n^2) Z_g G_g   (overwrites gZ; logm_pair_bwd adds the sparse part afterwards)
+template <int H>
 __global__ void __launch_bounds__(kThreads)
 logm_gram_bwd_kernel(const float* __restrict__ Z, const int32_t* __restrict__ graph_ptr, float scale, float* __restrict__ gZ) {
-  __shared__ float sG[HID * HID];
+  extern __shared__ float sG[];
   const int g = blockIdx.x;
   const int v0 = graph_ptr[g], v1 = graph_ptr[g + 1];
-  graph_gram(Z, v0, v1, sG);
+  graph_gram<H>(Z, v0, v1, sG);
   __syncthreads();
   const float n = (float)(v1 - v0);
   const float f = scale * 4.f / (n * n);
-  const int c = threadIdx.x & (HID - 1);
-  for (int r = v0 + (threadIdx.x >> 6); r < v1; r += kThreads / HID) {
-    const float* z = Z + (size_t)r * HID;
+  const int c = threadIdx.x & (H - 1);
+  for (int r = v0 + threadIdx.x / H; r < v1; r += kThreads / H) {
+    const float* z = Z + (size_t)r * H;
     float s = 0.f;
 #pragma unroll 8
-    for (int q = 0; q < HID; ++q) s = fmaf(__ldg(z + q), sG[q * HID + c], s);
-    gZ[(size_t)r * HID + c] = f * s;
+    for (int q = 0; q < H; ++q) s = fmaf(__ldg(z + q), sG[q * H + c], s);
+    gZ[(size_t)r * H + c] = f * s;
   }
 }
 
@@ -173,18 +186,38 @@ struct LogmPairArgs {
   int32_t* status;
 };
 
+// A lane's H / 32 channels of a Z row: float2 at H = 64, float4 at H = 128.
+template <int H> struct LaneZ;
+template <> struct LaneZ<64> {
+  float2 v;
+  __device__ __forceinline__ static LaneZ load(const float* p) { return {*reinterpret_cast<const float2*>(p)}; }
+  __device__ __forceinline__ void store(float* p) const { *reinterpret_cast<float2*>(p) = v; }
+  __device__ __forceinline__ float dot(const LaneZ& o) const { return v.x * o.v.x + v.y * o.v.y; }
+  __device__ __forceinline__ void fma(float f, const LaneZ& z) { v.x = fmaf(f, z.v.x, v.x); v.y = fmaf(f, z.v.y, v.y); }
+};
+template <> struct LaneZ<128> {
+  float4 v;
+  __device__ __forceinline__ static LaneZ load(const float* p) { return {*reinterpret_cast<const float4*>(p)}; }
+  __device__ __forceinline__ void store(float* p) const { *reinterpret_cast<float4*>(p) = v; }
+  __device__ __forceinline__ float dot(const LaneZ& o) const { return (v.x * o.v.x + v.y * o.v.y) + (v.z * o.v.z + v.w * o.v.w); }
+  __device__ __forceinline__ void fma(float f, const LaneZ& z) {
+    v.x = fmaf(f, z.v.x, v.x); v.y = fmaf(f, z.v.y, v.y); v.z = fmaf(f, z.v.z, v.z); v.w = fmaf(f, z.v.w, v.w);
+  }
+};
+
 // One warp per seed r.  x[i][a] = (A^i)[r][sorted[a]] by dynamic programming on the ball (a neighbour outside the ball is
 // further than k hops from r, so its count is 0 for every step that matters).
-template <bool BWD>
-__global__ void __launch_bounds__(kWarps * 32)
+template <bool BWD, int H>
+__global__ void __launch_bounds__(kWarps * 32, H == 64 ? 0 : 4)
 logm_pair_kernel(LogmPairArgs p) {
+  using LZ = LaneZ<H>;
   __shared__ int s_ball[kWarps][LCAP];
   __shared__ int s_sorted[kWarps][LCAP];
   __shared__ float s_x[kWarps][2][LCAP];
   __shared__ float s_coef[kWarps][LCAP];     // fwd: sum_i L_i[r][c] ; bwd: sum_i (L_i[r][c] + L_i[c][r])
   __shared__ float s_l2[kWarps][LCAP];       // fwd: sum_i L_i[r][c]^2
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int c2 = 2 * lane;
+  const int c2 = (H / 32) * lane;
   for (int r = blockIdx.x * kWarps + warp; r < p.N; r += gridDim.x * kWarps) {
     const int m = sorted_ball(p.indptr, p.indices, r, p.k, s_ball[warp], s_sorted[warp], lane, p.status);
     const int g = graph_of(p.graph_ptr, p.B, r);
@@ -220,27 +253,25 @@ logm_pair_kernel(LogmPairArgs p) {
       }
       __syncwarp();
     }
-    const float2 zr = *reinterpret_cast<const float2*>(p.Z + (size_t)r * HID + c2);
+    const LZ zr = LZ::load(p.Z + (size_t)r * H + c2);
     if (BWD) {
-      float2 acc = make_float2(0.f, 0.f);
+      LZ acc{};
       for (int a = 0; a < m; ++a) {
         const float cf = coef[a];
         if (cf == 0.f) continue;
-        const float2 zc = *reinterpret_cast<const float2*>(p.Z + (size_t)sorted[a] * HID + c2);
-        acc.x = fmaf(cf, zc.x, acc.x); acc.y = fmaf(cf, zc.y, acc.y);
+        acc.fma(cf, LZ::load(p.Z + (size_t)sorted[a] * H + c2));
       }
       const float f = -2.f * p.scale / ((float)p.k * n * n);
-      float2* dst = reinterpret_cast<float2*>(p.gZ + (size_t)r * HID + c2);
-      float2 cur = *dst;
-      cur.x = fmaf(f, acc.x, cur.x); cur.y = fmaf(f, acc.y, cur.y);
-      *dst = cur;
+      float* dst = p.gZ + (size_t)r * H + c2;
+      LZ cur = LZ::load(dst);
+      cur.fma(f, acc);
+      cur.store(dst);
     } else {
       float t = 0.f;                                                      // sum_c ( -2 (z_r . z_c) sum_i L + sum_i L^2 )
       for (int a = 0; a < m; ++a) {
         const float cf = coef[a];
         if (cf == 0.f) continue;
-        const float2 zc = *reinterpret_cast<const float2*>(p.Z + (size_t)sorted[a] * HID + c2);
-        const float h = warp_sum(zr.x * zc.x + zr.y * zc.y);
+        const float h = warp_sum(zr.dot(LZ::load(p.Z + (size_t)sorted[a] * H + c2)));
         t += fmaf(-2.f * h, cf, l2[a]);
       }
       if (lane == 0) p.pair[r] = t / (n * n);
@@ -269,22 +300,40 @@ logm_reduce_kernel(const float* __restrict__ gram, int B, const float* __restric
 
 int logm_max_steps() { return LK; }
 
-void launch_logm_fwd(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
-                     int k, float* walks, float* gram, float* pair, float* loss_out, int32_t* status, cudaStream_t s) {
+template <int H>
+static void launch_logm_fwd_t(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
+                              int k, float* walks, float* gram, float* pair, float* loss_out, int32_t* status, cudaStream_t s) {
+  static bool once = (cudaFuncSetAttribute(logm_gram_fwd_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, gram_smem_bytes<H>()), true);
+  (void)once;
   logm_walks_kernel<<<B, 128, 0, s>>>(graph_ptr, indptr, indices, N, k, walks);
-  logm_gram_fwd_kernel<<<B, kThreads, 0, s>>>(Z, graph_ptr, gram);
+  logm_gram_fwd_kernel<H><<<B, kThreads, gram_smem_bytes<H>(), s>>>(Z, graph_ptr, gram);
   LogmPairArgs a{Z, graph_ptr, indptr, indices, B, N, k, walks, pair, nullptr, 0.f, status};
   const int grid = min((N + kWarps - 1) / kWarps, 16 * num_sms());
-  logm_pair_kernel<false><<<grid, kWarps * 32, 0, s>>>(a);
+  logm_pair_kernel<false, H><<<grid, kWarps * 32, 0, s>>>(a);
   logm_reduce_kernel<<<1, kThreads, 0, s>>>(gram, B, pair, N, k, loss_out);
 }
 
-void launch_logm_bwd(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
-                     int k, const float* walks, float scale, float* gZ, int32_t* status, cudaStream_t s) {
-  logm_gram_bwd_kernel<<<B, kThreads, 0, s>>>(Z, graph_ptr, scale, gZ);
+template <int H>
+static void launch_logm_bwd_t(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
+                              int k, const float* walks, float scale, float* gZ, int32_t* status, cudaStream_t s) {
+  static bool once = (cudaFuncSetAttribute(logm_gram_bwd_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, gram_smem_bytes<H>()), true);
+  (void)once;
+  logm_gram_bwd_kernel<H><<<B, kThreads, gram_smem_bytes<H>(), s>>>(Z, graph_ptr, scale, gZ);
   LogmPairArgs a{Z, graph_ptr, indptr, indices, B, N, k, walks, nullptr, gZ, scale, status};
   const int grid = min((N + kWarps - 1) / kWarps, 16 * num_sms());
-  logm_pair_kernel<true><<<grid, kWarps * 32, 0, s>>>(a);
+  logm_pair_kernel<true, H><<<grid, kWarps * 32, 0, s>>>(a);
+}
+
+void launch_logm_fwd(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
+                     int k, float* walks, float* gram, float* pair, float* loss_out, int32_t* status, int hidden, cudaStream_t s) {
+  if (hidden == 64) launch_logm_fwd_t<64>(Z, graph_ptr, indptr, indices, B, N, k, walks, gram, pair, loss_out, status, s);
+  else launch_logm_fwd_t<128>(Z, graph_ptr, indptr, indices, B, N, k, walks, gram, pair, loss_out, status, s);
+}
+
+void launch_logm_bwd(const float* Z, const int32_t* graph_ptr, const int32_t* indptr, const int32_t* indices, int B, int N,
+                     int k, const float* walks, float scale, float* gZ, int32_t* status, int hidden, cudaStream_t s) {
+  if (hidden == 64) launch_logm_bwd_t<64>(Z, graph_ptr, indptr, indices, B, N, k, walks, scale, gZ, status, s);
+  else launch_logm_bwd_t<128>(Z, graph_ptr, indptr, indices, B, N, k, walks, scale, gZ, status, s);
 }
 
 }  // namespace scgib

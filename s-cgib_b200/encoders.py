@@ -63,14 +63,16 @@ class GraphSAGE(nn.Module):
         h3 = ops.linear_fwd(h2, c2.fc_self.weight, H, X1=m2, W1=c2.fc_neigh.weight, bias=c2.fc_self.bias, relu=False)
         return h3, (t, row_map, indptr, indices, m0, h1, m1, h2, m2)
 
-    def run_backward(self, saved, g_out):
-        """-> (gradient wrt the gathered input rows [V, in_feats], {parameter name: gradient})."""
+    def run_backward(self, saved, g_out, weights=True):
+        """-> (gradient wrt the gathered input rows [V, in_feats], {parameter name: gradient}); ``weights=False`` (every
+        parameter of this encoder frozen) skips the weight-gradient launches and returns an empty dict."""
         t, row_map, indptr, indices, m0, h1, m1, h2, m2 = saved
         H, c1, c2 = self.hidden_dim, self.conv1, self.conv2
         dev = g_out.device
         new = lambda *s: torch.empty(*s, device=dev)
         dWs1, dWn1, db1 = new(H, self.in_feats), new(H, self.in_feats), new(H)
         dWs2, dWn2, db2 = new(H, H), new(H, H), new(H)
+        bwd_w = ops.linear_bwd_w if weights else (lambda *a, **k: None)
         aggT = lambda u, add: ops.graph_aggregate(u, indptr, indices, NORM_MEAN, NORM_NONE, add=add)
 
         def through(g, mask, conv, width):      # gradient wrt the layer input: g Ws + A^T(g Wn), g masked by the layer's ReLU
@@ -79,17 +81,19 @@ class GraphSAGE(nn.Module):
             return aggT(u, gs)
 
         # third layer: conv2 without ReLU
-        ops.linear_bwd_w(g_out, h2, dWs2, db2)
-        ops.linear_bwd_w(g_out, m2, dWn2)
+        bwd_w(g_out, h2, dWs2, db2)
+        bwd_w(g_out, m2, dWn2)
         g_h2 = through(g_out, None, c2, H)
         # second layer: conv2 (its second use: the weight gradients accumulate), ReLU mask h2 > 0
-        ops.linear_bwd_w(g_h2, h1, dWs2, db2, M=h2, accumulate=True)
-        ops.linear_bwd_w(g_h2, m1, dWn2, M=h2, accumulate=True)
+        bwd_w(g_h2, h1, dWs2, db2, M=h2, accumulate=True)
+        bwd_w(g_h2, m1, dWn2, M=h2, accumulate=True)
         g_h1 = through(g_h2, h2, c2, H)
         # first layer: conv1 on the gathered t rows
-        ops.linear_bwd_w(g_h1, t, dWs1, db1, M=h1, map=row_map)
-        ops.linear_bwd_w(g_h1, m0, dWn1, M=h1)
+        bwd_w(g_h1, t, dWs1, db1, M=h1, map=row_map)
+        bwd_w(g_h1, m0, dWn1, M=h1)
         g_t = through(g_h1, h1, c1, self.in_feats)
+        if not weights:
+            return g_t, {}
         return g_t, {"conv1.fc_self.weight": dWs1, "conv1.fc_neigh.weight": dWn1, "conv1.fc_self.bias": db1,
                      "conv2.fc_self.weight": dWs2, "conv2.fc_neigh.weight": dWn2, "conv2.fc_self.bias": db2}
 
@@ -126,7 +130,7 @@ class GCN(nn.Module):
         h3 = ops.linear_fwd(a2, self.conv3.weight, H, w0_kxo=True, bias=self.conv3.bias, relu=False)
         return h3, (indptr, indices, a0, h1, a1, h2, a2)
 
-    def run_backward(self, saved, g_out):
+    def run_backward(self, saved, g_out, weights=True):
         indptr, indices, a0, h1, a1, h2, a2 = saved
         H, dev = self.hidden_dim, g_out.device
         new = lambda *s: torch.empty(*s, device=dev)
@@ -134,12 +138,15 @@ class GCN(nn.Module):
         dW1, db1 = new(self.in_feats, 2 * H), new(2 * H)
         dW2, db2 = new(2 * H, 2 * H), new(2 * H)
         dW3, db3 = new(2 * H, H), new(H)
-        ops.linear_bwd_w(g_out, a2, dW3, db3, kxo=True)
+        bwd_w = ops.linear_bwd_w if weights else (lambda *a, **k: None)
+        bwd_w(g_out, a2, dW3, db3, kxo=True)
         g_h2 = agg(ops.linear_fwd(g_out, self.conv3.weight, 2 * H))                      # g W3^T: W3 [2h, h] read as [O, K]
-        ops.linear_bwd_w(g_h2, a1, dW2, db2, M=h2, kxo=True)
+        bwd_w(g_h2, a1, dW2, db2, M=h2, kxo=True)
         g_h1 = agg(ops.linear_fwd(g_h2, self.conv2.weight, 2 * H, M0=h2))
-        ops.linear_bwd_w(g_h1, a0, dW1, db1, M=h1, kxo=True)
+        bwd_w(g_h1, a0, dW1, db1, M=h1, kxo=True)
         g_t = agg(ops.linear_fwd(g_h1, self.conv1.weight, self.in_feats, M0=h1))
+        if not weights:
+            return g_t, {}
         return g_t, {"conv1.weight": dW1, "conv1.bias": db1, "conv2.weight": dW2, "conv2.bias": db2,
                      "conv3.weight": dW3, "conv3.bias": db3}
 
@@ -180,9 +187,15 @@ def composed_features(outer, g, ego, t, gate_u, feat_u):
     S, sv2 = model.Encoder2.run_forward(t, ego.sub_indptr, ego.sub_indices, row_map=ego.ego_nodes)
     c = model.compressor
     gate = ops.CoreGate(Hd, _f(c[0].weight), _f(c[0].bias), _f(c[1].weight), _f(c[1].bias), _f(c[3].weight), _f(c[3].bias))
-    noisy, lam, readout, core, kl = gate.forward(Hf, g.graph_ptr, gate_u, feat_u)
-    if outer.training:                  # compressor.1 running statistics: B sequential updates, one per graph (models.py:642)
-        gate.update_running(c[1].running_mean, c[1].running_var)
+    bn = c[1]
+    # compressor.1 follows its own training flag, as nn.BatchNorm1d does: per-graph batch statistics and B sequential
+    # running-statistics updates, one per graph (models.py:642), or - in eval - the running statistics (forward only).
+    # The gate / feature noise is drawn in both modes (models.py:599, 650).
+    if bn.training:
+        noisy, lam, readout, core, kl = gate.forward(Hf, g.graph_ptr, gate_u, feat_u)
+        gate.update_running(bn.running_mean, bn.running_var)
+    else:
+        noisy, lam, readout, core, kl = gate.forward(Hf, g.graph_ptr, gate_u, feat_u, running=(bn.running_mean, bn.running_var))
     C = ops.segment_sum_w(S, ego.ego_ptr)
     w_cand = _f(model.attn_layer.weight[0, Hd:])
     alpha, _ = ops.core_cand_attn_fwd(C, g.graph_ptr, w_cand)
@@ -205,6 +218,39 @@ def composed_param_names(model):
     return names
 
 
+def composed_backward(outer, st, gZ, g_core, g_readout, kl_scale, names):
+    """The backward of ``composed_features`` + head MLP: gradients of <gZ, Z> + <g_core, core_readout> +
+    <g_readout, graph_readout> + kl_scale * KL for the parameter ``names`` (composed_param_names order), as a dict.
+    The input-gradient chain always runs down to transfer_d; an encoder none of whose parameters is named (all frozen:
+    fine-tuning) skips its weight-gradient launches."""
+    model = inner_of(outer)
+    g, ego = st["g"], st["ego"]
+    Hd = int(outer.hidden_dim)
+    gI, dW1h, db1h, dW2h, db2h = st["head"].backward(gZ)
+    gC, dw_cand = ops.core_cand_attn_bwd(st["C"], st["alpha"], gI[1], g.graph_ptr, st["w_cand"])
+    gH, dWc1, dbc1, dgam, dbet, dwc2, dbc2 = st["gate"].backward(gI[0], g_core, g_readout, kl_scale=kl_scale)
+    gS = ops.segment_sum_bwd(gC, ego.ego_ptr, st["Ns"])
+    w1 = any(n.startswith("Encoder1.") for n in names)
+    w2 = any(n.startswith("Encoder2.") for n in names)
+    gt0, ge1 = model.Encoder1.run_backward(st["sv1"], gH, weights=w1)
+    gt1, ge2 = model.Encoder2.run_backward(st["sv2"], gS, weights=w2)
+    dWt = ops.transfer_bwd(st["x"], gt0, gt1, ego.ego_nodes, normalize=True)
+    d_attn = torch.zeros(1, 2 * Hd, device=gH.device)
+    d_attn[0, Hd:] = dw_cand            # the core half and the bias cancel inside the per-graph softmax: exactly zero
+    grads = {"transfer_d.weight": dWt, "attn_layer.weight": d_attn, "attn_layer.bias": torch.zeros(1, device=gH.device),
+             "MLP.0.weight": dW1h, "MLP.0.bias": db1h, "MLP.2.weight": dW2h, "MLP.2.bias": db2h,
+             "compressor.0.weight": dWc1, "compressor.0.bias": dbc1, "compressor.1.weight": dgam, "compressor.1.bias": dbet,
+             "compressor.3.weight": dwc2.reshape(1, Hd), "compressor.3.bias": dbc2.reshape(1)}
+    grads.update({"Encoder1." + n: v for n, v in ge1.items()})
+    grads.update({"Encoder2." + n: v for n, v in ge2.items()})
+    return {n: grads[n] for n in names}
+
+
+def trainable_param_names(outer):
+    """composed_param_names restricted to the parameters that require a gradient (fine-tuning freezes the loaded model)."""
+    return [n for n in composed_param_names(outer) if resolve_param(outer, n).requires_grad]
+
+
 class ComposedPretrainFn(torch.autograd.Function):
     """Mainmodel.forward (models.py:662-700) for --encoder GraphSAGE / GCN: (KL, contrastive, reconstruction)."""
 
@@ -212,7 +258,10 @@ class ComposedPretrainFn(torch.autograd.Function):
     def forward(ctx, model, g, ego, x, gate_u, feat_u, names, *params):
         t = ops.input_proj(x, _f(model.transfer_d.weight))                 # F.normalize + transfer_d (idempotent on normalised x)
         out, st = composed_features(model, g, ego, t, gate_u, feat_u)
-        rec, gZ = ops.recon_adj(out["Z"], g.indptr, g.indices, 1.0)        # value and gradient in one launch sequence
+        if getattr(model, "recons_type", "adj") == "logM":                 # models.py:693-694: k-step log transition matrices
+            rec, gZ, _ = ops.recon_logm(out["Z"], g.graph_ptr, g.indptr, g.indices, int(model.k_transition), 1.0)
+        else:
+            rec, gZ = ops.recon_adj(out["Z"], g.indptr, g.indices, 1.0)    # value and gradient in one launch sequence
         con, g_core, g_readout = ops.contrastive(out["core_readout"], out["graph_readout"], 1.0)
         st.update(gZ=gZ, g_core=g_core, g_readout=g_readout, x=x, g=g, ego=ego)
         ctx.model, ctx.st, ctx.names = model, st, names
@@ -222,8 +271,6 @@ class ComposedPretrainFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_kl, g_con, g_rec):
         model, st, names = ctx.model, ctx.st, ctx.names
-        g, ego = st["g"], st["ego"]
-        Hd = int(model.hidden_dim)
         same = g_kl.data_ptr() == g_con.data_ptr() == g_rec.data_ptr() and g_kl.numel() == 1
         if same:        # loss = KL + recon + contrastive (exp_pretraining.py:320): scale the parameter gradients once, no host read
             s_kl = s_con = s_rec = 1.0
@@ -232,23 +279,82 @@ class ComposedPretrainFn(torch.autograd.Function):
         gZ = st["gZ"] if s_rec == 1.0 else st["gZ"] * s_rec
         g_core = st["g_core"] if s_con == 1.0 else st["g_core"] * s_con
         g_readout = st["g_readout"] if s_con == 1.0 else st["g_readout"] * s_con
-        gI, dW1h, db1h, dW2h, db2h = st["head"].backward(gZ)
-        gC, dw_cand = ops.core_cand_attn_bwd(st["C"], st["alpha"], gI[1], g.graph_ptr, st["w_cand"])
-        gH, dWc1, dbc1, dgam, dbet, dwc2, dbc2 = st["gate"].backward(gI[0], g_core, g_readout, kl_scale=s_kl)
-        gS = ops.segment_sum_bwd(gC, ego.ego_ptr, st["Ns"])
-        gt0, ge1 = inner_of(model).Encoder1.run_backward(st["sv1"], gH)
-        gt1, ge2 = inner_of(model).Encoder2.run_backward(st["sv2"], gS)
-        dWt = ops.transfer_bwd(st["x"], gt0, gt1, ego.ego_nodes, normalize=True)
-        d_attn = torch.zeros(1, 2 * Hd, device=gH.device)
-        d_attn[0, Hd:] = dw_cand            # the core half and the bias cancel inside the per-graph softmax: exactly zero
-        grads = {"transfer_d.weight": dWt, "attn_layer.weight": d_attn, "attn_layer.bias": torch.zeros(1, device=gH.device),
-                 "MLP.0.weight": dW1h, "MLP.0.bias": db1h, "MLP.2.weight": dW2h, "MLP.2.bias": db2h,
-                 "compressor.0.weight": dWc1, "compressor.0.bias": dbc1, "compressor.1.weight": dgam, "compressor.1.bias": dbet,
-                 "compressor.3.weight": dwc2.reshape(1, Hd), "compressor.3.bias": dbc2.reshape(1)}
-        grads.update({"Encoder1." + n: v for n, v in ge1.items()})
-        grads.update({"Encoder2." + n: v for n, v in ge2.items()})
+        grads = composed_backward(model, st, gZ, g_core, g_readout, s_kl, names)
         out = [grads[n] for n in names]
         if same:
             torch._foreach_mul_(out, g_kl.reshape(()).to(out[0].dtype))
         ctx.st = None
         return (None,) * 7 + tuple(out)
+
+
+def _zero_readout_grads(st, outer):
+    B, Hd = st["g"].batch_size, int(outer.hidden_dim)
+    z = torch.zeros(B, Hd, device=st["x"].device)
+    return z, z
+
+
+class ComposedFinetuneFn(torch.autograd.Function):
+    """Mainmodel_finetuning.forward (models.py:501-520) around GraphSAGE / GCN encoders: transfer_d -> the loaded model's
+    extract_features -> MLP -> Set2Set -> predict (-> sigmoid).  Parameters: ``names`` (composed_param_names of the ones that
+    require a gradient), then the head's FT_NAMES slots."""
+
+    @staticmethod
+    def forward(ctx, owner, g, ego, x, gate_u, feat_u, names, *params):
+        head = owner._head
+        t = ops.input_proj(x, _f(owner.transfer_d.weight))
+        out, st = composed_features(owner, g, ego, t, gate_u, feat_u)
+        scores = head.forward(out["Z"], g.graph_ptr)
+        st.update(x=x, g=g, ego=ego)
+        ctx.owner, ctx.st, ctx.names, ctx.params = owner, st, names, params
+        ctx.serial = head.fwd_serial
+        return scores
+
+    @staticmethod
+    def backward(ctx, g_scores):
+        from .models import _check_serial, _detach_aliased_grads
+        from .engine import FT_NAMES
+        owner, st, names = ctx.owner, ctx.st, ctx.names
+        head = owner._head
+        _check_serial("Mainmodel_finetuning (head)", head, ctx.serial)
+        _detach_aliased_grads(ctx.params, head.grads)
+        gZ = head.backward(g_scores)
+        g_core, g_readout = _zero_readout_grads(st, owner)
+        grads = composed_backward(owner, st, gZ, g_core, g_readout, 0.0, names)
+        hv = head.views(grads=True)
+        ctx.st = None
+        return (None,) * 7 + tuple(grads[n] for n in names) + tuple(hv.pop(n) for n in FT_NAMES)
+
+
+class ComposedDomainAdaptFn(torch.autograd.Function):
+    """Mainmodel_domainadapt.forward (models.py:254-269) around GraphSAGE / GCN encoders -> (r_transfer_d(s2s(MLP(
+    extract_features))) [B, 2 in_dim], s2s_rev(x) [B, 2 in_dim]).  Parameters: ``names``, the head's slots (r_transfer_d in
+    the predict slots), the four s2s_rev LSTM tensors."""
+
+    @staticmethod
+    def forward(ctx, owner, g, ego, x, gate_u, feat_u, x_norm, names, *params):
+        head, rev = owner._head, owner._rev
+        t = ops.input_proj(x, _f(owner.transfer_d.weight))
+        out, st = composed_features(owner, g, ego, t, gate_u, feat_u)
+        rec = head.forward(out["Z"], g.graph_ptr)
+        org = rev.forward(x_norm, g.graph_ptr)
+        st.update(x=x, g=g, ego=ego)
+        ctx.owner, ctx.st, ctx.names, ctx.params = owner, st, names, params
+        ctx.serial = (head.fwd_serial, rev.head.fwd_serial)
+        return rec, org
+
+    @staticmethod
+    def backward(ctx, g_rec, g_org):
+        from .models import _check_serial, _detach_aliased_grads
+        from .engine import FT_NAMES
+        owner, st, names = ctx.owner, ctx.st, ctx.names
+        head, rev = owner._head, owner._rev
+        _check_serial("Mainmodel_domainadapt (head)", head, ctx.serial[0])
+        _check_serial("Mainmodel_domainadapt (s2s_rev)", rev.head, ctx.serial[1])
+        _detach_aliased_grads(ctx.params, head.grads)
+        gZ = head.backward(g_rec)
+        g_core, g_readout = _zero_readout_grads(st, owner)
+        grads = composed_backward(owner, st, gZ, g_core, g_readout, 0.0, names)
+        hv = head.views(grads=True)
+        ctx.st = None
+        return ((None,) * 8 + tuple(grads[n] for n in names) + tuple(hv.pop(n) for n in FT_NAMES) +
+                tuple(rev.backward(g_org)))

@@ -227,6 +227,29 @@ def _check_args(args, encoder, allowed=("GIN",)):
         raise NotImplementedError("B200 path covers --readout_f sum --recons_type adj|logM --useAtt 1")
 
 
+def _own_encoders(encoder, in_dim, hidden_dim, gin_layers):
+    """Encoder1 / Encoder2 of the fine-tuning / domain-adaptation wrappers: constructed (state-dict keys, RNG draws) and never
+    called, with the switch Mainmodel_continue uses (models.py:576-581)."""
+    if encoder == "GIN":
+        return GIN(in_dim, hidden_dim, gin_layers), GIN(in_dim, hidden_dim, gin_layers)
+    from .encoders import make_encoder
+    return make_encoder(encoder, in_dim, hidden_dim), make_encoder(encoder, in_dim, hidden_dim)
+
+
+def _bump_compressor_batches(loaded, B):
+    """num_batches_tracked of the loaded compressor.1 after a composed forward: one BatchNorm call per graph (models.py:642)."""
+    bn = loaded.compressor[1]
+    if bn.training:
+        bn.num_batches_tracked += B
+
+
+def _loaded_encoder_kind(loaded):
+    """The encoders a fine-tuning / domain-adaptation forward runs are the LOADED module's (``self.model.Encoder1``,
+    models.py:508, 262), whatever the wrapper's own ``encoder`` argument: after domain adaptation that is the adapter's own
+    encoders (SURVEY 3.1).  They select the path: the fused GIN engine or the operator-composed GraphSAGE / GCN step."""
+    return getattr(loaded.Encoder1, "kind", "GIN")
+
+
 class _HotPathMixin:
     """forward / extract_features shared by Mainmodel and Mainmodel_continue."""
 
@@ -255,9 +278,6 @@ class _HotPathMixin:
         return torch.rand(N, device=device), torch.rand(N, H, device=device)
 
     def _composed_inputs(self, batch_g, flatten_batch_subgraphs, device):
-        if not self.training:
-            raise NotImplementedError("model.eval() with --encoder GraphSAGE / GCN: the operator-composed step implements the "
-                                      "training-mode BatchNorm of the compressor (use --encoder GIN for eval-mode forwards)")
         g = batch_g if batch_g.device == torch.device(device) else batch_g.to(device)
         ego = flatten_batch_subgraphs
         if not isinstance(ego, EgoBatch):
@@ -271,16 +291,16 @@ class _HotPathMixin:
     def _forward_composed(self, batch_g, batch_x, flatten_batch_subgraphs, device):
         """--encoder GraphSAGE / GCN: the step composed from operator kernels (encoders.py)."""
         from . import encoders
-        if getattr(self, "recons_type", "adj") != "adj":
-            raise NotImplementedError("--recons_type logM runs with --encoder GIN on the B200 path")
+        if not self.training:
+            raise NotImplementedError("model.eval() forward with --encoder GraphSAGE / GCN: the pre-training losses are built for "
+                                      "training mode (eval-mode features: extract_features, Mainmodel_finetuning)")
         g, ego = self._composed_inputs(batch_g, flatten_batch_subgraphs, device)
         x = batch_x.to(g.device).float().contiguous()
         gate_u, feat_u = self._noise(x.shape[0], g.device)
         names = encoders.composed_param_names(self)
         kl, con, rec = encoders.ComposedPretrainFn.apply(self, g, ego, x, gate_u.contiguous(), feat_u.contiguous(), names,
                                                          *[encoders.resolve_param(self, n) for n in names])
-        if self.training:
-            encoders.inner_of(self).compressor[1].num_batches_tracked += g.batch_size     # one BatchNorm call per graph (models.py:642)
+        _bump_compressor_batches(encoders.inner_of(self), g.batch_size)
         return None, kl, con, rec
 
     def forward(self, batch_g, batch_x, flatten_batch_subgraphs, batch_logMs, x_subs, current_epoch, edge_index,
@@ -474,7 +494,8 @@ class Mainmodel_finetuning(nn.Module):
 
     def __init__(self, args, in_dim, hidden_dim, num_layers, num_heads, k_transition, num_classes, cp_filename, encoder):
         super().__init__()
-        _check_args(args, encoder)
+        _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
+        _check_composed_width(encoder, hidden_dim)
         self.tau = 1.0
         self.dataset = args.dataset
         self.readout = args.readout_f
@@ -504,15 +525,16 @@ class Mainmodel_finetuning(nn.Module):
                                      nn.Linear(self.hidden_dim, out_dim))
         self.MLP = nn.Sequential(nn.Linear(2 * self.hidden_dim, self.hidden_dim), nn.ReLU(),
                                  nn.Linear(self.hidden_dim, self.hidden_dim))
-        self.Encoder1 = GIN(self.in_dim, hidden_dim, self.gin_layers)
-        self.Encoder2 = GIN(self.in_dim, hidden_dim, self.gin_layers)
+        self.Encoder1, self.Encoder2 = _own_encoders(encoder, self.in_dim, hidden_dim, self.gin_layers)
         print("Loading pre-trained model .pt  ... ")
         self.model = torch.load(cp_filename, map_location=args.device, weights_only=False)
         for name, para in self.model.named_parameters():     # models.py:424-435: the last list entry decides
-            para.requires_grad = "layers.2" in name
+            para.requires_grad = "layers.2" in name          # (no GraphSAGE / GCN name contains it: all frozen)
         self.compressor = nn.Sequential(nn.Linear(self.hidden_dim, self.hidden_dim), nn.BatchNorm1d(self.hidden_dim),
                                         nn.ReLU(), nn.Linear(self.hidden_dim, 1))
-        self._bridge = _Bridge(self, in_dim, self.gin_layers)
+        self.encoder_kind = _loaded_encoder_kind(self.model)
+        _check_composed_width(self.encoder_kind, hidden_dim)
+        self._bridge = _Bridge(self, in_dim, self.gin_layers) if self.encoder_kind == "GIN" else None
         self._head = None
 
     def __getstate__(self):
@@ -526,6 +548,7 @@ class Mainmodel_finetuning(nn.Module):
 
     _device_batch = _HotPathMixin._device_batch
     _noise = _HotPathMixin._noise
+    _composed_inputs = _HotPathMixin._composed_inputs
 
     def _sync_head(self, device):
         device = torch.device(device)
@@ -553,6 +576,8 @@ class Mainmodel_finetuning(nn.Module):
         """reference models.py:501-520 -> (scores [B,C], 0, 0, 0)."""
         self.batch_size = batch_size
         self.device = device
+        if getattr(self, "encoder_kind", "GIN") != "GIN":         # (wrappers pickled before encoder_kind existed are GIN)
+            return self._forward_composed(batch_g, batch_x, flatten_batch_subgraphs, device), 0, 0, 0
         params = self._bridge.sync(device) + self._sync_head(device)
         self._bridge.training = self.training
         b = self._device_batch(batch_g, batch_x, flatten_batch_subgraphs, device)
@@ -561,6 +586,19 @@ class Mainmodel_finetuning(nn.Module):
         if self.training:
             _HotPathMixin._bump_batches_tracked(self, b.B)
         return scores, 0, 0, 0
+
+    def _forward_composed(self, batch_g, batch_x, flatten_batch_subgraphs, device):
+        """GraphSAGE / GCN encoders in the loaded module: the feature path composed from operator kernels (encoders.py)."""
+        from . import encoders
+        g, ego = self._composed_inputs(batch_g, flatten_batch_subgraphs, device)
+        head_params = self._sync_head(device)
+        x = batch_x.to(g.device).float().contiguous()
+        gate_u, feat_u = self._noise(x.shape[0], g.device)
+        names = encoders.trainable_param_names(self)
+        scores = encoders.ComposedFinetuneFn.apply(self, g, ego, x, gate_u.contiguous(), feat_u.contiguous(), names,
+                                                   *[encoders.resolve_param(self, n) for n in names], *head_params)
+        _bump_compressor_batches(self.model, g.batch_size)
+        return scores
 
     # loss helpers: reference models.py:522-543 (operate on the [B,C] scores)
     def loss(self, scores, targets):
@@ -624,7 +662,8 @@ class Mainmodel_domainadapt(nn.Module):
 
     def __init__(self, args, in_dim, hidden_dim, num_layers, num_heads, k_transition, num_classes, cp_filename, encoder):
         super().__init__()
-        _check_args(args, encoder)
+        _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
+        _check_composed_width(encoder, hidden_dim)
         self.tau = 1.0
         self.readout = args.readout_f
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
@@ -650,8 +689,7 @@ class Mainmodel_domainadapt(nn.Module):
                                      nn.Linear(self.hidden_dim, out_dim))
         self.MLP = nn.Sequential(nn.Linear(2 * self.hidden_dim, self.hidden_dim), nn.ReLU(),
                                  nn.Linear(self.hidden_dim, self.hidden_dim))
-        self.Encoder1 = GIN(self.in_dim, hidden_dim, self.gin_layers)
-        self.Encoder2 = GIN(self.in_dim, hidden_dim, self.gin_layers)
+        self.Encoder1, self.Encoder2 = _own_encoders(encoder, self.in_dim, hidden_dim, self.gin_layers)
         print("Loading pre-trained model .pt  ... ")
         self.model = torch.load(cp_filename, map_location=args.device, weights_only=False)
         for p in self.model.parameters():
@@ -660,7 +698,9 @@ class Mainmodel_domainadapt(nn.Module):
                                         nn.ReLU(), nn.Linear(self.hidden_dim, 1))
         self.reconstructX = nn.Sequential(nn.Linear(self.hidden_dim, self.hidden_dim), nn.ReLU(),
                                           nn.Linear(self.hidden_dim, in_dim))
-        self._bridge = _Bridge(self, in_dim, self.gin_layers)
+        self.encoder_kind = _loaded_encoder_kind(self.model)
+        _check_composed_width(self.encoder_kind, hidden_dim)
+        self._bridge = _Bridge(self, in_dim, self.gin_layers) if self.encoder_kind == "GIN" else None
         self._head = None
         self._rev = None
 
@@ -677,6 +717,7 @@ class Mainmodel_domainadapt(nn.Module):
 
     _device_batch = _HotPathMixin._device_batch
     _noise = _HotPathMixin._noise
+    _composed_inputs = _HotPathMixin._composed_inputs
 
     def _sync_heads(self, device):
         device = torch.device(device)
@@ -706,6 +747,8 @@ class Mainmodel_domainadapt(nn.Module):
         """reference models.py:254-269 -> X_loss (scalar)."""
         self.batch_size = batch_size
         self.device = device
+        if getattr(self, "encoder_kind", "GIN") != "GIN":
+            return self._forward_composed(batch_g, batch_x, flatten_batch_subgraphs, device)
         params = self._bridge.sync(device) + self._sync_heads(device)
         self._bridge.training = self.training
         b = self._device_batch(batch_g, batch_x, flatten_batch_subgraphs, device)
@@ -713,6 +756,20 @@ class Mainmodel_domainadapt(nn.Module):
         rec, org = _DomainAdaptFn.apply(self, b, gate_u, feat_u, b.x, *params)
         if self.training:
             _HotPathMixin._bump_batches_tracked(self, b.B)
+        return self.loss_X(org, rec)
+
+    def _forward_composed(self, batch_g, batch_x, flatten_batch_subgraphs, device):
+        """GraphSAGE / GCN encoders in the loaded module: the feature path composed from operator kernels (encoders.py);
+        every parameter of the loaded model is trainable."""
+        from . import encoders
+        g, ego = self._composed_inputs(batch_g, flatten_batch_subgraphs, device)
+        head_params = self._sync_heads(device)
+        x = batch_x.to(g.device).float().contiguous()
+        gate_u, feat_u = self._noise(x.shape[0], g.device)
+        names = encoders.trainable_param_names(self)
+        rec, org = encoders.ComposedDomainAdaptFn.apply(self, g, ego, x, gate_u.contiguous(), feat_u.contiguous(), x, names,
+                                                        *[encoders.resolve_param(self, n) for n in names], *head_params)
+        _bump_compressor_batches(self.model, g.batch_size)
         return self.loss_X(org, rec)
 
     def loss_X(self, batch_x_org, interaction_map):

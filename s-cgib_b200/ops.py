@@ -96,6 +96,24 @@ def recon_adj(Z, indptr, indices, scale=1.0, want_grad=True):
     return loss, gZ
 
 
+def recon_logm(Z, graph_ptr, indptr, indices, k, scale=1.0, want_grad=True):
+    """loss_recon of --recons_type logM (models.py:770-782, k-step log transition matrices of util.py:60-91) and
+    scale * d loss / d Z, hidden 64 or 128; returns (loss[1], gZ or None, status[1]).  status is 1 when a k-hop ball
+    exceeded the ego-net capacity (its terms are dropped); it is left on the device (no host sync)."""
+    _cuda(Z, graph_ptr, indptr, indices)
+    lib = _lib.load()
+    Z = _c32(Z)
+    N, H, B = Z.shape[0], Z.shape[1], graph_ptr.numel() - 1
+    loss = torch.empty(1, device=Z.device)
+    status = torch.empty(1, dtype=torch.int32, device=Z.device)
+    gZ = torch.empty_like(Z) if want_grad else None
+    ws = _ws(lib.scgib_recon_logm_workspace_bytes(B, N, int(k)), Z.device)
+    _lib.check(lib.scgib_recon_logm_h_f32(_lib.ptr(Z), _lib.ptr(graph_ptr), _lib.ptr(indptr), _lib.ptr(indices), B, N, H, int(k),
+                                          float(scale), _lib.ptr(loss), _lib.ptr(gZ), _lib.ptr(status),
+                                          _lib.ptr(ws), ws.numel(), _stream(Z)), "recon_logm")
+    return loss, gZ, status
+
+
 def contrastive(core, readout, scale=1.0, want_grad=True):
     """batched_semi_loss (models.py:606-629) of the core / graph readouts and its gradients; returns (loss[1], g_core, g_readout)."""
     _cuda(core, readout)
@@ -129,23 +147,36 @@ class CoreGate:
         self.H = int(hidden)
         self.p = [t.contiguous().float() for t in (Wc1, bc1, gamma_c, beta_c, wc2, bc2)]
 
-    def forward(self, Hfeat, graph_ptr, gate_u, feat_u):
+    def forward(self, Hfeat, graph_ptr, gate_u, feat_u, running=None):
+        """``running`` = (running_mean, running_var) of compressor.1: model.eval() BatchNorm, forward only (no backward and
+        no running-statistics update may follow)."""
         _cuda(Hfeat, graph_ptr, gate_u, feat_u)
         lib, H, dev = _lib.load(), self.H, Hfeat.device
         N, B = Hfeat.shape[0], graph_ptr.numel() - 1
         self.ws = _ws(lib.scgib_core_gate_workspace_bytes(H, B, N), dev)
         self.saved = (graph_ptr, B, N, feat_u.contiguous())
+        self.eval_forward = running is not None
         noisy, lam = torch.empty(N, H, device=dev), torch.empty(N, device=dev)
         readout, core, kl = torch.empty(B, H, device=dev), torch.empty(B, H, device=dev), torch.empty(1, device=dev)
         W, b, g, be, w2, b2 = self.p
-        _lib.check(lib.scgib_core_gate_fwd_f32(_lib.ptr(Hfeat.contiguous()), _lib.ptr(graph_ptr), B, N, H, _lib.ptr(W), _lib.ptr(b),
-                                               _lib.ptr(g), _lib.ptr(be), _lib.ptr(w2), _lib.ptr(b2), _lib.ptr(gate_u.contiguous()),
-                                               _lib.ptr(self.saved[3]), _lib.ptr(noisy), _lib.ptr(lam), _lib.ptr(readout), _lib.ptr(core),
-                                               _lib.ptr(kl), _lib.ptr(self.ws), self.ws.numel(), _stream(Hfeat)), "core_gate_fwd")
+        common = (_lib.ptr(Hfeat.contiguous()), _lib.ptr(graph_ptr), B, N, H, _lib.ptr(W), _lib.ptr(b), _lib.ptr(g), _lib.ptr(be),
+                  _lib.ptr(w2), _lib.ptr(b2))
+        tail = (_lib.ptr(gate_u.contiguous()), _lib.ptr(self.saved[3]), _lib.ptr(noisy), _lib.ptr(lam), _lib.ptr(readout),
+                _lib.ptr(core), _lib.ptr(kl), _lib.ptr(self.ws), self.ws.numel(), _stream(Hfeat))
+        if running is None:
+            _lib.check(lib.scgib_core_gate_fwd_f32(*common, *tail), "core_gate_fwd")
+        else:
+            run = torch.stack([_c32(running[0]), _c32(running[1])]).contiguous()
+            _lib.check(lib.scgib_core_gate_eval_fwd_f32(*common, _lib.ptr(run), *tail), "core_gate_eval_fwd")
         return noisy, lam, readout, core, kl
+
+    def _check_train_forward(self, what):
+        if self.eval_forward:
+            raise RuntimeError("CoreGate.%s() after an eval-mode forward (running statistics): the eval gate is forward only" % what)
 
     def update_running(self, running_mean, running_var):
         """compressor.1's running statistics after this forward's B per-graph BatchNorm calls (models.py:642), in place."""
+        self._check_train_forward("update_running")
         graph_ptr, B, N, feat_u = self.saved
         run = torch.stack([running_mean, running_var]).contiguous().float()
         _lib.check(_lib.load().scgib_core_gate_ema_f32(B, N, self.H, _lib.ptr(run), _lib.ptr(self.ws), self.ws.numel(), _stream(run)),
@@ -153,6 +184,7 @@ class CoreGate:
         running_mean.copy_(run[0]); running_var.copy_(run[1])
 
     def backward(self, g_noisy, g_core, g_readout, kl_scale=1.0):
+        self._check_train_forward("backward")
         lib, H = _lib.load(), self.H
         graph_ptr, B, N, feat_u = self.saved
         dev = feat_u.device
