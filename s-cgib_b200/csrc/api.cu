@@ -1278,7 +1278,7 @@ extern "C" SCGIB_API int scgib_segment_sum_bwd_f32(const float* g_out, const int
 
 // head MLP (models.py:569-572, 676): Z = W2 relu(W1 [noisy || alpha C] + b1) + b2
 namespace scgib {
-struct HeadOpWs { float *w1t, *w2t, *aC, *r, *Zc, *w1a, *w1b, *bnid, *cvec, *ppart; int64_t off[4], pstride; size_t bytes; };
+struct HeadOpWs { float *w1t, *w2t, *aC, *r, *Zc, *w1a, *w1b, *bnid, *cvec, *ppart; unsigned int* xmax; int64_t off[4], pstride; size_t bytes; };
 static HeadOpWs head_op_carve(int H, int N, void* base) {
   HeadOpWs w;
   char* p = (char*)base;
@@ -1289,6 +1289,7 @@ static HeadOpWs head_op_carve(int H, int N, void* base) {
   w.off[0] = 0; w.off[1] = (int64_t)2 * H * H; w.off[2] = w.off[1] + H; w.off[3] = w.off[2] + (int64_t)H * H;   // W1 b1 W2 b2
   w.pstride = w.off[3] + H;
   w.ppart = take((size_t)num_sms() * w.pstride);
+  w.xmax = (unsigned int*)take(4);
   w.bytes = o;
   return w;
 }
@@ -1317,6 +1318,13 @@ extern "C" SCGIB_API int scgib_head_mlp_fwd_f32(const float* noisy, const float*
   launch_transposes(jobs, s);
   HeadFwdArgs a{noisy, C, alpha, N, w.w1t, b1, w.w2t, b2, interaction_map, w.aC, w.r, w.Zc};
   a.W1n = W1; a.W2n = W2;
+  if (H == 64) {      // any input magnitude (GraphSAGE / GCN features are unbounded): the tensor-core head's power-of-two pre-scale
+    cudaMemsetAsync(w.xmax, 0, 3 * sizeof(unsigned int), s);
+    launch_absmax(noisy, (size_t)N * H, w.xmax, s);
+    launch_absmax(C, (size_t)N * H, w.xmax + 1, s);
+    launch_absmax(alpha, (size_t)N, w.xmax + 2, s);
+    a.xmax = w.xmax;
+  }
   launch_head_fwd(a, H, s);
   cudaMemcpyAsync(Z, w.Zc, (size_t)N * H * sizeof(float), cudaMemcpyDeviceToDevice, s);
   return (int)cudaGetLastError();

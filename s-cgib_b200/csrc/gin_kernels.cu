@@ -149,20 +149,28 @@ void launch_fwd_prep(FwdPrepArgs a, cudaStream_t s, bool out_bf16) {
   else launch_k((fwd_prep_kernel<false>), dim3(grid), dim3(kThreads), 0, s, a);
 }
 
-__global__ void __launch_bounds__(kThreads) absmax_kernel(const float* __restrict__ x, size_t n4, unsigned int* __restrict__ slot) {
+template <bool VEC>      // VEC: float4 loads (x 16-byte aligned, n a multiple of 4)
+__global__ void __launch_bounds__(kThreads) absmax_kernel(const float* __restrict__ x, size_t n, unsigned int* __restrict__ slot) {
   pdl_sync();
   float m = 0.f;
-  for (size_t i = (size_t)blockIdx.x * kThreads + threadIdx.x; i < n4; i += (size_t)gridDim.x * kThreads) {
-    const float4 v = ld4(x + 4 * i);
-    m = fmaxf(fmaxf(m, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
+  for (size_t i = (size_t)blockIdx.x * kThreads + threadIdx.x; i < (VEC ? n / 4 : n); i += (size_t)gridDim.x * kThreads) {
+    if (VEC) {
+      const float4 v = ld4(x + 4 * i);
+      m = fmaxf(fmaxf(m, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
+    } else {
+      m = fmaxf(m, fabsf(x[i]));
+    }
   }
   m = warp_max(m);
   if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(slot, __float_as_uint(m));
 }
-void launch_absmax(const float* x, size_t n, unsigned int* slot, cudaStream_t s) {   // n multiple of 4
-  const size_t n4 = n / 4;
-  const int grid = (int)min((size_t)(4 * num_sms()), (n4 + kThreads - 1) / kThreads);
-  if (n4 > 0) launch_k((absmax_kernel), dim3(grid), dim3(kThreads), 0, s, x, n4, slot);
+void launch_absmax(const float* x, size_t n, unsigned int* slot, cudaStream_t s) {
+  const bool vec = (n & 3) == 0 && ((uintptr_t)x & 15u) == 0;
+  const size_t units = vec ? n / 4 : n;
+  const int grid = (int)min((size_t)(4 * num_sms()), (units + kThreads - 1) / kThreads);
+  if (units == 0) return;
+  if (vec) launch_k((absmax_kernel<true>), dim3(grid), dim3(kThreads), 0, s, x, n, slot);
+  else launch_k((absmax_kernel<false>), dim3(grid), dim3(kThreads), 0, s, x, n, slot);
 }
 
 __global__ void __launch_bounds__(kThreads) f32_to_bf16_kernel(const float* __restrict__ in, bf16_t* __restrict__ out, size_t n4) {

@@ -6,8 +6,13 @@
 // 22 significand bits at every magnitude) and a product is two kind::f16 MMAs per K = 16 step: A_hi x [B_hi | B_lo'] (N = 128:
 // the hi hi and hi lo' parts in separate accumulator columns) and A_lo' x B_hi accumulated into the lo' columns; the epilogue
 // forms hh + 2^-11 (hl' + l'h) - the same 2^-22-class product as the 3xTF32 scheme of the GIN kernels, with half the MMAs
-// (16 + 8 per 128-row tile) and half the operand bytes.  Forward activations are O(1), far inside fp16's range (clamped to
-// +-65504); the weights are scaled by 2^4 (undone exactly in the epilogues).  r = relu(u + b1) goes to GEMM2 through TENSOR
+// (16 + 8 per 128-row tile) and half the operand bytes.  The weights are scaled by 2^4 (undone exactly in the epilogues).  The
+// inputs are used as they are when their magnitudes stay below 2^5 (GIN: relu(BN(.)) features, O(1)); otherwise (GraphSAGE /
+// GCN features end without an activation, and the op entry accepts any magnitude) the caller passes max |noisy|, max |C| and
+// max |alpha| in device slots (xmax) and the producers multiply [noisy || alpha C] by the power of two S that brings that bound
+// into [2^4, 2^5).  The head is positively homogeneous up to its biases, so r' = relu(W1 S x + S b1) = S r and the epilogues undo
+// S exactly with the 2^-4 of the weights: no rounding changes, no host synchronisation.  fp16's range then holds r' up to
+// ||W1||_inf ~ 2^11; the operands are still clamped to +-65504 as a last resort.  r = relu(u + b1) goes to GEMM2 through TENSOR
 // MEMORY (16-bit A operand: two K values per column).
 // Producers build [noisy || alpha C] (never materialised in HBM unless the caller asks for interaction_map) with 32-byte
 // loads of 8 channels; alpha C and r are saved for the head backward.  Replaces the FP32-FFMA head_fwd_kernel (75 -> ~25 us
@@ -113,6 +118,16 @@ head_fwd_tc_kernel(HeadFwdArgs p) {
   __syncthreads();
   fence_after_sync();
   const uint32_t tmem = *s_tmem;
+  float S = 1.f;                                              // input pre-scale (header): 1 unless the inputs exceed 2^5
+  if (!GATE && p.xmax) {
+    const float bound = fmaxf(__uint_as_float(__ldcg(p.xmax)), __uint_as_float(__ldcg(p.xmax + 1)) * __uint_as_float(__ldcg(p.xmax + 2)));
+    if (bound >= 32.f && bound <= 3.0e38f) {
+      int e;
+      (void)frexpf(bound, &e);                                // bound = m 2^e, m in [0.5, 1): S bound in [2^4, 2^5)
+      S = exp2f((float)(5 - e));
+    }
+  }
+  const float kInvS = (1.f / kWScale) / S;                    // exact: powers of two
 
   if (warp > kMmaWarp) {
     // =========================================================================== producers: [noisy || alpha C] -> fp16 hi / lo tiles
@@ -205,7 +220,7 @@ head_fwd_tc_kernel(HeadFwdArgs p) {
           }
           uint32_t hi[4], lo[4];
 #pragma unroll
-          for (int q = 0; q < 4; ++q) split_f16x2_s11(clamp16(v[j][2 * q]), clamp16(v[j][2 * q + 1]), hi[q], lo[q]);
+          for (int q = 0; q < 4; ++q) split_f16x2_s11(clamp16(v[j][2 * q] * S), clamp16(v[j][2 * q + 1] * S), hi[q], lo[q]);
           const int off = tile_b_off(r, c8);
           *reinterpret_cast<uint4*>(ahi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
           *reinterpret_cast<uint4*>(alo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
@@ -262,7 +277,6 @@ head_fwd_tc_kernel(HeadFwdArgs p) {
     const int row = q * 32 + lane;
     const int c0 = half * 32;
     const uint32_t tl = (uint32_t)(q * 32) << 16;
-    constexpr float kInv = 1.f / kWScale;
     auto epi1 = [&](int i) {
       const int s = i & 1, use = i >> 1;
       const int gv = tile_base(i) + row;
@@ -280,7 +294,7 @@ head_fwd_tc_kernel(HeadFwdArgs p) {
         __syncwarp();
         if (lane == 0) mbar_arrive(&bars[B_E2 + s]);           // the stage's TMEM columns may be overwritten by its next tile
 #pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = fmaf(fmaf(v2[j], kLoScale, v[j]), kInv, s_b1[c0 + j]);
+        for (int j = 0; j < 32; ++j) v[j] = fmaf(fmaf(v2[j], kLoScale, v[j]), kInvS, s_b1[c0 + j]);
         if (gv < p.N) {
 #pragma unroll
           for (int j = 0; j < 4; ++j) st8(p.Z + (size_t)gv * HID + c0 + 8 * j, v + 8 * j);
@@ -288,10 +302,10 @@ head_fwd_tc_kernel(HeadFwdArgs p) {
         return;
       }
 #pragma unroll
-      for (int j = 0; j < 32; ++j) v[j] = fmaxf(fmaf(fmaf(v2[j], kLoScale, v[j]), kInv, s_b1[c0 + j]), 0.f);
+      for (int j = 0; j < 32; ++j) v[j] = fmaxf(fmaf(fmaf(v2[j], kLoScale, v[j]), kInvS, s_b1[c0 + j]), 0.f);
       uint32_t hi[16], lo[16];
 #pragma unroll
-      for (int j = 0; j < 16; ++j) split_f16x2_s11(fminf(v[2 * j], 65504.f), fminf(v[2 * j + 1], 65504.f), hi[j], lo[j]);
+      for (int j = 0; j < 16; ++j) split_f16x2_s11(fminf(v[2 * j] * S, 65504.f), fminf(v[2 * j + 1] * S, 65504.f), hi[j], lo[j]);
       tmem_st16u(t0 + kColR + c0 / 2, hi);
       tmem_st16u(t0 + kColR + 32 + c0 / 2, lo);
       if (p.r && gv < p.N) {
@@ -326,7 +340,7 @@ head_fwd_tc_kernel(HeadFwdArgs p) {
       __syncwarp();
       if (lane == 0) mbar_arrive(&bars[B_E2 + s]);           // the stage's TMEM columns may be overwritten by its next tile
 #pragma unroll
-      for (int j = 0; j < 32; ++j) y[j] = fmaf(fmaf(y2[j], kLoScale, y[j]), kInv, s_b2[c0 + j]);
+      for (int j = 0; j < 32; ++j) y[j] = fmaf(fmaf(y2[j], kLoScale, y[j]), kInvS, s_b2[c0 + j]);
       if (gv < p.N) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) st8(p.Z + (size_t)gv * HID + c0 + 8 * j, y + 8 * j);

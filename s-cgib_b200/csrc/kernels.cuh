@@ -240,6 +240,8 @@ struct HeadFwdArgs {
   const float* bn = nullptr;                    // head_tc.cu GATE mode only: {mean, rstd, gamma, beta}[HID] of the producing layer
   const float *W1n = nullptr, *W2n = nullptr;   // natural [HID][2*HID], [HID][HID]: when set (hidden 64, fp32 saves) the tensor-core
                                                 //  kernel head_tc.cu runs instead of the FFMA tiles
+  const unsigned int* xmax = nullptr;           // head_tc.cu: optional device slots {max |noisy|, max |C|, max |alpha|} (float bits,
+                                                //  launch_absmax): inputs beyond 2^5 are pre-scaled by a power of two (see head_tc.cu)
 };
 void launch_head_fwd(const HeadFwdArgs& a, int hidden, cudaStream_t s);
 void launch_head_fwd_tc(const HeadFwdArgs& a, cudaStream_t s);
