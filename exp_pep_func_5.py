@@ -181,7 +181,7 @@ def build_parser():
     # additions of the B200 port (not in the reference)
     parser.add_argument("--gin_layers", type=int, default=4, help="GINConv per encoder (4 in the published models.py)")
     parser.add_argument("--device_loader", type=int, default=1, help="1: splits resident in HBM + GPU-side batch assembly; 0: torch DataLoader + collate")
-    parser.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"], help="bf16 = bf16 activations in the GIN encoders (see exp_pretraining.py)")
+    parser.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"], help="bf16 = bf16 activations inside the GIN / GraphSAGE / GCN encoders (see exp_pretraining.py)")
     parser.add_argument("--engine_loop", type=int, default=1, help="pre-training stage: epoch through the engine API (see exp_pretraining.py)")
     parser.add_argument("--synthetic", type=int, default=512, help="synthetic molecules when pts/<dataset>_csr.pt is absent")
     return parser

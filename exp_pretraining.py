@@ -264,7 +264,7 @@ def build_parser():
     parser.add_argument("--file_name", default="outputs_excels.xlsx", help="file_name dataset")
     # additions of the B200 port (not in the reference)
     parser.add_argument("--gin_layers", type=int, default=4, help="GINConv per encoder (4 in the published models.py; 5 = paper / shipped checkpoint)")
-    parser.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"], help="fp32 = reference precision; bf16 = bf16 activations + single-pass bf16 tensor-core MLPs in the GIN encoders (parameters / optimiser stay fp32)")
+    parser.add_argument("--dtype", default="fp32", choices=["fp32", "bf16"], help="fp32 = reference precision; bf16 = bf16 activations inside the encoders, on single-pass bf16 tensor-core products (the GIN MLPs; the GraphSAGE / GCN linear layers and their weight gradients); parameters / optimiser stay fp32")
     parser.add_argument("--engine_loop", type=int, default=1, help="1: drive the epoch through the engine API (prefetch stream, one host read per epoch); 0: the reference's loop body")
     parser.add_argument("--device_loader", type=int, default=1, help="1: datasets resident in HBM + GPU-side batch assembly (DeviceLoader); 0: torch DataLoader + collate as in the reference")
     parser.add_argument("--synthetic", type=int, default=2048, help="synthetic molecules per dataset when pts/<name>_csr.pt is absent")

@@ -418,6 +418,35 @@ SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32_t normaliz
                                      const int32_t* indptr1, const int32_t* indices1, const int32_t* map1, float* dWt,
                                      void* workspace, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * The same building blocks in bf16 mode (--dtype bf16; csrc/encoder_bf16.cu): activations, masks and layer gradients are
+ * bf16 storage (raw 16-bit words), weights / bias / dW / db fp32; every sum is fp32.  All data pointers 16-byte aligned
+ * (SCGIB_E_ALIGN), widths in {32, 64, 128, 256} (SCGIB_E_SHAPE), V >= 1 (SCGIB_E_RANGE); checked before any launch.
+ *
+ *  scgib_input_proj_fwd_bf16  : scgib_input_proj_fwd_f32 with the [N][32] output rounded to bf16.
+ *  scgib_f32_to_bf16          : out = rnd(in), n a multiple of 8.
+ *  scgib_graph_aggregate_bf16 : scgib_graph_aggregate_f32 on bf16 in / add; out bf16, or fp32 when out_f32.
+ *  scgib_linear_fwd_bf16      : scgib_linear_fwd_f32 on bf16 Xp / Mp, single-pass tcgen05 MMAs with the weights rounded to
+ *      bf16 and an fp32 accumulator; Y bf16, or fp32 when y_f32.  The weights and one 128-row tile per pair live in shared
+ *      memory: a pair of wide operands beyond 227 KB (e.g. K0 = K1 = 256 at O = 256) is SCGIB_E_SHAPE.
+ *  scgib_linear_bwd_w_bf16    : scgib_linear_bwd_w_f32 on bf16 G / M / X (O in {64, 128, 256}); the row contraction runs on
+ *      tcgen05; workspace from scgib_linear_bwd_w_bf16_workspace_bytes.
+ * ------------------------------------------------------------------------------------------ */
+SCGIB_API int scgib_input_proj_fwd_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t, void* stream);
+SCGIB_API int scgib_f32_to_bf16(const float* in, int64_t n, void* out, void* stream);
+SCGIB_API int scgib_graph_aggregate_bf16(const void* in, int32_t W, const int32_t* row_map, const int32_t* indptr,
+                                         const int32_t* indices, int32_t V, int32_t src_norm, int32_t dst_norm,
+                                         const void* add, void* out, int32_t out_f32, void* stream);
+SCGIB_API int scgib_linear_fwd_bf16(const void* X0, const void* M0, const int32_t* map0, const float* W0, int32_t K0,
+                                    int32_t w0_kxo, const void* X1, const void* M1, const float* W1, int32_t K1,
+                                    int32_t w1_kxo, const float* bias, int32_t relu, int32_t V, int32_t O, void* Y,
+                                    int32_t y_f32, void* stream);
+SCGIB_API size_t scgib_linear_bwd_w_bf16_workspace_bytes(int32_t V, int32_t O, int32_t K);
+SCGIB_API int scgib_linear_bwd_w_bf16(const void* G, const void* M, const void* X, const int32_t* map, int32_t V, int32_t O,
+                                      int32_t K, int32_t kxo, int32_t accumulate, float* dW, float* db, void* workspace,
+                                      size_t workspace_bytes, void* stream);
+
+
 /* Debugging aid: byte offset of a named intermediate inside the pre-training workspace ("t", "H", "q", "C",
  * "alpha", "lam", "y<enc>_<layer>", "gH", ...), -1 if unknown.  Tests compare intermediates with the oracle. */
 SCGIB_API int64_t scgib_pretrain_workspace_offset(const ScgibDims* d, int32_t B, int32_t N, int32_t E, int32_t Ns,

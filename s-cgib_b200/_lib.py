@@ -123,6 +123,15 @@ _SIGNATURES = {
     "scgib_transfer_bwd_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
     "scgib_transfer_bwd_f32": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "scgib_input_proj_fwd_bf16": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    "scgib_f32_to_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
+    "scgib_graph_aggregate_bf16": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p,
+                                           c_void_p, c_int32, c_void_p]),
+    "scgib_linear_fwd_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                      c_int32, c_int32, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p]),
+    "scgib_linear_bwd_w_bf16_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "scgib_linear_bwd_w_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32,
+                                        c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "scgib_profile_enable": (None, [c_int]),
     "scgib_profile_count": (c_int, []),
     "scgib_profile_get": (c_int, [c_int, POINTER(c_char_p), POINTER(c_float)]),

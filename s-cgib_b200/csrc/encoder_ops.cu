@@ -11,6 +11,7 @@
 //
 // These layers are plain FP32 FFMA tiles (the host composes them per layer; s-cgib_b200/encoders.py): the tensor-core
 // pipeline of this library is built around the GIN layer (gin_tc3.cu / gin_bwd_h.cu), which the CLI default selects.
+// --dtype bf16 runs the same operators on bf16 activations with tcgen05 products: encoder_bf16.cu.
 #include "kernels.cuh"
 #include "../../include/scgib.h"
 
@@ -256,6 +257,13 @@ void launch_linear_plain(const float* X, const float* W, const float* bias, int 
   launch_k((linear_fwd_kernel), dim3((V + LTM - 1) / LTM, O / LTN), dim3(kThreads), 0, s, a);
 }
 
+void launch_linear_bwd_w_reduce(const float* part, int chunks, int O, int K, int kxo, int accumulate, float* dW, float* db,
+                                cudaStream_t s) {
+  const int n = O * K + O;
+  launch_k((linear_bwd_w_reduce_kernel), dim3(min((n + kThreads - 1) / kThreads, 4 * num_sms())), dim3(kThreads), 0, s,
+           part, chunks, O, K, kxo, accumulate, dW, db);
+}
+
 // row chunks of the weight-gradient reduction: enough (chunks x output tiles) CTAs for two per SM, at least 256 rows per chunk
 static int bwd_w_chunks(int V, int O, int K) {
   int tiles = (O / WT) * ((K + WT - 1) / WT);
@@ -340,8 +348,6 @@ extern "C" SCGIB_API int scgib_linear_bwd_w_f32(const float* G, const float* M, 
   const int chunks = bwd_w_chunks(V, O, K);
   LinearBwdWArgs a{G, M, X, map, V, O, K, ((V + chunks - 1) / chunks + WR - 1) / WR * WR, (float*)workspace};
   launch_k((linear_bwd_w_kernel), dim3(chunks, O / WT, (K + WT - 1) / WT), dim3(kThreads), 0, s, a);
-  const int n = O * K + O;
-  launch_k((linear_bwd_w_reduce_kernel), dim3(min((n + kThreads - 1) / kThreads, 4 * num_sms())), dim3(kThreads), 0, s,
-           (const float*)workspace, chunks, O, K, kxo, accumulate, dW, db);
+  launch_linear_bwd_w_reduce((const float*)workspace, chunks, O, K, kxo, accumulate, dW, db, s);
   return (int)cudaGetLastError();
 }

@@ -139,6 +139,10 @@ void launch_input_proj_bwd(const InputProjBwdArgs& a, cudaStream_t s);
 // ---------------------------------------------------------------- encoder_ops.cu
 // Y[V][O] = X[V][K] W^T + bias, W [O][K] (nn.Linear layout); K, O multiples of 32
 void launch_linear_plain(const float* X, const float* W, const float* bias, int V, int K, int O, float* Y, cudaStream_t s);
+// dW (+)= / db (+)= the fixed-order sum of `chunks` partials [chunks][O*K + O] (dW part [o][k]; kxo: dW stored [K][O]);
+// shared by the fp32 and the bf16 (encoder_bf16.cu) weight-gradient entries
+void launch_linear_bwd_w_reduce(const float* part, int chunks, int O, int K, int kxo, int accumulate, float* dW, float* db,
+                                cudaStream_t s);
 
 // ---------------------------------------------------------------- head_kernels.cu
 // H = relu(BN(y_last)) materialised; q = H Wc1^T + bc1   (compressor.0, models.py:590)

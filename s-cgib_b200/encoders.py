@@ -7,6 +7,12 @@ core-candidate attention, head MLP, the two batch losses, the transfer_d backwar
 launches and keeps the saved activations: no torch kernels compute anything on this path except the final scaling of the
 parameter gradients by the upstream loss gradient, and nothing falls back to torch or the CPU.
 
+bf16 mode (``act_dtype == "bf16"`` on the outer module, --dtype bf16): the encoders follow the dtype of their input ``t``.  A
+bf16 ``t`` keeps every tensor inside the two encoders in bf16 (the aggregated inputs, the layer outputs, the layer
+gradients and the backward products) and runs the tcgen05 linear layers of csrc/encoder_bf16.cu; the encoder output h3
+and the input gradient g_t stay fp32, as do everything after the encoders and every parameter and gradient.  The
+rounding points are listed in DESIGN §3.5.
+
 The parameter containers reproduce DGL 1.1.x's state-dict keys and default initialisation (``convN.fc_self.weight`` /
 ``convN.fc_neigh.weight`` / ``convN.fc_self.bias`` for SAGEConv, ``convN.weight`` [in, out] / ``convN.bias`` for GraphConv), so a
 reference checkpoint loads unchanged.  DGL itself is not available offline: its semantics are restated
@@ -21,6 +27,11 @@ from . import ops
 from .ops import NORM_MEAN, NORM_NONE, NORM_SQRT
 
 DTR = 32
+
+
+def _f32_out(x):
+    """keyword of the operators that leave the encoders (h3, g_t): fp32 output when the encoder runs in bf16."""
+    return {"out_dtype": torch.float32} if x.dtype == torch.bfloat16 else {}
 
 
 # ---------------------------------------------------------------------------------------------- parameter containers
@@ -60,7 +71,7 @@ class GraphSAGE(nn.Module):
         m1 = agg(h1)
         h2 = ops.linear_fwd(h1, c2.fc_self.weight, H, X1=m1, W1=c2.fc_neigh.weight, bias=c2.fc_self.bias, relu=True)
         m2 = agg(h2)
-        h3 = ops.linear_fwd(h2, c2.fc_self.weight, H, X1=m2, W1=c2.fc_neigh.weight, bias=c2.fc_self.bias, relu=False)
+        h3 = ops.linear_fwd(h2, c2.fc_self.weight, H, X1=m2, W1=c2.fc_neigh.weight, bias=c2.fc_self.bias, relu=False, **_f32_out(t))
         return h3, (t, row_map, indptr, indices, m0, h1, m1, h2, m2)
 
     def run_backward(self, saved, g_out, weights=True):
@@ -73,12 +84,14 @@ class GraphSAGE(nn.Module):
         dWs1, dWn1, db1 = new(H, self.in_feats), new(H, self.in_feats), new(H)
         dWs2, dWn2, db2 = new(H, H), new(H, H), new(H)
         bwd_w = ops.linear_bwd_w if weights else (lambda *a, **k: None)
-        aggT = lambda u, add: ops.graph_aggregate(u, indptr, indices, NORM_MEAN, NORM_NONE, add=add)
+        aggT = lambda u, add, **od: ops.graph_aggregate(u, indptr, indices, NORM_MEAN, NORM_NONE, add=add, **od)
+        if h1.dtype == torch.bfloat16:
+            g_out = ops.to_bf16(g_out)
 
-        def through(g, mask, conv, width):      # gradient wrt the layer input: g Ws + A^T(g Wn), g masked by the layer's ReLU
+        def through(g, mask, conv, width, **od):     # gradient wrt the layer input: g Ws + A^T(g Wn), g masked by the layer's ReLU
             u = ops.linear_fwd(g, conv.fc_neigh.weight, width, w0_kxo=True, M0=mask)
             gs = ops.linear_fwd(g, conv.fc_self.weight, width, w0_kxo=True, M0=mask)
-            return aggT(u, gs)
+            return aggT(u, gs, **od)
 
         # third layer: conv2 without ReLU
         bwd_w(g_out, h2, dWs2, db2)
@@ -91,7 +104,7 @@ class GraphSAGE(nn.Module):
         # first layer: conv1 on the gathered t rows
         bwd_w(g_h1, t, dWs1, db1, M=h1, map=row_map)
         bwd_w(g_h1, m0, dWn1, M=h1)
-        g_t = through(g_h1, h1, c1, self.in_feats)
+        g_t = through(g_h1, h1, c1, self.in_feats, **_f32_out(h1))
         if not weights:
             return g_t, {}
         return g_t, {"conv1.fc_self.weight": dWs1, "conv1.fc_neigh.weight": dWn1, "conv1.fc_self.bias": db1,
@@ -127,14 +140,16 @@ class GCN(nn.Module):
         a1 = agg(h1)
         h2 = ops.linear_fwd(a1, self.conv2.weight, 2 * H, w0_kxo=True, bias=self.conv2.bias, relu=True)
         a2 = agg(h2)
-        h3 = ops.linear_fwd(a2, self.conv3.weight, H, w0_kxo=True, bias=self.conv3.bias, relu=False)
+        h3 = ops.linear_fwd(a2, self.conv3.weight, H, w0_kxo=True, bias=self.conv3.bias, relu=False, **_f32_out(t))
         return h3, (indptr, indices, a0, h1, a1, h2, a2)
 
     def run_backward(self, saved, g_out, weights=True):
         indptr, indices, a0, h1, a1, h2, a2 = saved
         H, dev = self.hidden_dim, g_out.device
         new = lambda *s: torch.empty(*s, device=dev)
-        agg = lambda h: ops.graph_aggregate(h, indptr, indices, NORM_SQRT, NORM_SQRT)       # self-adjoint on the symmetric CSR
+        agg = lambda h, **od: ops.graph_aggregate(h, indptr, indices, NORM_SQRT, NORM_SQRT, **od)   # self-adjoint on the CSR
+        if h1.dtype == torch.bfloat16:
+            g_out = ops.to_bf16(g_out)
         dW1, db1 = new(self.in_feats, 2 * H), new(2 * H)
         dW2, db2 = new(2 * H, 2 * H), new(2 * H)
         dW3, db3 = new(2 * H, H), new(H)
@@ -144,7 +159,7 @@ class GCN(nn.Module):
         bwd_w(g_h2, a1, dW2, db2, M=h2, kxo=True)
         g_h1 = agg(ops.linear_fwd(g_h2, self.conv2.weight, 2 * H, M0=h2))
         bwd_w(g_h1, a0, dW1, db1, M=h1, kxo=True)
-        g_t = agg(ops.linear_fwd(g_h1, self.conv1.weight, self.in_feats, M0=h1))
+        g_t = agg(ops.linear_fwd(g_h1, self.conv1.weight, self.in_feats, M0=h1), **_f32_out(h1))
         if not weights:
             return g_t, {}
         return g_t, {"conv1.weight": dW1, "conv1.bias": db1, "conv2.weight": dW2, "conv2.bias": db2,
@@ -162,6 +177,18 @@ def make_encoder(encoder, in_dim, hidden_dim):
 # ---------------------------------------------------------------------------------------------- the composed step
 def _f(t):
     return t.detach().contiguous().float()
+
+
+def act_dtype(outer):
+    """torch dtype of the activations inside the encoders: the outer module's own --dtype (its ``act_dtype``)."""
+    return torch.bfloat16 if getattr(outer, "act_dtype", "fp32") == "bf16" else torch.float32
+
+
+def _input_proj(outer, x):
+    """transfer_d(F.normalize(x)), written in bf16 directly in bf16 mode."""
+    if act_dtype(outer) == torch.bfloat16:
+        return ops.input_proj(x, _f(outer.transfer_d.weight), torch.bfloat16)
+    return ops.input_proj(x, _f(outer.transfer_d.weight))
 
 
 def inner_of(model):
@@ -183,6 +210,8 @@ def composed_features(outer, g, ego, t, gate_u, feat_u):
     and everything the backward needs."""
     model = inner_of(outer)
     Hd = int(outer.hidden_dim)
+    if act_dtype(outer) == torch.bfloat16 and t.dtype != torch.bfloat16:
+        t = ops.to_bf16(t)
     Hf, sv1 = model.Encoder1.run_forward(t, g.indptr, g.indices)
     S, sv2 = model.Encoder2.run_forward(t, ego.sub_indptr, ego.sub_indices, row_map=ego.ego_nodes)
     c = model.compressor
@@ -256,7 +285,7 @@ class ComposedPretrainFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, model, g, ego, x, gate_u, feat_u, names, *params):
-        t = ops.input_proj(x, _f(model.transfer_d.weight))                 # F.normalize + transfer_d (idempotent on normalised x)
+        t = _input_proj(model, x)                                          # F.normalize + transfer_d (idempotent on normalised x)
         out, st = composed_features(model, g, ego, t, gate_u, feat_u)
         if getattr(model, "recons_type", "adj") == "logM":                 # models.py:693-694: k-step log transition matrices
             rec, gZ, _ = ops.recon_logm(out["Z"], g.graph_ptr, g.indptr, g.indices, int(model.k_transition), 1.0)
@@ -301,7 +330,7 @@ class ComposedFinetuneFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, owner, g, ego, x, gate_u, feat_u, names, *params):
         head = owner._head
-        t = ops.input_proj(x, _f(owner.transfer_d.weight))
+        t = _input_proj(owner, x)
         out, st = composed_features(owner, g, ego, t, gate_u, feat_u)
         scores = head.forward(out["Z"], g.graph_ptr)
         st.update(x=x, g=g, ego=ego)
@@ -333,7 +362,7 @@ class ComposedDomainAdaptFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, owner, g, ego, x, gate_u, feat_u, x_norm, names, *params):
         head, rev = owner._head, owner._rev
-        t = ops.input_proj(x, _f(owner.transfer_d.weight))
+        t = _input_proj(owner, x)
         out, st = composed_features(owner, g, ego, t, gate_u, feat_u)
         rec = head.forward(out["Z"], g.graph_ptr)
         org = rev.forward(x_norm, g.graph_ptr)

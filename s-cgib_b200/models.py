@@ -366,7 +366,7 @@ class Mainmodel(_HotPathMixin, nn.Module):
         self.hidden_dim = hidden_dim
         self.k_transition = k_transition
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
-        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations in the GIN encoders (--dtype bf16)
+        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations inside the encoders (--dtype bf16)
         self.in_dim_raw = in_dim
         self.fc1 = nn.Linear(hidden_dim, 1)
         self.in_dim = args.d_transfer
@@ -415,7 +415,7 @@ class Mainmodel_continue(_HotPathMixin, nn.Module):
         self.tau = 1.0
         self.readout = args.readout_f
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
-        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations in the GIN encoders (--dtype bf16)
+        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations inside the encoders (--dtype bf16)
         self.in_dim_raw = in_dim
         self.s2s = _Set2SetParams(hidden_dim, 2, 1)
         self.s2s_rev = _Set2SetParams(in_dim, 2, 1)
@@ -500,7 +500,7 @@ class Mainmodel_finetuning(nn.Module):
         self.dataset = args.dataset
         self.readout = args.readout_f
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
-        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations in the GIN encoders (--dtype bf16)
+        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations inside the encoders (--dtype bf16)
         self.in_dim_raw = in_dim
         self.s2s = _Set2SetParams(hidden_dim, 2, 1)
         self.in_dim = args.d_transfer
@@ -667,7 +667,7 @@ class Mainmodel_domainadapt(nn.Module):
         self.tau = 1.0
         self.readout = args.readout_f
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
-        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations in the GIN encoders (--dtype bf16)
+        self.act_dtype = getattr(args, "dtype", "fp32")      # "bf16": bf16 activations inside the encoders (--dtype bf16)
         self.in_dim_raw = in_dim
         self.s2s = _Set2SetParams(hidden_dim, 2, 1)
         self.s2s_rev = _Set2SetParams(in_dim, 2, 1)

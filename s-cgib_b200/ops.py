@@ -21,14 +21,23 @@ def _cuda(*ts):
             raise RuntimeError("scgib_b200 ops need CUDA tensors (no CPU fallback)")
 
 
-def input_proj(x: torch.Tensor, Wt: torch.Tensor) -> torch.Tensor:
-    """transfer_d(F.normalize(x))  (exp_pretraining.py:312, models.py:668)."""
+def input_proj(x: torch.Tensor, Wt: torch.Tensor, out_dtype=torch.float32) -> torch.Tensor:
+    """transfer_d(F.normalize(x))  (exp_pretraining.py:312, models.py:668); ``out_dtype`` torch.bfloat16 rounds the output."""
     _cuda(x, Wt)
     x, Wt = x.contiguous().float(), Wt.contiguous().float()
-    t = torch.empty(x.shape[0], DTR, device=x.device)
-    _lib.check(_lib.load().scgib_input_proj_fwd_f32(_lib.ptr(x), _lib.ptr(Wt), x.shape[0], x.shape[1], Wt.shape[0],
-                                                    _lib.ptr(t), _stream(x)), "input_proj_fwd")
+    t = torch.empty(x.shape[0], DTR, device=x.device, dtype=out_dtype)
+    entry = _lib.load().scgib_input_proj_fwd_bf16 if out_dtype == torch.bfloat16 else _lib.load().scgib_input_proj_fwd_f32
+    _lib.check(entry(_lib.ptr(x), _lib.ptr(Wt), x.shape[0], x.shape[1], Wt.shape[0], _lib.ptr(t), _stream(x)), "input_proj_fwd")
     return t
+
+
+def to_bf16(t: torch.Tensor) -> torch.Tensor:
+    """round an fp32 tensor (numel a multiple of 8) to bf16 on the device."""
+    _cuda(t)
+    t = _c32(t)
+    out = torch.empty(t.shape, device=t.device, dtype=torch.bfloat16)
+    _lib.check(_lib.load().scgib_f32_to_bf16(_lib.ptr(t), t.numel(), _lib.ptr(out), _stream(t)), "f32_to_bf16")
+    return out
 
 
 def gin_layer_fwd(h, indptr, indices, W1, b1, W2, b2, row_map=None, bn_in=None, running=None, save=False):
@@ -268,10 +277,29 @@ def segment_sum_bwd(g_out, seg_ptr, rows):
 NORM_NONE, NORM_MEAN, NORM_SQRT = 0, 1, 2
 
 
-def graph_aggregate(h, indptr, indices, src_norm, dst_norm, row_map=None, add=None):
+def _b16(t):
+    """contiguous bf16 operand of the bf16-mode entries (csrc/encoder_bf16.cu); refuses other dtypes."""
+    if t is None:
+        return None
+    if t.dtype != torch.bfloat16:
+        raise TypeError("bf16-mode operator: every activation operand must be torch.bfloat16, got %s" % t.dtype)
+    return t.detach().contiguous()
+
+
+def graph_aggregate(h, indptr, indices, src_norm, dst_norm, row_map=None, add=None, out_dtype=None):
     """out[v] = (add[v]) + fd(deg v) sum_{u in N(v)} fs(deg u) h[map(u)]; the SAGEConv mean (NONE, MEAN), its backward
-    (MEAN, NONE) and the GraphConv normalised sum (SQRT, SQRT; self-adjoint) on the symmetric CSR."""
+    (MEAN, NONE) and the GraphConv normalised sum (SQRT, SQRT; self-adjoint) on the symmetric CSR.
+    A torch.bfloat16 ``h`` (and ``add``) runs the bf16-mode kernel: output bf16, or fp32 with ``out_dtype=torch.float32``."""
     _cuda(h, indptr, indices)
+    if h.dtype == torch.bfloat16:
+        h, add = _b16(h), _b16(add)
+        V, W = indptr.numel() - 1, h.shape[1]
+        od = torch.bfloat16 if out_dtype is None else out_dtype
+        out = torch.empty(V, W, device=h.device, dtype=od)
+        _lib.check(_lib.load().scgib_graph_aggregate_bf16(_lib.ptr(h), W, _lib.ptr(row_map), _lib.ptr(indptr), _lib.ptr(indices), V,
+                                                          src_norm, dst_norm, _lib.ptr(add), _lib.ptr(out),
+                                                          int(od == torch.float32), _stream(h)), "graph_aggregate_bf16")
+        return out
     h = _c32(h)
     add = None if add is None else _c32(add)
     V, W = indptr.numel() - 1, h.shape[1]
@@ -291,9 +319,23 @@ def segment_sum_w(h, seg_ptr):
     return out
 
 
-def linear_fwd(X0, W0, O, w0_kxo=False, X1=None, W1=None, w1_kxo=False, bias=None, relu=False, map0=None, M0=None, M1=None, V=None):
-    """Y[V,O] = act(X0[map0] (.) (M0 > 0) W0 + X1 (.) (M1 > 0) W1 + bias); W [O,K] (nn.Linear) or [K,O] (w_kxo)."""
+def linear_fwd(X0, W0, O, w0_kxo=False, X1=None, W1=None, w1_kxo=False, bias=None, relu=False, map0=None, M0=None, M1=None, V=None,
+               out_dtype=None):
+    """Y[V,O] = act(X0[map0] (.) (M0 > 0) W0 + X1 (.) (M1 > 0) W1 + bias); W [O,K] (nn.Linear) or [K,O] (w_kxo).
+    A torch.bfloat16 ``X0`` runs the bf16-mode tensor-core kernel (X1, M0, M1 bf16 too; weights and bias fp32): output bf16,
+    or fp32 with ``out_dtype=torch.float32``."""
     _cuda(X0, W0)
+    if X0.dtype == torch.bfloat16:
+        X0, X1, M0, M1 = (_b16(t) for t in (X0, X1, M0, M1))
+        W0, W1, bias = (None if t is None else _c32(t) for t in (W0, W1, bias))
+        V = int(V if V is not None else (map0.numel() if map0 is not None else X0.shape[0]))
+        od = torch.bfloat16 if out_dtype is None else out_dtype
+        Y = torch.empty(V, O, device=X0.device, dtype=od)
+        _lib.check(_lib.load().scgib_linear_fwd_bf16(_lib.ptr(X0), _lib.ptr(M0), _lib.ptr(map0), _lib.ptr(W0), X0.shape[1], int(w0_kxo),
+                                                     _lib.ptr(X1), _lib.ptr(M1), _lib.ptr(W1), 0 if X1 is None else X1.shape[1],
+                                                     int(w1_kxo), _lib.ptr(bias), int(relu), V, O, _lib.ptr(Y),
+                                                     int(od == torch.float32), _stream(X0)), "linear_fwd_bf16")
+        return Y
     X0, W0, X1, W1, bias, M0, M1 = (None if t is None else _c32(t) for t in (X0, W0, X1, W1, bias, M0, M1))
     V = int(V if V is not None else (map0.numel() if map0 is not None else X0.shape[0]))
     Y = torch.empty(V, O, device=X0.device)
@@ -304,10 +346,19 @@ def linear_fwd(X0, W0, O, w0_kxo=False, X1=None, W1=None, w1_kxo=False, bias=Non
 
 
 def linear_bwd_w(G, X, dW, db=None, M=None, map=None, kxo=False, accumulate=False):
-    """dW (+)= (G (.) (M > 0))^T X[map] ([O,K], or [K,O] with kxo), db (+)= column sums; in place on dW / db."""
+    """dW (+)= (G (.) (M > 0))^T X[map] ([O,K], or [K,O] with kxo), db (+)= column sums; in place on dW / db.
+    A torch.bfloat16 ``G`` runs the bf16-mode tensor-core kernel (M, X bf16 too; dW / db stay fp32)."""
     _cuda(G, X, dW)
     if not (dW.is_contiguous() and dW.dtype == torch.float32) or (db is not None and not db.is_contiguous()):
         raise ValueError("linear_bwd_w writes dW / db in place: contiguous fp32 tensors")
+    if G.dtype == torch.bfloat16:
+        G, X, M = _b16(G), _b16(X), _b16(M)
+        lib = _lib.load()
+        V, O, K = G.shape[0], G.shape[1], X.shape[1]
+        ws = _ws(lib.scgib_linear_bwd_w_bf16_workspace_bytes(V, O, K), G.device)
+        _lib.check(lib.scgib_linear_bwd_w_bf16(_lib.ptr(G), _lib.ptr(M), _lib.ptr(X), _lib.ptr(map), V, O, K, int(kxo), int(accumulate),
+                                               _lib.ptr(dW), _lib.ptr(db), _lib.ptr(ws), ws.numel(), _stream(G)), "linear_bwd_w_bf16")
+        return dW, db
     G, X, M = _c32(G), _c32(X), None if M is None else _c32(M)
     lib = _lib.load()
     V, O, K = G.shape[0], G.shape[1], X.shape[1]
