@@ -131,6 +131,7 @@ def load_graphdataset(dataset_name):
     samples_all = []
     if os.path.exists(path):
         big, _ = load_shard(path)             # written by scgib_b200.graph.pack_shard from PyG-style (edge_index, x, y)
+        args.num_features = int(big.ndata["x"].shape[1])      # the shard's own feature width (e.g. NCI1 37, DD 89)
     else:
         print("[I] %s not found: generating %d synthetic molecules of the %s shape" % (path, args.synthetic, dataset_name))
         big = synth_batch(zlib.crc32(dataset_name.encode()) % 1000, args.synthetic)     # the same molecules in every process

@@ -37,7 +37,7 @@ extern "C" {
 enum {
   SCGIB_OK = 0,
   SCGIB_E_NULL = -1,      /* required pointer is NULL */
-  SCGIB_E_SHAPE = -2,     /* unsupported dimension (hidden must be 64 or 128, d_transfer 32, 1 <= L <= 8, F <= 32) */
+  SCGIB_E_SHAPE = -2,     /* unsupported dimension (hidden must be 64 or 128, d_transfer 32, 1 <= L <= 8, 1 <= F <= 128, fine-tuning head C <= 1024) */
   SCGIB_E_ALIGN = -3,     /* pointer not 16-byte aligned */
   SCGIB_E_WORKSPACE = -4, /* workspace too small */
   SCGIB_E_RANGE = -5,     /* size out of range (e.g. k < 1, graph with < 2 nodes) */
@@ -55,7 +55,7 @@ SCGIB_API int scgib_num_sms(void);
  * State-dict names on the reference side are listed in INTEGRATION.md.
  * ------------------------------------------------------------------------------------------ */
 typedef struct ScgibDims {
-  int32_t in_dim;     /* F: raw feature width (9 PCQM4Mv2 / mol-PCBA, 11 QM9)  exp_pretraining.py:219 */
+  int32_t in_dim;     /* F: raw feature width (9 PCQM4Mv2 / mol-PCBA, 11 QM9, 37 NCI1, 89 DD), 1 <= F <= 128  exp_pretraining.py:219 */
   int32_t d_transfer; /* 32                                                      exp_pretraining.py:378 */
   int32_t hidden;     /* 64 or 128 (--dims)                                      exp_pretraining.py:390 */
   int32_t gin_layers; /* L: GINConv per encoder (4 in models.py:57-58)                               */
@@ -220,7 +220,8 @@ SCGIB_API int scgib_extract_forward_f32(const ScgibDims* d, const float* params,
  * r_g = sum alpha_v z_v, q* = [q || r]) -> predict = Linear(2H,H)-ReLU-Linear(H,C) (models.py:386-397) -> sigmoid
  * (models.py:519-520; sigmoid = 0 for the regression datasets, models.py:516-517).  One kernel per direction.
  * head_params / head_grads: one flat fp32 buffer, slots below (scgib_finetune_head_layout gives offsets, each slot
- * padded to 4 floats).  H in {32, 64, 128}, 0 <= C <= 64, T <= 8.  The forward leaves its saved state in `workspace`
+ * padded to 4 floats).  H in {32, 64, 128}, 0 <= C <= 1024 (above 64 the output layer
+ * runs as tiled kernels over [B x C]), T <= 8.  The forward leaves its saved state in `workspace`
  * (scgib_finetune_head_workspace_bytes, 256-byte aligned); the backward must get the same workspace and Z.
  *   fwd: scores [B,C]; optional readout [B,2H] (= q* after the last iteration, the Set2Set output).
  *   bwd: gZ [N,H] (overwritten) = d(<g_scores, scores> + <g_readout, readout>)/dZ; g_readout [B,2H] is optional;
@@ -261,7 +262,7 @@ SCGIB_API int scgib_adam_step_f32(float* params, const float* grads, float* exp_
  * Individual operators (what the autograd Functions of the drop-in modules call; also the
  * unit-test surface).  H = 64.
  * ------------------------------------------------------------------------------------------ */
-/* F.normalize(x) then transfer_d (exp_pretraining.py:312-314, models.py:668): t[N,DT]. */
+/* F.normalize(x) then transfer_d (exp_pretraining.py:312-314, models.py:668): t[N,DT].  1 <= F <= 128. */
 SCGIB_API int scgib_input_proj_fwd_f32(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT,
                              float* t, void* stream);
 
@@ -399,7 +400,7 @@ SCGIB_API int scgib_segment_sum_bwd_f32(const float* g_out, const int32_t* seg_p
  *  scgib_linear_bwd_w_f32    : dW (+)= (G (.) (M > 0))^T X[map] as [O][K] (kxo = 0) or [K][O] (kxo = 1), db (+)= column sums;
  *      fixed-order two-stage reduction (bit-identical reruns).  O multiple of 64.  workspace 16-byte aligned.
  *  scgib_transfer_bwd_f32    : d transfer_d.weight [32][F] = sum over two row sets of g_r (x) xrow_r, xrow_r = x_hat[p(r)]
- *      (+ the x_hat rows of r's neighbours when a CSR is given).  workspace 256-byte aligned.
+ *      (+ the x_hat rows of r's neighbours when a CSR is given).  1 <= F <= 128.  workspace 256-byte aligned.
  * ------------------------------------------------------------------------------------------ */
 SCGIB_API int scgib_graph_aggregate_f32(const float* in, int32_t W, const int32_t* row_map, const int32_t* indptr,
                                         const int32_t* indices, int32_t V, int32_t src_norm, int32_t dst_norm,

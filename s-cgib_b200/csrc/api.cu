@@ -116,7 +116,7 @@ static inline void debug_check(const char* name, cudaStream_t s) {
 
 static bool dims_ok(const ScgibDims* d) {
   return d && (d->hidden == 64 || d->hidden == 128) && d->d_transfer == DTR && d->gin_layers >= 1 && d->gin_layers <= 8 && d->in_dim >= 1 &&
-         d->in_dim <= 32 && (d->act_dtype == SCGIB_ACT_F32 || d->act_dtype == SCGIB_ACT_BF16);
+         d->in_dim <= kMaxInDim && (d->act_dtype == SCGIB_ACT_F32 || d->act_dtype == SCGIB_ACT_BF16);
 }
 
 struct Layout {
@@ -174,14 +174,14 @@ struct Ws {
 
 static inline int xagg_stride(const ScgibDims* d) { return (d->in_dim + 3) / 4 * 4; }
 
-static size_t small_part_floats(int N, int Ns, int HID) {
+static size_t small_part_floats(int N, int Ns, int HID, int F) {
   const int Vmax = N > Ns ? N : Ns;
   size_t a = (size_t)((Vmax + 63) / 64) * 2 * HID;                   // gin fwd tile partials (64-row tiles)
   const size_t a2 = (size_t)num_sms() * 3 * HID * 2;                  // gin_tc2: per-CTA (n, mean, M2) in fp64
   a = a > a2 ? a : a2;
   size_t b = (size_t)(gin_bwd_pre_grid(N + Ns) + 2) * 2 * HID;       // dgamma/dbeta partials (per problem of a shared launch)
   size_t c = (size_t)4 * num_sms() * 5 * HID;                        // gate partials
-  size_t d = (size_t)input_proj_bwd_grid(N, Ns) * DTR * 32;          // transfer_d partials
+  size_t d = input_proj_bwd_part_floats(N, Ns, F);                     // transfer_d partials
   size_t m = a > b ? a : b;
   m = m > c ? m : c;
   return m > d ? m : d;
@@ -211,7 +211,7 @@ static Ws carve(const ScgibDims* d, const Layout& lo, int B, int N, int E, int N
   w.head_w1t = take(2 * HID * HID); w.head_w2t = take(HID * HID); w.comp_w1t = take(HID * HID);
   w.t = take_act((size_t)N * DTR);
   w.cvec[0] = take(2 * HID); w.cvec[1] = take(2 * HID);
-  w.small_part = take(small_part_floats(N, Ns, HID)); w.small_part2 = take(small_part_floats(N, Ns, HID));
+  w.small_part = take(small_part_floats(N, Ns, HID, d->in_dim)); w.small_part2 = take(small_part_floats(N, Ns, HID, d->in_dim));
   w.counters = (unsigned int*)take(64);
   w.H = take((size_t)N * HID); w.q = take((size_t)N * HID); w.C = take((size_t)N * HID);
   w.logit = take(N); w.alpha = take(N); w.lam = take(N);
@@ -270,7 +270,7 @@ extern "C" SCGIB_API const char* scgib_error_string(int code) {
   switch (code) {
     case SCGIB_OK: return "ok";
     case SCGIB_E_NULL: return "required pointer is NULL";
-    case SCGIB_E_SHAPE: return "unsupported dimensions (hidden must be 64 or 128, d_transfer 32, 1 <= gin_layers <= 8, in_dim <= 32; --recons_type logM and the op-level entries: hidden 64)";
+    case SCGIB_E_SHAPE: return "unsupported dimensions (hidden must be 64 or 128, d_transfer 32, 1 <= gin_layers <= 8, 1 <= in_dim <= 128, fine-tuning head outputs C <= 1024; --recons_type logM and the op-level entries: hidden 64)";
     case SCGIB_E_ALIGN: return "pointer not 16-byte aligned";
     case SCGIB_E_WORKSPACE: return "workspace too small";
     case SCGIB_E_RANGE: return "size out of range";
@@ -714,7 +714,8 @@ static FtWs ft_carve(int H, int C, int T, int B, int N, void* base) {
   w.gates = take((size_t)T * B * 4 * H); w.cst = take((size_t)T * B * H); w.qstar = take((size_t)T * B * 2 * H);
   w.alpha = take((size_t)T * N); w.rp = take((size_t)B * H); w.g_pre = take((size_t)B * C); w.g_u = take((size_t)B * H);
   w.dgates = take((size_t)T * B * 4 * H); w.gp = take(N);
-  w.scratch = take((size_t)atb_splits(T * B) * 4 * H * 2 * H);     // row-split partials of the weight-gradient reductions
+  const size_t wmax = (size_t)C * H > (size_t)8 * H * H ? (size_t)C * H : (size_t)8 * H * H;   // dWp2 [C][H] or dWih [4H][2H]
+  w.scratch = take((size_t)atb_splits(T * B) * wmax);     // row-split partials of the weight-gradient reductions
   w.bytes = o;
   return w;
 }
@@ -810,7 +811,7 @@ extern "C" SCGIB_API int scgib_finetune_head_bwd_f32(const float* head_params, i
 // ---------------------------------------------------------------- individual operators
 extern "C" SCGIB_API int scgib_input_proj_fwd_f32(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, float* t, void* stream) {
   if (!x || !Wt || !t) return SCGIB_E_NULL;
-  if (DT != DTR || F < 1 || F > 32) return SCGIB_E_SHAPE;
+  if (DT != DTR || F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
   if (N < 1) return SCGIB_E_RANGE;
   launch_input_proj_fwd(x, Wt, N, F, 1, t, (cudaStream_t)stream);
   return (int)cudaGetLastError();
@@ -820,14 +821,14 @@ extern "C" SCGIB_API int scgib_input_proj_fwd_f32(const float* x, const float* W
 // x_hat rows of r's neighbours when a CSR is given: the layer-0 aggregation backward of the GIN path moved to the features)
 extern "C" SCGIB_API size_t scgib_transfer_bwd_workspace_bytes(int32_t V0, int32_t V1, int32_t F) {
   const size_t xs = (size_t)(F + 3) / 4 * 4;
-  return al((size_t)V0 * xs * 4) + al((size_t)V1 * xs * 4) + al((size_t)input_proj_bwd_grid(V0, V1) * DTR * 32 * 4) + 256;
+  return al((size_t)V0 * xs * 4) + al((size_t)V1 * xs * 4) + al(input_proj_bwd_part_floats(V0, V1, F) * 4) + 256;
 }
 extern "C" SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32_t normalize, const float* g0, int32_t V0,
                                                 const int32_t* indptr0, const int32_t* indices0, const float* g1, int32_t V1,
                                                 const int32_t* indptr1, const int32_t* indices1, const int32_t* map1,
                                                 float* dWt, void* workspace, size_t workspace_bytes, void* stream) {
   if (!x || !g0 || !dWt || !workspace || (V1 > 0 && (!g1 || !map1))) return SCGIB_E_NULL;
-  if (F < 1 || F > 32) return SCGIB_E_SHAPE;
+  if (F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
   if (V0 < 1 || V1 < 0) return SCGIB_E_RANGE;
   if (((uintptr_t)workspace & 255u) != 0) return SCGIB_E_ALIGN;
   if (workspace_bytes < scgib_transfer_bwd_workspace_bytes(V0, V1, F)) return SCGIB_E_WORKSPACE;
@@ -836,7 +837,7 @@ extern "C" SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32
   char* p = (char*)workspace;
   float* xa0 = (float*)p; p += al((size_t)V0 * xs * 4);
   float* xa1 = (float*)p; p += al((size_t)V1 * xs * 4);
-  float* part = (float*)p; p += al((size_t)input_proj_bwd_grid(V0, V1) * DTR * 32 * 4);
+  float* part = (float*)p; p += al(input_proj_bwd_part_floats(V0, V1, F) * 4);
   unsigned int* counter = (unsigned int*)p;
   cudaMemsetAsync(counter, 0, 64, s);
   FwdPrepArgs pa;

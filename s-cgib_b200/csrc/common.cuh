@@ -8,6 +8,8 @@ namespace scgib {
 constexpr int HID = 64;        // hidden width (exp_pretraining.py:390)
 constexpr int DTR = 32;        // d_transfer   (exp_pretraining.py:378)
 constexpr int kThreads = 256;  // CTA size of every tile kernel
+constexpr int kMaxInDim = 128; // widest raw node-feature input (transfer_d, s2s_rev on the H = 128 Set2Set instance)
+constexpr int kMaxClasses = 1024;   // widest fine-tuning head output (C; 2 * kMaxInDim for r_transfer_d)
 constexpr float kBnEps = 1e-5f;
 typedef uint16_t bf16_t;       // raw bfloat16 storage (bf16 mode: activations of the GIN encoders)
 

@@ -355,7 +355,7 @@ static bool al16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
 extern "C" SCGIB_API int scgib_input_proj_fwd_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t,
                                                    void* stream) {
   if (!x || !Wt || !t) return SCGIB_E_NULL;
-  if (DT != DTR || F < 1 || F > 32) return SCGIB_E_SHAPE;
+  if (DT != DTR || F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
   if (N < 1) return SCGIB_E_RANGE;
   if (!al16(t)) return SCGIB_E_ALIGN;
   launch_input_proj_fwd(x, Wt, N, F, 1, reinterpret_cast<float*>(t), (cudaStream_t)stream, true);

@@ -8,12 +8,16 @@
 // (e_v = z_v . q, softmax over the graph, r = sum alpha_v z_v), and after the last iteration the predict MLP.
 // The backward is one per-graph kernel of the same shape (activation gradients, g_Z) followed by small fixed-order
 // A^T B reductions over the graphs for the weight gradients (no float atomics).
+// Heads with more than kMaxC outputs keep everything up to u = relu(Wp1 q* + bp1) in the per-graph kernels; the output
+// layer scores = act(u Wp2^T + bp2) and its backward g_u = relu'(u) * ((g_scores . act') Wp2) run as tiled kernels over
+// [B x C] / [B x H] instead of one Wp2 row per thread.
 #include "kernels.cuh"
 
 namespace scgib {
 
 namespace {
 constexpr int FG = 8;   // graphs per CTA = warps per CTA
+constexpr int kMaxC = 64;   // widest output layer run inside the per-graph kernels (s_gpre of the backward)
 
 __device__ __forceinline__ float sigmoidf_acc(float x) { return 1.f / (1.f + expf(-x)); }
 
@@ -189,6 +193,7 @@ __global__ void __launch_bounds__(kThreads) finetune_head_fwd_kernel(FinetuneHea
     sm.mid[g][c] = u;
     if (g0 + g < B) p.rp[(size_t)(g0 + g) * H + c] = u;
   }
+  if (p.C > kMaxC) return;              // the output layer runs as a tiled kernel (ft_out_fwd_kernel)
   __syncthreads();
   for (int i = threadIdx.x; i < FG * p.C; i += kThreads) {
     const int g = i / p.C, c = i % p.C;
@@ -228,8 +233,6 @@ struct FtBwdSmem {
   float tmp[FG][H];
 };
 
-constexpr int kMaxC = 64;
-
 template <int H>
 __global__ void __launch_bounds__(kThreads) finetune_head_bwd_kernel(FinetuneHeadBwdArgs p) {
   __shared__ FtBwdSmem<H> sm;
@@ -238,7 +241,15 @@ __global__ void __launch_bounds__(kThreads) finetune_head_bwd_kernel(FinetuneHea
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int B = p.B, T = p.T, C = p.C;
   for (int i = threadIdx.x; i < FG * H; i += kThreads) { (&sm.gh[0][0])[i] = 0.f; (&sm.gc[0][0])[i] = 0.f; }
-  if (C > 0) {
+  if (C > kMaxC) {
+    // ---- predict backward from g_u (masked, written by ft_out_bwd_kernel)
+    for (int i = threadIdx.x; i < FG * H; i += kThreads) {
+      const int g = i / H, c = i % H;
+      sm.tmp[g][c] = g0 + g < B ? p.g_u[(size_t)(g0 + g) * H + c] : 0.f;
+    }
+    __syncthreads();
+    matvec_natural(p.Wp1, H, 2 * H, &sm.tmp[0][0], H, &sm.gq[0][0], 2 * H);    // g wrt q*_{T-1}
+  } else if (C > 0) {
     // ---- predict backward
     for (int i = threadIdx.x; i < FG * C; i += kThreads) {
       const int g = i / C, c = i % C;
@@ -387,6 +398,121 @@ __global__ void __launch_bounds__(kThreads) finetune_head_bwd_kernel(FinetuneHea
   }
 }
 
+// Output layer of heads with C > kMaxC.  A CTA owns a tile of RI * 16 graphs x 64 columns; thread (tx, ty) of the
+// 16 x 16 grid owns graphs ty + 16 i and columns tx + 16 j (coalesced stores).  Operands go through shared memory in
+// k-major chunks of 32.  Each output is a sequential fmaf chain over k (over c in the backward) from the bias (from 0),
+// the order of the in-kernel path.
+constexpr int OT = 64, OK = 32;
+
+// scores[b][c] = act(bp2[c] + sum_k rp[b][k] Wp2[c][k])
+__global__ void __launch_bounds__(kThreads) ft_out_fwd_kernel(const float* __restrict__ rp, const float* __restrict__ Wp2,
+                                                              const float* __restrict__ bp2, int B, int C, int H, int sigmoid,
+                                                              float* __restrict__ scores) {
+  constexpr int RI = 4;
+  __shared__ float sa[OK][RI * 16 + 1], sw[OK][OT + 1];     // [k][graph], [k][class]
+  const int g0 = blockIdx.y * RI * 16, c0 = blockIdx.x * OT;
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  float acc[RI][4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int c = c0 + tx + 16 * j;
+    const float b = c < C ? __ldg(bp2 + c) : 0.f;
+#pragma unroll
+    for (int i = 0; i < RI; ++i) acc[i][j] = b;
+  }
+  for (int k0 = 0; k0 < H; k0 += OK) {
+    __syncthreads();
+    for (int e = threadIdx.x; e < RI * 16 * OK; e += kThreads) {
+      const int r = e / OK, k = e % OK;
+      sa[k][r] = g0 + r < B ? __ldg(rp + (size_t)(g0 + r) * H + k0 + k) : 0.f;
+    }
+    for (int e = threadIdx.x; e < OT * OK; e += kThreads) {
+      const int r = e / OK, k = e % OK;
+      sw[k][r] = c0 + r < C ? __ldg(Wp2 + (size_t)(c0 + r) * H + k0 + k) : 0.f;
+    }
+    __syncthreads();
+#pragma unroll 8
+    for (int k = 0; k < OK; ++k) {
+      float a[RI], w[4];
+#pragma unroll
+      for (int i = 0; i < RI; ++i) a[i] = sa[k][ty + 16 * i];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) w[j] = sw[k][tx + 16 * j];
+#pragma unroll
+      for (int i = 0; i < RI; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(w[j], a[i], acc[i][j]);
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < RI; ++i) {
+    const int g = g0 + ty + 16 * i;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int c = c0 + tx + 16 * j;
+      if (g < B && c < C) scores[(size_t)g * C + c] = sigmoid ? sigmoidf_acc(acc[i][j]) : acc[i][j];
+    }
+  }
+}
+
+// g_pre[b][c] = g_scores[b][c] * act'(scores[b][c])  (written by the CTAs of the first column tile);
+// g_u[b][k] = rp[b][k] > 0 ? sum_c g_pre[b][c] Wp2[c][k] : 0
+__global__ void __launch_bounds__(kThreads) ft_out_bwd_kernel(const float* __restrict__ rp, const float* __restrict__ Wp2,
+                                                              const float* __restrict__ scores, const float* __restrict__ g_scores,
+                                                              int B, int C, int H, int sigmoid, float* __restrict__ g_pre,
+                                                              float* __restrict__ g_u) {
+  constexpr int RI = 2;
+  __shared__ float sg[OK][RI * 16 + 1], sw[OK][OT + 1];     // [c][graph], [c][k]
+  const int g0 = blockIdx.y * RI * 16, k0 = blockIdx.x * OT;
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  const bool write_pre = blockIdx.x == 0;
+  float acc[RI][4];
+#pragma unroll
+  for (int i = 0; i < RI; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+  for (int cb = 0; cb < C; cb += OK) {
+    __syncthreads();
+    for (int e = threadIdx.x; e < RI * 16 * OK; e += kThreads) {
+      const int r = e / OK, c = e % OK;
+      const int g = g0 + r, cc = cb + c;
+      float v = 0.f;
+      if (g < B && cc < C) {
+        v = __ldg(g_scores + (size_t)g * C + cc);
+        if (sigmoid) { const float sc = __ldg(scores + (size_t)g * C + cc); v *= sc * (1.f - sc); }
+        if (write_pre) g_pre[(size_t)g * C + cc] = v;
+      }
+      sg[c][r] = v;
+    }
+    for (int e = threadIdx.x; e < OK * OT; e += kThreads) {
+      const int c = e / OT, k = e % OT;
+      sw[c][k] = (cb + c < C && k0 + k < H) ? __ldg(Wp2 + (size_t)(cb + c) * H + k0 + k) : 0.f;
+    }
+    __syncthreads();
+    const int nc = min(OK, C - cb);
+    for (int c = 0; c < nc; ++c) {
+      float a[RI], w[4];
+#pragma unroll
+      for (int i = 0; i < RI; ++i) a[i] = sg[c][ty + 16 * i];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) w[j] = sw[c][tx + 16 * j];
+#pragma unroll
+      for (int i = 0; i < RI; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(w[j], a[i], acc[i][j]);
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < RI; ++i) {
+    const int g = g0 + ty + 16 * i;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int k = k0 + tx + 16 * j;
+      if (g < B && k < H) g_u[(size_t)g * H + k] = __ldg(rp + (size_t)g * H + k) > 0.f ? acc[i][j] : 0.f;
+    }
+  }
+}
+
 // part[z][m][n] = sum over the rows of split z of A[r][m] * Bm[r][n]   (32x32 output tile per CTA, blockIdx.z = row split;
 // Bm == nullptr: Bm is a column of ones (column sums of A, Nn = 1)).  atb_reduce_kernel adds the splits in order:
 // out[m][n] = sum_z part[z][m][n] - a fixed order, no float atomics.
@@ -439,10 +565,15 @@ void launch_finetune_head_fwd(const FinetuneHeadFwdArgs& a, cudaStream_t s) {
   if (a.H == 32) finetune_head_fwd_kernel<32><<<grid, kThreads, 0, s>>>(a);
   else if (a.H == 64) finetune_head_fwd_kernel<64><<<grid, kThreads, 0, s>>>(a);
   else finetune_head_fwd_kernel<128><<<grid, kThreads, 0, s>>>(a);
+  if (a.C > kMaxC)
+    ft_out_fwd_kernel<<<dim3((a.C + OT - 1) / OT, (a.B + 63) / 64), kThreads, 0, s>>>(a.rp, a.Wp2, a.bp2, a.B, a.C, a.H, a.sigmoid, a.scores);
 }
 
 void launch_finetune_head_bwd(const FinetuneHeadBwdArgs& a, cudaStream_t s) {
   const int grid = (a.B + FG - 1) / FG;
+  if (a.C > kMaxC)
+    ft_out_bwd_kernel<<<dim3((a.H + OT - 1) / OT, (a.B + 31) / 32), kThreads, 0, s>>>(a.rp, a.Wp2, a.scores, a.g_scores, a.B, a.C, a.H,
+                                                                                   a.sigmoid, a.g_pre, a.g_u);
   if (a.H == 32) finetune_head_bwd_kernel<32><<<grid, kThreads, 0, s>>>(a);
   else if (a.H == 64) finetune_head_bwd_kernel<64><<<grid, kThreads, 0, s>>>(a);
   else finetune_head_bwd_kernel<128><<<grid, kThreads, 0, s>>>(a);
@@ -460,6 +591,6 @@ void launch_atb(const float* A, int lda, const float* Bm, int ldb, float* out, i
   atb_reduce_kernel<<<(M * Nn + kThreads - 1) / kThreads, kThreads, 0, s>>>(scratch, S, M, Nn, out, ldo, out2);
 }
 
-int finetune_max_classes() { return kMaxC; }
+int finetune_max_classes() { return kMaxClasses; }
 
 }  // namespace scgib

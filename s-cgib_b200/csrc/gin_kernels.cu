@@ -16,14 +16,15 @@
 namespace scgib {
 
 // ------------------------------------------------------------------------------------------------
-// x_hat = x / max(||x||_2, 1e-12);  t = x_hat Wt^T          (Wt [DTR][F])
+// x_hat = x / max(||x||_2, 1e-12);  t = x_hat Wt^T          (Wt [DTR][F], F <= FMAX)
+// The row norm and each output are sequential sums over f = 0..F-1, whatever FMAX: FMAX only sizes the weight copy.
 // ------------------------------------------------------------------------------------------------
-template <bool OUT_BF16>
+template <bool OUT_BF16, int FMAX>
 __global__ void __launch_bounds__(kThreads)
 input_proj_fwd_kernel(const float* __restrict__ x, const float* __restrict__ Wt, int N, int F, int normalize,
                       float* __restrict__ t) {
   pdl_sync();
-  __shared__ __align__(16) float s_w[32 * DTR];  // [f][o]
+  __shared__ __align__(16) float s_w[FMAX * DTR];  // [f][o]
   for (int i = threadIdx.x; i < F * DTR; i += kThreads) {
     const int o = i / F, f = i % F;
     s_w[f * DTR + o] = Wt[i];
@@ -48,8 +49,13 @@ input_proj_fwd_kernel(const float* __restrict__ x, const float* __restrict__ Wt,
 // out_bf16: t is bf16 storage (bf16 mode: the layer-0 input of the GIN encoders)
 void launch_input_proj_fwd(const float* x, const float* Wt, int N, int F, int normalize, float* t, cudaStream_t s, bool out_bf16) {
   const int grid = min((N + 31) / 32, 148 * 8);
-  if (out_bf16) launch_k((input_proj_fwd_kernel<true>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
-  else launch_k((input_proj_fwd_kernel<false>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+  if (F <= 32) {
+    if (out_bf16) launch_k((input_proj_fwd_kernel<true, 32>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+    else launch_k((input_proj_fwd_kernel<false, 32>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+  } else {
+    if (out_bf16) launch_k((input_proj_fwd_kernel<true, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+    else launch_k((input_proj_fwd_kernel<false, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -88,13 +94,50 @@ __device__ __forceinline__ void xagg_rows(const FwdPrepArgs& p, int cta) {
   }
 }
 
-template <bool OUT_BF16>
+// F > 32: one warp per row, lane l holds the columns l, l + 32, l + 64, l + 96 (coalesced loads, four accumulators).
+// The norm of a neighbour row is the lane partials summed by a butterfly: the same fixed order on every lane and run.
+__device__ __forceinline__ void xagg_rows_wide(const FwdPrepArgs& p, int cta) {
+  constexpr int NC = kMaxInDim / 32;
+  const int V0 = p.xa_V[0], V1 = p.xa_V[1], F = p.F;
+  const int lane = threadIdx.x & 31, wpc = kThreads / 32;
+  for (int i = cta * wpc + (threadIdx.x >> 5); i < V0 + V1; i += p.nxagg * wpc) {
+    const int set = i < V0 ? 0 : 1, v = set == 0 ? i : i - V0;
+    const int32_t* indices = p.xa_indices[set];
+    const int32_t* map = set == 0 ? nullptr : p.xa_map;
+    const int32_t* ip = p.xa_indptr[set];
+    const int e0 = ip ? __ldg(ip + v) : 0, e1 = ip ? __ldg(ip + v + 1) : 0;
+    float acc[NC];
+#pragma unroll
+    for (int c = 0; c < NC; ++c) acc[c] = 0.f;
+    for (int e = e0 - 1; e < e1; ++e) {          // e0 - 1: the row itself
+      const int u = e < e0 ? v : __ldg(indices + e);
+      const float* xr = p.xa_x + (size_t)(map ? __ldg(map + u) : u) * F;
+      float xv[NC];
+      float ss = 0.f;
+#pragma unroll
+      for (int c = 0; c < NC; ++c) { const int f = lane + 32 * c; xv[c] = f < F ? __ldg(xr + f) : 0.f; ss = fmaf(xv[c], xv[c], ss); }
+      ss = warp_sum(ss);
+      const float inv = p.normalize ? 1.f / fmaxf(sqrtf(ss), 1e-12f) : 1.f;
+#pragma unroll
+      for (int c = 0; c < NC; ++c) acc[c] = fmaf(xv[c], inv, acc[c]);
+    }
+    float* d = p.xagg[set] + (size_t)v * p.xa_stride;
+#pragma unroll
+    for (int c = 0; c < NC; ++c)
+      if (lane + 32 * c < p.xa_stride) d[lane + 32 * c] = acc[c];
+  }
+}
+
+// FMAX: 32 for F <= 32, kMaxInDim above (the weight copy of the projection CTAs and the xagg row scheme)
+template <bool OUT_BF16, int FMAX>
 __global__ void __launch_bounds__(kThreads) fwd_prep_kernel(FwdPrepArgs p) {
   pdl_sync();
-  __shared__ __align__(16) float s_w[32 * DTR];  // [f][o]
+  __shared__ __align__(16) float s_w[FMAX * DTR];  // [f][o]
   int b = (int)blockIdx.x;
   if (b < p.nxagg) {
-    if (p.F <= 12) xagg_rows<12>(p, b); else xagg_rows<32>(p, b);
+    if constexpr (FMAX > 32) xagg_rows_wide(p, b);
+    else if (p.F <= 12) xagg_rows<12>(p, b);
+    else xagg_rows<32>(p, b);
     return;
   }
   b -= p.nxagg;
@@ -142,11 +185,18 @@ __global__ void __launch_bounds__(kThreads) fwd_prep_kernel(FwdPrepArgs p) {
 }
 void launch_fwd_prep(FwdPrepArgs a, cudaStream_t s, bool out_bf16) {
   a.nproj = a.x ? min((a.N + 31) / 32, 148 * 8) : 0;
-  a.nxagg = (a.xa_x && a.xagg[0]) ? min((a.xa_V[0] + a.xa_V[1] + kThreads - 1) / kThreads, 148 * 8) : 0;
+  const bool wide = a.F > 32;
+  const int rows_per_cta = wide ? kThreads / 32 : kThreads;     // xagg: a warp per row (wide) or a thread per row
+  a.nxagg = (a.xa_x && a.xagg[0]) ? min((a.xa_V[0] + a.xa_V[1] + rows_per_cta - 1) / rows_per_cta, 148 * 8) : 0;
   const int grid = a.nxagg + a.nproj + a.jobs.n + (a.headW1 ? 8 : 0);
   if (grid == 0) return;
-  if (out_bf16) launch_k((fwd_prep_kernel<true>), dim3(grid), dim3(kThreads), 0, s, a);
-  else launch_k((fwd_prep_kernel<false>), dim3(grid), dim3(kThreads), 0, s, a);
+  if (wide) {
+    if (out_bf16) launch_k((fwd_prep_kernel<true, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, a);
+    else launch_k((fwd_prep_kernel<false, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, a);
+  } else {
+    if (out_bf16) launch_k((fwd_prep_kernel<true, 32>), dim3(grid), dim3(kThreads), 0, s, a);
+    else launch_k((fwd_prep_kernel<false, 32>), dim3(grid), dim3(kThreads), 0, s, a);
+  }
 }
 
 template <bool VEC>      // VEC: float4 loads (x 16-byte aligned, n a multiple of 4)
@@ -674,12 +724,13 @@ void launch_gin_bwd_main(const GinBwdMainArgs& a, int kin, int hidden, int grid,
 // streams Ga0 and xagg (it was a latency-bound CSR gather of 128-byte rows before: 59 us at B = 4096).
 // Two row sets (parent batch, ego batch) in one launch; last CTA finalises into grads.
 // ------------------------------------------------------------------------------------------------
-constexpr int FP = 32;    // padded feature width of a partial row
+// padded feature width of a partial row: 32 up to F = 32, else F rounded up to the FC = 16 columns of a pass
+__host__ __device__ __forceinline__ int ipb_fp(int F) { return F <= 32 ? 32 : (F + 15) / 16 * 16; }
 constexpr int IPB_THREADS = 1024;   // 32 warps per CTA, one CTA per SM: 148 partials for the final (last-CTA) reduction
 
 // lane = output channel o of transfer_d; every warp streams 32-row blocks straight from global memory (coalesced 128-byte
 // Ga0 rows, xagg rows one per lane and broadcast by shuffles) into acc[f] = sum_r Ga0_r[o] xagg_r[f]
-template <int FC>
+template <int FC, bool WIDE>     // WIDE: F > 32
 __global__ void __launch_bounds__(IPB_THREADS, 1)
 input_proj_bwd_kernel(InputProjBwdArgs p) {
   pdl_sync();
@@ -688,6 +739,7 @@ input_proj_bwd_kernel(InputProjBwdArgs p) {
   const int V0 = p.V[0], Vt = p.V[0] + p.V[1], XS = p.xa_stride;
   const int nwarps = (int)gridDim.x * 32;
   const int gw = (int)blockIdx.x * 32 + warp;
+  const int FP = WIDE ? ipb_fp(p.F) : 32;
   for (int fb = 0; fb < XS; fb += FC) {      // FC feature columns per pass over the rows (one pass for F <= 16)
   float acc[FC];
 #pragma unroll
@@ -762,10 +814,12 @@ int input_proj_bwd_grid(int V0, int V1) {
   (void)V0; (void)V1;
   return num_sms();
 }
+size_t input_proj_bwd_part_floats(int V0, int V1, int F) { return (size_t)input_proj_bwd_grid(V0, V1) * DTR * ipb_fp(F); }
 void launch_input_proj_bwd(const InputProjBwdArgs& a, cudaStream_t s) {
   const int grid = input_proj_bwd_grid(a.V[0], a.V[1]);
-  if (a.F <= 12) launch_k((input_proj_bwd_kernel<12>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
-  else launch_k((input_proj_bwd_kernel<16>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+  if (a.F <= 12) launch_k((input_proj_bwd_kernel<12, false>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+  else if (a.F <= 32) launch_k((input_proj_bwd_kernel<16, false>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+  else launch_k((input_proj_bwd_kernel<16, true>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
 }
 
 }  // namespace scgib

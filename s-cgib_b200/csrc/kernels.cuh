@@ -129,11 +129,12 @@ struct InputProjBwdArgs {
   int xa_stride;
   int V[2];
   int F;
-  float* part;              // [grid][DTR*32]
+  float* part;              // [grid][DTR][FP], FP = 32 for F <= 32 (input_proj_bwd_part_floats)
   unsigned int* counter;
   float* d_Wt;              // [DTR][F]
 };
 int input_proj_bwd_grid(int V0, int V1);
+size_t input_proj_bwd_part_floats(int V0, int V1, int F);
 void launch_input_proj_bwd(const InputProjBwdArgs& a, cudaStream_t s);
 
 // ---------------------------------------------------------------- encoder_ops.cu

@@ -522,17 +522,18 @@ class FinetuneHead:
 
 
 class PaddedSet2Set:
-    """``dgl.nn.Set2Set(h, n_iters, 1)`` for a small feature width h <= 32 (Mainmodel_domainadapt.s2s_rev over the raw
-    node features, models.py:114, 267) on the H = 32 instance of the head kernels: weights and features are zero-padded
-    to 32 channels.  A padded hidden unit has zero gate pre-activations (i = f = o = 1/2, g = 0), so its cell and
-    hidden state stay exactly 0 and the real channels are untouched.  The scatter / gather between the module's
+    """``dgl.nn.Set2Set(h, n_iters, 1)`` for a feature width h <= 128 (Mainmodel_domainadapt.s2s_rev over the raw
+    node features, models.py:114, 267) on the smallest H in {32, 64, 128} >= h of the head kernels: weights and features
+    are zero-padded to H channels.  A padded hidden unit has zero gate pre-activations (i = f = o = 1/2, g = 0), so its
+    cell and hidden state stay exactly 0 and the real channels are untouched.  The scatter / gather between the module's
     real-shaped LSTM parameters and the padded flat buffer is index plumbing on four small tensors."""
 
-    P = 32
+    WIDTHS = (32, 64, 128)
 
     def __init__(self, h: int, n_iters: int = 2, device="cuda:0"):
-        if not 1 <= h <= self.P:
-            raise NotImplementedError("PaddedSet2Set: feature width must be <= 32")
+        if not 1 <= h <= self.WIDTHS[-1]:
+            raise NotImplementedError("PaddedSet2Set: feature width must be between 1 and %d, got %d" % (self.WIDTHS[-1], h))
+        self.P = next(w for w in self.WIDTHS if w >= h)
         self.h, self.device = int(h), torch.device(device)
         self.head = FinetuneHead(self.P, 0, n_iters=n_iters, sigmoid=False, device=device)
         P, dev = self.P, self.device

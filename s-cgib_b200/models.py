@@ -217,6 +217,18 @@ def _check_composed_width(encoder, hidden_dim):
         raise NotImplementedError("--encoder %s runs at --dims 64 or 128 on the B200 path" % encoder)
 
 
+MAX_IN_DIM, MAX_CLASSES = 128, 1024     # raw node-feature width and fine-tuning head outputs the kernels take
+
+
+def _check_io_widths(cls, in_dim, num_out=0):
+    """Refuse widths the kernels do not take before any device work: 1 <= in_dim <= 128 (transfer_d, s2s_rev on the
+    widest Set2Set instance) and 0 <= head outputs <= 1024."""
+    if not 1 <= int(in_dim) <= MAX_IN_DIM:
+        raise NotImplementedError("%s: node-feature width in_dim = %d is outside 1..%d on the B200 path" % (cls, in_dim, MAX_IN_DIM))
+    if not 0 <= int(num_out) <= MAX_CLASSES:
+        raise NotImplementedError("%s: %d prediction outputs is outside 0..%d on the B200 path" % (cls, num_out, MAX_CLASSES))
+
+
 def _check_args(args, encoder, allowed=("GIN",)):
     if encoder not in allowed:
         # the reference's own unknown-encoder branch (models.py:585-587); Transformer is outside SURVEY section 8
@@ -358,6 +370,7 @@ class Mainmodel(_HotPathMixin, nn.Module):
         super().__init__()
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
+        _check_io_widths("Mainmodel", in_dim)
         self.encoder_kind = encoder
         self.tau = 1.0
         self.recons_type = args.recons_type
@@ -411,6 +424,7 @@ class Mainmodel_continue(_HotPathMixin, nn.Module):
         super().__init__()
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
+        _check_io_widths("Mainmodel_continue", in_dim)
         self.encoder_kind = encoder
         self.tau = 1.0
         self.readout = args.readout_f
@@ -521,6 +535,7 @@ class Mainmodel_finetuning(nn.Module):
             out_dim = num_classes
         else:
             raise NotImplementedError("task must be graph_regression or graph_classification (models.py:385-399)")
+        _check_io_widths("Mainmodel_finetuning", in_dim, out_dim)
         self.predict = nn.Sequential(nn.Linear(2 * self.hidden_dim, self.hidden_dim), nn.ReLU(),
                                      nn.Linear(self.hidden_dim, out_dim))
         self.MLP = nn.Sequential(nn.Linear(2 * self.hidden_dim, self.hidden_dim), nn.ReLU(),
@@ -664,6 +679,7 @@ class Mainmodel_domainadapt(nn.Module):
         super().__init__()
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
+        _check_io_widths("Mainmodel_domainadapt", in_dim)
         self.tau = 1.0
         self.readout = args.readout_f
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
