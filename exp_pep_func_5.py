@@ -159,7 +159,8 @@ def build_parser():
     parser.add_argument("--pretrained_mode", type=int, default=0)
     parser.add_argument("--domain_adapt", type=int, default=0)
     parser.add_argument("--pretrained_ds", default="pre_training_v1", help="Loading pretrained model ")
-    parser.add_argument("--d_transfer", type=int, default=32)
+    parser.add_argument("--d_transfer", type=int, default=32,
+                        help="width of transfer_d, the encoders' input: 32, 64 or 128, at most --dims (default 32)")
     parser.add_argument("--layer_relax", type=int, default=0)
     parser.add_argument("--readout_f", default="sum")
     parser.add_argument("--adapt_epoches", type=int, default=50)

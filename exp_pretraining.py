@@ -243,7 +243,8 @@ def build_parser():
     parser.add_argument("--device", default="cuda:0", help="GPU ids")
     parser.add_argument("--pretrained_mode", type=int, default=1)
     parser.add_argument("--domain_adapt", type=int, default=0)
-    parser.add_argument("--d_transfer", type=int, default=32)
+    parser.add_argument("--d_transfer", type=int, default=32,
+                        help="width of transfer_d, the encoders' input: 32, 64 or 128, at most --dims (default 32)")
     parser.add_argument("--layer_relax", type=int, default=0)
     parser.add_argument("--readout_f", default="sum")
     parser.add_argument("--batch_size", type=int, default=128)

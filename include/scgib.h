@@ -37,7 +37,7 @@ extern "C" {
 enum {
   SCGIB_OK = 0,
   SCGIB_E_NULL = -1,      /* required pointer is NULL */
-  SCGIB_E_SHAPE = -2,     /* unsupported dimension (hidden must be 64 or 128, d_transfer 32, 1 <= L <= 8, 1 <= F <= 128, fine-tuning head C <= 1024) */
+  SCGIB_E_SHAPE = -2,     /* unsupported dimension (hidden must be 64 or 128, d_transfer 32 / 64 / 128 and <= hidden, 1 <= L <= 8, 1 <= F <= 128, fine-tuning head C <= 1024) */
   SCGIB_E_ALIGN = -3,     /* pointer not 16-byte aligned */
   SCGIB_E_WORKSPACE = -4, /* workspace too small */
   SCGIB_E_RANGE = -5,     /* size out of range (e.g. k < 1, graph with < 2 nodes) */
@@ -56,7 +56,7 @@ SCGIB_API int scgib_num_sms(void);
  * ------------------------------------------------------------------------------------------ */
 typedef struct ScgibDims {
   int32_t in_dim;     /* F: raw feature width (9 PCQM4Mv2 / mol-PCBA, 11 QM9, 37 NCI1, 89 DD), 1 <= F <= 128  exp_pretraining.py:219 */
-  int32_t d_transfer; /* 32                                                      exp_pretraining.py:378 */
+  int32_t d_transfer; /* DT: 32, 64 or 128, at most hidden (the layer-0 input width)  exp_pretraining.py:378 */
   int32_t hidden;     /* 64 or 128 (--dims)                                      exp_pretraining.py:390 */
   int32_t gin_layers; /* L: GINConv per encoder (4 in models.py:57-58)                               */
   int32_t act_dtype;  /* SCGIB_ACT_F32 (reference precision, 1e-5) or SCGIB_ACT_BF16: the GIN encoders keep their
@@ -262,7 +262,7 @@ SCGIB_API int scgib_adam_step_f32(float* params, const float* grads, float* exp_
  * Individual operators (what the autograd Functions of the drop-in modules call; also the
  * unit-test surface).  H = 64.
  * ------------------------------------------------------------------------------------------ */
-/* F.normalize(x) then transfer_d (exp_pretraining.py:312-314, models.py:668): t[N,DT].  1 <= F <= 128. */
+/* F.normalize(x) then transfer_d (exp_pretraining.py:312-314, models.py:668): t[N,DT].  1 <= F <= 128, DT 32, 64 or 128. */
 SCGIB_API int scgib_input_proj_fwd_f32(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT,
                              float* t, void* stream);
 
@@ -399,8 +399,10 @@ SCGIB_API int scgib_segment_sum_bwd_f32(const float* g_out, const int32_t* seg_p
  *      (backward products g (.) (h > 0)); X1 NULL = one operand pair.
  *  scgib_linear_bwd_w_f32    : dW (+)= (G (.) (M > 0))^T X[map] as [O][K] (kxo = 0) or [K][O] (kxo = 1), db (+)= column sums;
  *      fixed-order two-stage reduction (bit-identical reruns).  O multiple of 64.  workspace 16-byte aligned.
- *  scgib_transfer_bwd_f32    : d transfer_d.weight [32][F] = sum over two row sets of g_r (x) xrow_r, xrow_r = x_hat[p(r)]
- *      (+ the x_hat rows of r's neighbours when a CSR is given).  1 <= F <= 128.  workspace 256-byte aligned.
+ *  scgib_transfer_bwd_d_f32  : d transfer_d.weight [DT][F] = sum over two row sets of g_r (x) xrow_r, xrow_r = x_hat[p(r)]
+ *      (+ the x_hat rows of r's neighbours when a CSR is given); g0 / g1 are [V][DT].  1 <= F <= 128, DT 32, 64 or 128.
+ *      workspace 256-byte aligned, from scgib_transfer_bwd_workspace_bytes_d (0 for an unsupported DT).
+ *  scgib_transfer_bwd_f32    : scgib_transfer_bwd_d_f32 at DT = 32 (and its workspace query).
  * ------------------------------------------------------------------------------------------ */
 SCGIB_API int scgib_graph_aggregate_f32(const float* in, int32_t W, const int32_t* row_map, const int32_t* indptr,
                                         const int32_t* indices, int32_t V, int32_t src_norm, int32_t dst_norm,
@@ -418,13 +420,19 @@ SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32_t normaliz
                                      const int32_t* indptr0, const int32_t* indices0, const float* g1, int32_t V1,
                                      const int32_t* indptr1, const int32_t* indices1, const int32_t* map1, float* dWt,
                                      void* workspace, size_t workspace_bytes, void* stream);
+SCGIB_API size_t scgib_transfer_bwd_workspace_bytes_d(int32_t V0, int32_t V1, int32_t F, int32_t DT);
+SCGIB_API int scgib_transfer_bwd_d_f32(const float* x, int32_t F, int32_t DT, int32_t normalize, const float* g0, int32_t V0,
+                                       const int32_t* indptr0, const int32_t* indices0, const float* g1, int32_t V1,
+                                       const int32_t* indptr1, const int32_t* indices1, const int32_t* map1, float* dWt,
+                                       void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * The same building blocks in bf16 mode (--dtype bf16; csrc/encoder_bf16.cu): activations, masks and layer gradients are
  * bf16 storage (raw 16-bit words), weights / bias / dW / db fp32; every sum is fp32.  All data pointers 16-byte aligned
  * (SCGIB_E_ALIGN), widths in {32, 64, 128, 256} (SCGIB_E_SHAPE), V >= 1 (SCGIB_E_RANGE); checked before any launch.
  *
- *  scgib_input_proj_fwd_bf16  : scgib_input_proj_fwd_f32 with the [N][32] output rounded to bf16.
+ *  scgib_input_proj_fwd_d_bf16 : scgib_input_proj_fwd_f32 with the [N][DT] output rounded to bf16, DT 32, 64 or 128.
+ *  scgib_input_proj_fwd_bf16  : scgib_input_proj_fwd_d_bf16 at DT = 32 (any other DT: SCGIB_E_SHAPE).
  *  scgib_f32_to_bf16          : out = rnd(in), n a multiple of 8.
  *  scgib_graph_aggregate_bf16 : scgib_graph_aggregate_f32 on bf16 in / add; out bf16, or fp32 when out_f32.
  *  scgib_linear_fwd_bf16      : scgib_linear_fwd_f32 on bf16 Xp / Mp, single-pass tcgen05 MMAs with the weights rounded to
@@ -434,6 +442,7 @@ SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32_t normaliz
  *      tcgen05; workspace from scgib_linear_bwd_w_bf16_workspace_bytes.
  * ------------------------------------------------------------------------------------------ */
 SCGIB_API int scgib_input_proj_fwd_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t, void* stream);
+SCGIB_API int scgib_input_proj_fwd_d_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t, void* stream);
 SCGIB_API int scgib_f32_to_bf16(const float* in, int64_t n, void* out, void* stream);
 SCGIB_API int scgib_graph_aggregate_bf16(const void* in, int32_t W, const int32_t* row_map, const int32_t* indptr,
                                          const int32_t* indices, int32_t V, int32_t src_norm, int32_t dst_norm,

@@ -123,7 +123,11 @@ _SIGNATURES = {
     "scgib_transfer_bwd_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
     "scgib_transfer_bwd_f32": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "scgib_transfer_bwd_workspace_bytes_d": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "scgib_transfer_bwd_d_f32": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
+                                         c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "scgib_input_proj_fwd_bf16": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    "scgib_input_proj_fwd_d_bf16": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "scgib_f32_to_bf16": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "scgib_graph_aggregate_bf16": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p,
                                            c_void_p, c_int32, c_void_p]),

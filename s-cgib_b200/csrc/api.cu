@@ -115,7 +115,7 @@ static inline void debug_check(const char* name, cudaStream_t s) {
 #define PROF(name, stmt) do { prof_begin(name, s); stmt; prof_end(s); debug_check(name, s); } while (0)
 
 static bool dims_ok(const ScgibDims* d) {
-  return d && (d->hidden == 64 || d->hidden == 128) && d->d_transfer == DTR && d->gin_layers >= 1 && d->gin_layers <= 8 && d->in_dim >= 1 &&
+  return d && (d->hidden == 64 || d->hidden == 128) && transfer_width_ok(d->d_transfer, d->hidden) && d->gin_layers >= 1 && d->gin_layers <= 8 && d->in_dim >= 1 &&
          d->in_dim <= kMaxInDim && (d->act_dtype == SCGIB_ACT_F32 || d->act_dtype == SCGIB_ACT_BF16);
 }
 
@@ -134,14 +134,14 @@ static Layout make_layout(const ScgibDims* d) {
       (int64_t)HID * 2 * HID, HID, (int64_t)HID * HID, HID,      // head
       (int64_t)HID * HID, HID, HID, HID, HID, 1,                  // compressor
       2 * HID, 1,                                                 // attention
-      (int64_t)DTR * d->in_dim};                                  // transfer_d
+      (int64_t)d->d_transfer * d->in_dim};                        // transfer_d
   int n = 0;
   int64_t o = 0;
   auto push = [&](int64_t s) { lo.off[n] = o; lo.size[n] = s; o += (s + 3) / 4 * 4; ++n; };
   for (int i = 0; i < SCGIB_P_ENC; ++i) push(sizes[i]);
   for (int e = 0; e < 2; ++e)
     for (int l = 0; l < L; ++l) {
-      const int kin = (l == 0) ? DTR : HID;
+      const int kin = (l == 0) ? d->d_transfer : HID;
       push((int64_t)HID * kin); push(HID); push((int64_t)HID * HID); push(HID); push(HID); push(HID);
     }
   lo.n = n;
@@ -174,14 +174,14 @@ struct Ws {
 
 static inline int xagg_stride(const ScgibDims* d) { return (d->in_dim + 3) / 4 * 4; }
 
-static size_t small_part_floats(int N, int Ns, int HID, int F) {
+static size_t small_part_floats(int N, int Ns, int HID, int F, int DT) {
   const int Vmax = N > Ns ? N : Ns;
   size_t a = (size_t)((Vmax + 63) / 64) * 2 * HID;                   // gin fwd tile partials (64-row tiles)
   const size_t a2 = (size_t)num_sms() * 3 * HID * 2;                  // gin_tc2: per-CTA (n, mean, M2) in fp64
   a = a > a2 ? a : a2;
   size_t b = (size_t)(gin_bwd_pre_grid(N + Ns) + 2) * 2 * HID;       // dgamma/dbeta partials (per problem of a shared launch)
   size_t c = (size_t)4 * num_sms() * 5 * HID;                        // gate partials
-  size_t d = input_proj_bwd_part_floats(N, Ns, F);                     // transfer_d partials
+  size_t d = input_proj_bwd_part_floats(N, Ns, F, DT);                   // transfer_d partials
   size_t m = a > b ? a : b;
   m = m > c ? m : c;
   return m > d ? m : d;
@@ -200,7 +200,7 @@ static Ws carve(const ScgibDims* d, const Layout& lo, int B, int N, int E, int N
   const int Vmax = N > Ns ? N : Ns;
   for (int e = 0; e < 2; ++e)
     for (int l = 0; l < L; ++l) {
-      const int kin = l == 0 ? DTR : HID;
+      const int kin = l == 0 ? d->d_transfer : HID;
       w.enc_w1t[e][l] = take((size_t)kin * HID);
       w.enc_w2t[e][l] = take((size_t)HID * HID);
       w.a[e][l] = take_act((size_t)V[e] * kin);
@@ -209,9 +209,10 @@ static Ws carve(const ScgibDims* d, const Layout& lo, int B, int N, int E, int N
       w.bn[e][l] = take(4 * HID);
     }
   w.head_w1t = take(2 * HID * HID); w.head_w2t = take(HID * HID); w.comp_w1t = take(HID * HID);
-  w.t = take_act((size_t)N * DTR);
+  w.t = take_act((size_t)N * d->d_transfer);
   w.cvec[0] = take(2 * HID); w.cvec[1] = take(2 * HID);
-  w.small_part = take(small_part_floats(N, Ns, HID, d->in_dim)); w.small_part2 = take(small_part_floats(N, Ns, HID, d->in_dim));
+  w.small_part = take(small_part_floats(N, Ns, HID, d->in_dim, d->d_transfer));
+  w.small_part2 = take(small_part_floats(N, Ns, HID, d->in_dim, d->d_transfer));
   w.counters = (unsigned int*)take(64);
   w.H = take((size_t)N * HID); w.q = take((size_t)N * HID); w.C = take((size_t)N * HID);
   w.logit = take(N); w.alpha = take(N); w.lam = take(N);
@@ -230,7 +231,7 @@ static Ws carve(const ScgibDims* d, const Layout& lo, int B, int N, int E, int N
   w.g_o[0] = take_act((size_t)N * HID); w.g_o[1] = take_act((size_t)Ns * HID);
   w.Ga[0] = take_act((size_t)N * HID); w.Ga[1] = take_act((size_t)Ns * HID);
   (void)Vmax;
-  w.ga0[0] = take((size_t)N * DTR); w.ga0[1] = take((size_t)Ns * DTR);
+  w.ga0[0] = take((size_t)N * d->d_transfer); w.ga0[1] = take((size_t)Ns * d->d_transfer);
   w.xagg[0] = take((size_t)N * xagg_stride(d)); w.xagg[1] = take((size_t)Ns * xagg_stride(d));
   w.logm_walks = take((size_t)logm_max_steps() * N); w.logm_gram = take(B); w.logm_pair = take(N); w.logm_loss = take(4);
   w.aC = take((size_t)N * HID); w.head_w1a = take(HID * HID); w.head_w1b = take(HID * HID);
@@ -270,7 +271,7 @@ extern "C" SCGIB_API const char* scgib_error_string(int code) {
   switch (code) {
     case SCGIB_OK: return "ok";
     case SCGIB_E_NULL: return "required pointer is NULL";
-    case SCGIB_E_SHAPE: return "unsupported dimensions (hidden must be 64 or 128, d_transfer 32, 1 <= gin_layers <= 8, 1 <= in_dim <= 128, fine-tuning head outputs C <= 1024; --recons_type logM and the op-level entries: hidden 64)";
+    case SCGIB_E_SHAPE: return "unsupported dimensions (hidden must be 64 or 128, d_transfer 32, 64 or 128 and <= hidden, 1 <= gin_layers <= 8, 1 <= in_dim <= 128, fine-tuning head outputs C <= 1024; --recons_type logM and the op-level entries: hidden 64)";
     case SCGIB_E_ALIGN: return "pointer not 16-byte aligned";
     case SCGIB_E_WORKSPACE: return "workspace too small";
     case SCGIB_E_RANGE: return "size out of range";
@@ -316,7 +317,7 @@ static int forward_impl(const ScgibDims* d, const float* params, float* bn_runni
   const Ws w = carve(d, lo, b->B, b->N, b->E, b->Ns, b->Es, workspace);
   if (workspace_bytes < w.bytes) return SCGIB_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream_;
-  const int L = d->gin_layers, HID = d->hidden;
+  const int L = d->gin_layers, HID = d->hidden, DT = d->d_transfer;
   const bool eval = b->eval_mode != 0;       // model.eval(): BatchNorm layers use (and do not update) their running statistics
   if (eval && !bn_running) return SCGIB_E_NULL;
   const bool bf = d->act_dtype == SCGIB_ACT_BF16;   // bf16 mode: GIN activations in bf16, single-pass bf16 tensor-core MLPs
@@ -336,7 +337,7 @@ static int forward_impl(const ScgibDims* d, const float* params, float* bn_runni
     if (enc_ffma)
       for (int e = 0; e < 2; ++e)
         for (int l = 0; l < L; ++l) {
-          add(params + lo.enc(e, l, L, SCGIB_ENC_W1), w.enc_w1t[e][l], HID, l == 0 ? DTR : HID);
+          add(params + lo.enc(e, l, L, SCGIB_ENC_W1), w.enc_w1t[e][l], HID, l == 0 ? DT : HID);
           add(params + lo.enc(e, l, L, SCGIB_ENC_W2), w.enc_w2t[e][l], HID, HID);
           if (jobs.n >= 20) { launch_transposes(jobs, s); jobs.n = 0; }
         }
@@ -346,11 +347,11 @@ static int forward_impl(const ScgibDims* d, const float* params, float* bn_runni
     pa.headW1 = params + lo.off[SCGIB_P_HEAD_W1]; pa.W1a = w.head_w1a; pa.W1b = w.head_w1b; pa.bn = w.head_bn; pa.cvec = w.head_cvec;
     pa.hid = HID;
     if (b->t_override && bf)
-      launch_f32_to_bf16(b->t_override, w.t, (size_t)b->N * DTR, s);
+      launch_f32_to_bf16(b->t_override, w.t, (size_t)b->N * DT, s);
     else if (b->t_override)
-      cudaMemcpyAsync(w.t, b->t_override, (size_t)b->N * DTR * sizeof(float), cudaMemcpyDeviceToDevice, s);
+      cudaMemcpyAsync(w.t, b->t_override, (size_t)b->N * DT * sizeof(float), cudaMemcpyDeviceToDevice, s);
     else {
-      pa.x = b->x; pa.Wt = params + lo.off[SCGIB_P_TRANSFER]; pa.N = b->N; pa.F = d->in_dim; pa.normalize = b->normalize_x; pa.t = w.t;
+      pa.x = b->x; pa.Wt = params + lo.off[SCGIB_P_TRANSFER]; pa.N = b->N; pa.F = d->in_dim; pa.DT = DT; pa.normalize = b->normalize_x; pa.t = w.t;
       if (!eval) {      // the backward pass of this step contracts the layer-0 input gradients with the aggregated features
         pa.xa_indptr[0] = b->indptr; pa.xa_indptr[1] = b->sub_indptr; pa.xa_indices[0] = b->indices; pa.xa_indices[1] = b->sub_indices;
         pa.xa_x = b->x; pa.xa_map = b->ego_nodes; pa.xa_V[0] = b->N; pa.xa_V[1] = b->Ns;
@@ -380,11 +381,12 @@ static int forward_impl(const ScgibDims* d, const float* params, float* bn_runni
       a.running = (bn_running && !eval) ? bn_running + (size_t)(e * L + l) * 2 * HID : nullptr;
       a.reverse = (l & 1) && fwd_alternate();
     }
-    const int kin = l == 0 ? DTR : HID;
+    const int kin = l == 0 ? DT : HID;
     if (bf) {
       PROF("gin_fwd_bf16.enc1+2", launch_gin_fwd_bf16(ga[0], &ga[1], kin, HID, s));
     } else if (tc64 && tensor_core_mode() != 0) {
-      if (kin == HID && fwd_tc4_mode()) PROF("gin_fwd_tc4.enc1+2", launch_gin_fwd_tc4_pair(ga[0], ga[1], s));
+      // gin_tc4 has no ego row map: layer 0 stays on gin_fwd_tc3 also when d_transfer = hidden
+      if (l > 0 && fwd_tc4_mode()) PROF("gin_fwd_tc4.enc1+2", launch_gin_fwd_tc4_pair(ga[0], ga[1], s));
       else PROF("gin_fwd_tc.enc1+2", launch_gin_fwd_tc3_pair(ga[0], ga[1], kin, s));
     } else {
       for (int e = 0; e < 2; ++e) PROF(e == 0 ? "gin_fwd_ffma.enc1" : "gin_fwd_ffma.enc2", launch_gin_fwd(ga[e], kin, HID, s));
@@ -490,7 +492,7 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
   const Ws w = carve(d, lo, b->B, b->N, b->E, b->Ns, b->Es, workspace);
   if (workspace_bytes < w.bytes) return SCGIB_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream_;
-  const int L = d->gin_layers, HID = d->hidden;
+  const int L = d->gin_layers, HID = d->hidden, DT = d->d_transfer;
   const int GP = num_sms();
   const float s_kl = loss_scale[0], s_con = loss_scale[1], s_rec = loss_scale[2];
   const bool bf = d->act_dtype == SCGIB_ACT_BF16;
@@ -601,7 +603,7 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
   const int enc_split = pair_split(GP, (b->N + 127) / 128, (b->Ns + 127) / 128);   // CTAs of Encoder1 in a shared launch
   const bool pair_main = bf || tc_bwd;
   for (int l = L - 1; l >= 0; --l) {
-    const int kin = l == 0 ? DTR : HID;
+    const int kin = l == 0 ? DT : HID;
     GinBwdPreArgs pa[2];
     GinBwdMainArgs ma[2];
     for (int e = 0; e < 2; ++e) {
@@ -627,7 +629,7 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
     }
     if (bf) {
       PROF("gin_bwd_pre_bf16.enc1+2", launch_gin_bwd_pre_bf16(pa[0], &pa[1], HID, s));
-      PROF("gin_bwd_main_bf16.enc1+2", launch_gin_bwd_main_bf16(ma[0], &ma[1], kin, HID, GP, s));
+      PROF("gin_bwd_main_bf16.enc1+2", launch_gin_bwd_main_bf16(ma[0], &ma[1], kin, HID, GP, s, l == 0));
       continue;
     }
     PROF("gin_bwd_pre.enc1+2", launch_gin_bwd_pre_pair(pa[0], pa[1], HID, s));
@@ -643,7 +645,7 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
   {
     InputProjBwdArgs a;
     a.ga[0] = w.ga0[0]; a.ga[1] = w.ga0[1]; a.xagg[0] = w.xagg[0]; a.xagg[1] = w.xagg[1]; a.xa_stride = xagg_stride(d);
-    a.V[0] = b->N; a.V[1] = b->Ns; a.F = d->in_dim; a.part = w.small_part; a.counter = w.counters + 3;
+    a.V[0] = b->N; a.V[1] = b->Ns; a.F = d->in_dim; a.DT = DT; a.part = w.small_part; a.counter = w.counters + 3;
     a.d_Wt = grads + lo.off[SCGIB_P_TRANSFER];
     PROF("input_proj_bwd", launch_input_proj_bwd(a, s));
   }
@@ -811,33 +813,38 @@ extern "C" SCGIB_API int scgib_finetune_head_bwd_f32(const float* head_params, i
 // ---------------------------------------------------------------- individual operators
 extern "C" SCGIB_API int scgib_input_proj_fwd_f32(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, float* t, void* stream) {
   if (!x || !Wt || !t) return SCGIB_E_NULL;
-  if (DT != DTR || F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
+  if (!transfer_width_ok(DT, kMaxTransfer) || F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
   if (N < 1) return SCGIB_E_RANGE;
-  launch_input_proj_fwd(x, Wt, N, F, 1, t, (cudaStream_t)stream);
+  launch_input_proj_fwd(x, Wt, N, F, DT, 1, t, (cudaStream_t)stream);
   return (int)cudaGetLastError();
 }
 
 // transfer_d backward as an operator: dWt[o][f] = sum over both row sets of g_r[o] * xrow_r[f], xrow_r = x_hat[p(r)] (+ the
-// x_hat rows of r's neighbours when a CSR is given: the layer-0 aggregation backward of the GIN path moved to the features)
-extern "C" SCGIB_API size_t scgib_transfer_bwd_workspace_bytes(int32_t V0, int32_t V1, int32_t F) {
+// x_hat rows of r's neighbours when a CSR is given: the layer-0 aggregation backward of the GIN path moved to the features).
+// The *_d entries take the width DT of g0 / g1 / dWt (32, 64 or 128); the others are DT = 32.
+extern "C" SCGIB_API size_t scgib_transfer_bwd_workspace_bytes_d(int32_t V0, int32_t V1, int32_t F, int32_t DT) {
+  if (!transfer_width_ok(DT, kMaxTransfer)) return 0;
   const size_t xs = (size_t)(F + 3) / 4 * 4;
-  return al((size_t)V0 * xs * 4) + al((size_t)V1 * xs * 4) + al(input_proj_bwd_part_floats(V0, V1, F) * 4) + 256;
+  return al((size_t)V0 * xs * 4) + al((size_t)V1 * xs * 4) + al(input_proj_bwd_part_floats(V0, V1, F, DT) * 4) + 256;
 }
-extern "C" SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32_t normalize, const float* g0, int32_t V0,
-                                                const int32_t* indptr0, const int32_t* indices0, const float* g1, int32_t V1,
-                                                const int32_t* indptr1, const int32_t* indices1, const int32_t* map1,
-                                                float* dWt, void* workspace, size_t workspace_bytes, void* stream) {
+extern "C" SCGIB_API size_t scgib_transfer_bwd_workspace_bytes(int32_t V0, int32_t V1, int32_t F) {
+  return scgib_transfer_bwd_workspace_bytes_d(V0, V1, F, 32);
+}
+extern "C" SCGIB_API int scgib_transfer_bwd_d_f32(const float* x, int32_t F, int32_t DT, int32_t normalize, const float* g0, int32_t V0,
+                                                  const int32_t* indptr0, const int32_t* indices0, const float* g1, int32_t V1,
+                                                  const int32_t* indptr1, const int32_t* indices1, const int32_t* map1,
+                                                  float* dWt, void* workspace, size_t workspace_bytes, void* stream) {
   if (!x || !g0 || !dWt || !workspace || (V1 > 0 && (!g1 || !map1))) return SCGIB_E_NULL;
-  if (F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
+  if (F < 1 || F > kMaxInDim || !transfer_width_ok(DT, kMaxTransfer)) return SCGIB_E_SHAPE;
   if (V0 < 1 || V1 < 0) return SCGIB_E_RANGE;
   if (((uintptr_t)workspace & 255u) != 0) return SCGIB_E_ALIGN;
-  if (workspace_bytes < scgib_transfer_bwd_workspace_bytes(V0, V1, F)) return SCGIB_E_WORKSPACE;
+  if (workspace_bytes < scgib_transfer_bwd_workspace_bytes_d(V0, V1, F, DT)) return SCGIB_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
   const int xs = (F + 3) / 4 * 4;
   char* p = (char*)workspace;
   float* xa0 = (float*)p; p += al((size_t)V0 * xs * 4);
   float* xa1 = (float*)p; p += al((size_t)V1 * xs * 4);
-  float* part = (float*)p; p += al(input_proj_bwd_part_floats(V0, V1, F) * 4);
+  float* part = (float*)p; p += al(input_proj_bwd_part_floats(V0, V1, F, DT) * 4);
   unsigned int* counter = (unsigned int*)p;
   cudaMemsetAsync(counter, 0, 64, s);
   FwdPrepArgs pa;
@@ -849,9 +856,16 @@ extern "C" SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32
   launch_fwd_prep(pa, s, false);
   InputProjBwdArgs a;
   a.ga[0] = g0; a.ga[1] = g1 ? g1 : g0; a.xagg[0] = xa0; a.xagg[1] = xa1; a.xa_stride = xs;
-  a.V[0] = V0; a.V[1] = V1; a.F = F; a.part = part; a.counter = counter; a.d_Wt = dWt;
+  a.V[0] = V0; a.V[1] = V1; a.F = F; a.DT = DT; a.part = part; a.counter = counter; a.d_Wt = dWt;
   launch_input_proj_bwd(a, s);
   return (int)cudaGetLastError();
+}
+extern "C" SCGIB_API int scgib_transfer_bwd_f32(const float* x, int32_t F, int32_t normalize, const float* g0, int32_t V0,
+                                                const int32_t* indptr0, const int32_t* indices0, const float* g1, int32_t V1,
+                                                const int32_t* indptr1, const int32_t* indices1, const int32_t* map1,
+                                                float* dWt, void* workspace, size_t workspace_bytes, void* stream) {
+  return scgib_transfer_bwd_d_f32(x, F, 32, normalize, g0, V0, indptr0, indices0, g1, V1, indptr1, indices1, map1, dWt, workspace,
+                                  workspace_bytes, stream);
 }
 
 extern "C" SCGIB_API size_t scgib_gin_workspace_bytes(int32_t V) {
@@ -867,7 +881,7 @@ extern "C" SCGIB_API int scgib_gin_layer_fwd_f32(const float* in, int32_t kin, c
                                        float* y_out, float* bn_out, float* running, void* workspace,
                                        size_t workspace_bytes, void* stream_) {
   if (!in || !indptr || !W1 || !b1 || !W2 || !b2 || !y_out || !bn_out || !workspace) return SCGIB_E_NULL;
-  if (kin != DTR && kin != HID) return SCGIB_E_SHAPE;
+  if (kin != 32 && kin != HID) return SCGIB_E_SHAPE;
   if (bn_in && kin != HID) return SCGIB_E_SHAPE;
   if (V < 1) return SCGIB_E_RANGE;
   if (workspace_bytes < scgib_gin_workspace_bytes(V)) return SCGIB_E_WORKSPACE;
@@ -912,7 +926,7 @@ static GinBwdOpWs gin_bwd_op_carve(int V, int kin, void* base) {
 }  // namespace scgib
 
 extern "C" SCGIB_API size_t scgib_gin_layer_bwd_workspace_bytes(int32_t V, int32_t kin) {
-  if (V < 1 || (kin != DTR && kin != HID)) return 0;
+  if (V < 1 || (kin != 32 && kin != HID)) return 0;
   return gin_bwd_op_carve(V, kin, nullptr).bytes;
 }
 
@@ -924,7 +938,7 @@ extern "C" SCGIB_API int scgib_gin_layer_bwd_f32(const float* g_next, const int3
   if (!g_next || !y || !r || !a || !bn || !W1 || !W2 || !g_a || !dW1 || !db1 || !dW2 || !db2 || !dgamma || !dbeta || !workspace)
     return SCGIB_E_NULL;
   if (indptr && !indices) return SCGIB_E_NULL;
-  if (kin != DTR && kin != HID) return SCGIB_E_SHAPE;
+  if (kin != 32 && kin != HID) return SCGIB_E_SHAPE;
   if (V < 1) return SCGIB_E_RANGE;
   if (((uintptr_t)workspace & 255u) != 0) return SCGIB_E_ALIGN;
   const GinBwdOpWs w = gin_bwd_op_carve(V, kin, workspace);

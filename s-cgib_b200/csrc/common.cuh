@@ -6,7 +6,10 @@
 namespace scgib {
 
 constexpr int HID = 64;        // hidden width (exp_pretraining.py:390)
-constexpr int DTR = 32;        // d_transfer   (exp_pretraining.py:378)
+// d_transfer (exp_pretraining.py:378, the layer-0 input width of the encoders): 32, 64 or 128 and at most hidden.  Tensor-core
+// tiles are built from 32-column lines and the gin_fwd_tc3 stage holds windows of at most 64 columns.
+constexpr int kMaxTransfer = 128;
+__host__ __device__ constexpr bool transfer_width_ok(int d, int hidden) { return (d == 32 || d == 64 || d == 128) && d <= hidden; }
 constexpr int kThreads = 256;  // CTA size of every tile kernel
 constexpr int kMaxInDim = 128; // widest raw node-feature input (transfer_d, s2s_rev on the H = 128 Set2Set instance)
 constexpr int kMaxClasses = 1024;   // widest fine-tuning head output (C; 2 * kMaxInDim for r_transfer_d)

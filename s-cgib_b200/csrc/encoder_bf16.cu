@@ -352,14 +352,23 @@ using namespace scgib;
 static bool width_ok_b(int W) { return W == 32 || W == 64 || W == 128 || W == 256; }
 static bool al16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
 
-extern "C" SCGIB_API int scgib_input_proj_fwd_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t,
-                                                   void* stream) {
+// DT: 32, 64 or 128 (the *_d entry); scgib_input_proj_fwd_bf16 keeps its contract DT = 32
+static int input_proj_fwd_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, int32_t max_dt, void* t,
+                               void* stream) {
   if (!x || !Wt || !t) return SCGIB_E_NULL;
-  if (DT != DTR || F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
+  if (!transfer_width_ok(DT, max_dt) || F < 1 || F > kMaxInDim) return SCGIB_E_SHAPE;
   if (N < 1) return SCGIB_E_RANGE;
   if (!al16(t)) return SCGIB_E_ALIGN;
-  launch_input_proj_fwd(x, Wt, N, F, 1, reinterpret_cast<float*>(t), (cudaStream_t)stream, true);
+  launch_input_proj_fwd(x, Wt, N, F, DT, 1, reinterpret_cast<float*>(t), (cudaStream_t)stream, true);
   return (int)cudaGetLastError();
+}
+extern "C" SCGIB_API int scgib_input_proj_fwd_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t,
+                                                   void* stream) {
+  return input_proj_fwd_bf16(x, Wt, N, F, DT, 32, t, stream);
+}
+extern "C" SCGIB_API int scgib_input_proj_fwd_d_bf16(const float* x, const float* Wt, int32_t N, int32_t F, int32_t DT, void* t,
+                                                     void* stream) {
+  return input_proj_fwd_bf16(x, Wt, N, F, DT, kMaxTransfer, t, stream);
 }
 
 extern "C" SCGIB_API int scgib_f32_to_bf16(const float* in, int64_t n, void* out, void* stream) {

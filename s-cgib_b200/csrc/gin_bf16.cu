@@ -539,9 +539,11 @@ void launch_gin_fwd_bf16(const GinFwdArgs& a0, const GinFwdArgs* a1, int kin, in
   if (dbg < 0) { const char* e = getenv("SCGIB_DBG"); dbg = e ? atoi(e) : 0; }
   pp.a[0].dbg = pp.a[1].dbg = dbg;
   if (hidden == 64) {
-    if (kin == DTR) launch_fwd_bf16<DTR, 64>(pp, grid, s); else launch_fwd_bf16<64, 64>(pp, grid, s);
+    if (kin == 32) launch_fwd_bf16<32, 64>(pp, grid, s); else launch_fwd_bf16<64, 64>(pp, grid, s);
   } else {
-    if (kin == DTR) launch_fwd_bf16<DTR, 128>(pp, grid, s); else launch_fwd_bf16<128, 128>(pp, grid, s);
+    if (kin == 32) launch_fwd_bf16<32, 128>(pp, grid, s);
+    else if (kin == 64) launch_fwd_bf16<64, 128>(pp, grid, s);      // layer 0 at d_transfer 64
+    else launch_fwd_bf16<128, 128>(pp, grid, s);
   }
 }
 

@@ -562,7 +562,8 @@ static void launch_bwd_bf16_t(const GinBwdMainPair& pp, int grid, cudaStream_t s
 }
 
 // CTAs [0, split) write the partial gradients of a0, [split, grid) of a1 (a1 == nullptr: one problem).  g_o / y / r / a are
-// bf16; g_a is bf16, except for kin == DTR (layer 0), where it is fp32.
+// bf16; g_a is bf16, except with ga_f32 (layer 0 and the head backward), where it is fp32.  kin < hidden happens at layer 0
+// only, which always takes fp32 g_a.
 void launch_gin_bwd_main_bf16(const GinBwdMainArgs& a0, const GinBwdMainArgs* a1, int kin, int hidden, int grid, cudaStream_t s,
                               bool ga_f32) {
   GinBwdMainPair pp;
@@ -571,11 +572,12 @@ void launch_gin_bwd_main_bf16(const GinBwdMainArgs& a0, const GinBwdMainArgs* a1
   pp.trace = 0;
   pp.reverse = 1;
   if (hidden == 64) {
-    if (kin == DTR) launch_bwd_bf16_t<DTR, 64, true>(pp, grid, s);
+    if (kin == 32) launch_bwd_bf16_t<32, 64, true>(pp, grid, s);
     else if (ga_f32) launch_bwd_bf16_t<64, 64, true>(pp, grid, s);
     else launch_bwd_bf16_t<64, 64, false>(pp, grid, s);
   } else {
-    if (kin == DTR) launch_bwd_bf16_t<DTR, 128, true>(pp, grid, s);
+    if (kin == 32) launch_bwd_bf16_t<32, 128, true>(pp, grid, s);
+    else if (kin == 64) launch_bwd_bf16_t<64, 128, true>(pp, grid, s);
     else if (ga_f32) launch_bwd_bf16_t<128, 128, true>(pp, grid, s);
     else launch_bwd_bf16_t<128, 128, false>(pp, grid, s);
   }

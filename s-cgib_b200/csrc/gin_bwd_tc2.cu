@@ -446,7 +446,7 @@ void launch_gin_bwd_main_tc2(const GinBwdMainArgs& a, int kin, int grid, cudaStr
   pp.split = grid;
   pp.trace = 0;
   pp.reverse = 0;
-  if (kin == DTR) launch_bwd2<DTR>(pp, grid, s); else launch_bwd2<HID>(pp, grid, s);
+  if (kin == 32) launch_bwd2<32>(pp, grid, s); else launch_bwd2<HID>(pp, grid, s);
 }
 
 // the same layer of both encoders in one launch: CTAs [0, split) write the partial gradients of a0, [split, grid) of a1
@@ -461,7 +461,7 @@ void launch_gin_bwd_main_tc2_pair(const GinBwdMainArgs& a0, const GinBwdMainArgs
   static int rev = -1;
   if (rev < 0) { const char* e = getenv("SCGIB_BWD_REV"); rev = (e && e[0] == '0') ? 0 : 1; }
   pp.reverse = rev;
-  if (kin == DTR) launch_bwd2<DTR>(pp, grid, s); else launch_bwd2<HID>(pp, grid, s);
+  if (kin == 32) launch_bwd2<32>(pp, grid, s); else launch_bwd2<HID>(pp, grid, s);
 }
 
 }  // namespace scgib

@@ -16,22 +16,19 @@
 namespace scgib {
 
 // ------------------------------------------------------------------------------------------------
-// x_hat = x / max(||x||_2, 1e-12);  t = x_hat Wt^T          (Wt [DTR][F], F <= FMAX)
+// x_hat = x / max(||x||_2, 1e-12);  t = x_hat Wt^T          (Wt [DT][F], F <= FMAX, DT = 32, 64 or 128)
 // The row norm and each output are sequential sums over f = 0..F-1, whatever FMAX: FMAX only sizes the weight copy.
+// The outputs are computed in passes over 32-column groups (kProjGroup): the weight copy holds one group, so it stays
+// within the static shared-memory limit at F = 128, DT = 128, and DT = 32 is the single pass it always was.
 // ------------------------------------------------------------------------------------------------
-template <bool OUT_BF16, int FMAX>
-__global__ void __launch_bounds__(kThreads)
-input_proj_fwd_kernel(const float* __restrict__ x, const float* __restrict__ Wt, int N, int F, int normalize,
-                      float* __restrict__ t) {
-  pdl_sync();
-  __shared__ __align__(16) float s_w[FMAX * DTR];  // [f][o]
-  for (int i = threadIdx.x; i < F * DTR; i += kThreads) {
-    const int o = i / F, f = i % F;
-    s_w[f * DTR + o] = Wt[i];
-  }
-  __syncthreads();
+constexpr int kProjGroup = 32;
+
+// the rows [v0, N) step vstep of one 32-column output group g0 of a projection CTA (s_w: this group's weights, [f][o])
+template <bool OUT_BF16>
+__device__ __forceinline__ void input_proj_rows(const float* __restrict__ x, const float* s_w, int v0, int vstep, int N, int F,
+                                                int DT, int g0, int normalize, float* __restrict__ t) {
   const int q = threadIdx.x & 7;  // output quad
-  for (int v = blockIdx.x * (kThreads / 8) + (threadIdx.x >> 3); v < N; v += gridDim.x * (kThreads / 8)) {
+  for (int v = v0 + (threadIdx.x >> 3); v < N; v += vstep) {
     const float* xr = x + (size_t)v * F;
     float ss = 0.f;
     for (int f = 0; f < F; ++f) { const float a = __ldg(xr + f); ss = fmaf(a, a, ss); }
@@ -39,22 +36,42 @@ input_proj_fwd_kernel(const float* __restrict__ x, const float* __restrict__ Wt,
     float4 acc = make4(0.f);
     for (int f = 0; f < F; ++f) {
       const float a = __ldg(xr + f) * inv;
-      const float4 w = ld4(s_w + f * DTR + q * 4);
+      const float4 w = ld4(s_w + f * kProjGroup + q * 4);
       acc.x = fmaf(a, w.x, acc.x); acc.y = fmaf(a, w.y, acc.y); acc.z = fmaf(a, w.z, acc.z); acc.w = fmaf(a, w.w, acc.w);
     }
-    st4a<OUT_BF16>(t, (size_t)v * DTR + q * 4, acc);
+    st4a<OUT_BF16>(t, (size_t)v * DT + g0 + q * 4, acc);
+  }
+}
+__device__ __forceinline__ void stage_proj_group(float* s_w, const float* __restrict__ Wt, int F, int g0) {
+  for (int i = threadIdx.x; i < F * kProjGroup; i += kThreads) {
+    const int o = i / F, f = i % F;
+    s_w[f * kProjGroup + o] = Wt[(size_t)g0 * F + i];
+  }
+}
+
+template <bool OUT_BF16, int FMAX>
+__global__ void __launch_bounds__(kThreads)
+input_proj_fwd_kernel(const float* __restrict__ x, const float* __restrict__ Wt, int N, int F, int DT, int normalize,
+                      float* __restrict__ t) {
+  pdl_sync();
+  __shared__ __align__(16) float s_w[FMAX * kProjGroup];  // [f][o]
+  for (int g0 = 0; g0 < DT; g0 += kProjGroup) {
+    if (g0 > 0) __syncthreads();     // every reader of the previous group's weights is done
+    stage_proj_group(s_w, Wt, F, g0);
+    __syncthreads();
+    input_proj_rows<OUT_BF16>(x, s_w, blockIdx.x * (kThreads / 8), gridDim.x * (kThreads / 8), N, F, DT, g0, normalize, t);
   }
 }
 
 // out_bf16: t is bf16 storage (bf16 mode: the layer-0 input of the GIN encoders)
-void launch_input_proj_fwd(const float* x, const float* Wt, int N, int F, int normalize, float* t, cudaStream_t s, bool out_bf16) {
+void launch_input_proj_fwd(const float* x, const float* Wt, int N, int F, int DT, int normalize, float* t, cudaStream_t s, bool out_bf16) {
   const int grid = min((N + 31) / 32, 148 * 8);
   if (F <= 32) {
-    if (out_bf16) launch_k((input_proj_fwd_kernel<true, 32>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
-    else launch_k((input_proj_fwd_kernel<false, 32>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+    if (out_bf16) launch_k((input_proj_fwd_kernel<true, 32>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, DT, normalize, t);
+    else launch_k((input_proj_fwd_kernel<false, 32>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, DT, normalize, t);
   } else {
-    if (out_bf16) launch_k((input_proj_fwd_kernel<true, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
-    else launch_k((input_proj_fwd_kernel<false, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, normalize, t);
+    if (out_bf16) launch_k((input_proj_fwd_kernel<true, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, DT, normalize, t);
+    else launch_k((input_proj_fwd_kernel<false, kMaxInDim>), dim3(grid), dim3(kThreads), 0, s, x, Wt, N, F, DT, normalize, t);
   }
 }
 
@@ -132,7 +149,7 @@ __device__ __forceinline__ void xagg_rows_wide(const FwdPrepArgs& p, int cta) {
 template <bool OUT_BF16, int FMAX>
 __global__ void __launch_bounds__(kThreads) fwd_prep_kernel(FwdPrepArgs p) {
   pdl_sync();
-  __shared__ __align__(16) float s_w[FMAX * DTR];  // [f][o]
+  __shared__ __align__(16) float s_w[FMAX * kProjGroup];  // [f][o] of one 32-column output group
   int b = (int)blockIdx.x;
   if (b < p.nxagg) {
     if constexpr (FMAX > 32) xagg_rows_wide(p, b);
@@ -142,25 +159,11 @@ __global__ void __launch_bounds__(kThreads) fwd_prep_kernel(FwdPrepArgs p) {
   }
   b -= p.nxagg;
   if (b < p.nproj) {
-    const int F = p.F;
-    for (int i = threadIdx.x; i < F * DTR; i += kThreads) {
-      const int o = i / F, f = i % F;
-      s_w[f * DTR + o] = p.Wt[i];
-    }
-    __syncthreads();
-    const int q = threadIdx.x & 7;  // output quad
-    for (int v = b * (kThreads / 8) + (threadIdx.x >> 3); v < p.N; v += p.nproj * (kThreads / 8)) {
-      const float* xr = p.x + (size_t)v * F;
-      float ss = 0.f;
-      for (int f = 0; f < F; ++f) { const float a = __ldg(xr + f); ss = fmaf(a, a, ss); }
-      const float inv = p.normalize ? 1.f / fmaxf(sqrtf(ss), 1e-12f) : 1.f;
-      float4 acc = make4(0.f);
-      for (int f = 0; f < F; ++f) {
-        const float a = __ldg(xr + f) * inv;
-        const float4 w = ld4(s_w + f * DTR + q * 4);
-        acc.x = fmaf(a, w.x, acc.x); acc.y = fmaf(a, w.y, acc.y); acc.z = fmaf(a, w.z, acc.z); acc.w = fmaf(a, w.w, acc.w);
-      }
-      st4a<OUT_BF16>(p.t, (size_t)v * DTR + q * 4, acc);
+    for (int g0 = 0; g0 < p.DT; g0 += kProjGroup) {
+      if (g0 > 0) __syncthreads();
+      stage_proj_group(s_w, p.Wt, p.F, g0);
+      __syncthreads();
+      input_proj_rows<OUT_BF16>(p.x, s_w, b * (kThreads / 8), p.nproj * (kThreads / 8), p.N, p.F, p.DT, g0, p.normalize, p.t);
     }
     return;
   }
@@ -440,8 +443,10 @@ static void launch_gin_fwd_t(const GinFwdArgs& a, cudaStream_t s) {
   launch_k((gin_fwd_kernel<KIN, H>), dim3(grid), dim3(kThreads), sizeof(GinFwdSmem<KIN, H>), s, a);
 }
 void launch_gin_fwd(const GinFwdArgs& a, int kin, int hidden, cudaStream_t s) {
-  if (hidden == 64) { if (kin == DTR) launch_gin_fwd_t<DTR, 64>(a, s); else launch_gin_fwd_t<64, 64>(a, s); }
-  else { if (kin == DTR) launch_gin_fwd_t<DTR, 128>(a, s); else launch_gin_fwd_t<128, 128>(a, s); }
+  if (hidden == 64) { if (kin == 32) launch_gin_fwd_t<32, 64>(a, s); else launch_gin_fwd_t<64, 64>(a, s); }
+  else if (kin == 32) launch_gin_fwd_t<32, 128>(a, s);
+  else if (kin == 64) launch_gin_fwd_t<64, 128>(a, s);        // layer 0 at d_transfer 64
+  else launch_gin_fwd_t<128, 128>(a, s);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -712,13 +717,15 @@ static void launch_gin_bwd_main_t(const GinBwdMainArgs& a, int grid, cudaStream_
   launch_k((gin_bwd_main_kernel<KIN, H, GTB>), dim3(grid), dim3(kThreads), sizeof(S), s, a);
 }
 void launch_gin_bwd_main(const GinBwdMainArgs& a, int kin, int hidden, int grid, cudaStream_t s) {
-  if (hidden == 64) { if (kin == DTR) launch_gin_bwd_main_t<DTR, 64, 128>(a, grid, s); else launch_gin_bwd_main_t<64, 64, 128>(a, grid, s); }
-  else { if (kin == DTR) launch_gin_bwd_main_t<DTR, 128, 32>(a, grid, s); else launch_gin_bwd_main_t<128, 128, 32>(a, grid, s); }
+  if (hidden == 64) { if (kin == 32) launch_gin_bwd_main_t<32, 64, 128>(a, grid, s); else launch_gin_bwd_main_t<64, 64, 128>(a, grid, s); }
+  else if (kin == 32) launch_gin_bwd_main_t<32, 128, 32>(a, grid, s);
+  else if (kin == 64) launch_gin_bwd_main_t<64, 128, 32>(a, grid, s);     // layer 0 at d_transfer 64
+  else launch_gin_bwd_main_t<128, 128, 32>(a, grid, s);
 }
 
 // ------------------------------------------------------------------------------------------------
 // transfer_d backward: dWt[o][f] = sum_rows gt_row[o] * x_hat[map(row)][f] with gt_row = Ga0_row + sum_{u in N(row)} Ga0_u
-// (layer-0 aggregation backward; Ga0 is [V][DTR]).  The adjacency is symmetric, so the gather moves to the features:
+// (layer-0 aggregation backward; Ga0 is [V][DT]).  The adjacency is symmetric, so the gather moves to the features:
 //   dWt[o][f] = sum_u Ga0_u[o] * xagg_u[f],   xagg_u = x_hat[p(u)] + sum_{v in N(u)} x_hat[p(v)]
 // xagg is a constant of the batch, produced by side CTAs of the forward's prologue launch (fwd_prep); this kernel only
 // streams Ga0 and xagg (it was a latency-bound CSR gather of 128-byte rows before: 59 us at B = 4096).
@@ -728,9 +735,10 @@ void launch_gin_bwd_main(const GinBwdMainArgs& a, int kin, int hidden, int grid,
 __host__ __device__ __forceinline__ int ipb_fp(int F) { return F <= 32 ? 32 : (F + 15) / 16 * 16; }
 constexpr int IPB_THREADS = 1024;   // 32 warps per CTA, one CTA per SM: 148 partials for the final (last-CTA) reduction
 
-// lane = output channel o of transfer_d; every warp streams 32-row blocks straight from global memory (coalesced 128-byte
-// Ga0 rows, xagg rows one per lane and broadcast by shuffles) into acc[f] = sum_r Ga0_r[o] xagg_r[f]
-template <int FC, bool WIDE>     // WIDE: F > 32
+// lane = output channel og + o of transfer_d (og: 32-channel group, one pass over the rows each); every warp streams 32-row
+// blocks straight from global memory (coalesced 128-byte Ga0 row segments, xagg rows one per lane and broadcast by shuffles)
+// into acc[f] = sum_r Ga0_r[og + o] xagg_r[f]
+template <int FC, bool WIDE, int DT>     // WIDE: F > 32; DT: d_transfer (a compile-time stride, so DT = 32 keeps its code)
 __global__ void __launch_bounds__(IPB_THREADS, 1)
 input_proj_bwd_kernel(InputProjBwdArgs p) {
   pdl_sync();
@@ -740,6 +748,7 @@ input_proj_bwd_kernel(InputProjBwdArgs p) {
   const int nwarps = (int)gridDim.x * 32;
   const int gw = (int)blockIdx.x * 32 + warp;
   const int FP = WIDE ? ipb_fp(p.F) : 32;
+  for (int og = 0; og < DT; og += 32)
   for (int fb = 0; fb < XS; fb += FC) {      // FC feature columns per pass over the rows (one pass for F <= 16)
   float acc[FC];
 #pragma unroll
@@ -761,7 +770,7 @@ input_proj_bwd_kernel(InputProjBwdArgs p) {
       for (int j = 0; j < 8; ++j) {
         const int r = rb + j0 + j;
         const int set = r < V0 ? 0 : 1, v = r < V0 ? r : r - V0;
-        g[j] = r < Vt ? __ldcs(p.ga[set] + (size_t)v * DTR + lane) : 0.f;
+        g[j] = r < Vt ? __ldcs(p.ga[set] + (size_t)v * DT + og + lane) : 0.f;
       }
 #pragma unroll
       for (int j = 0; j < 8; ++j)
@@ -775,7 +784,7 @@ input_proj_bwd_kernel(InputProjBwdArgs p) {
     }
   }
   // CTA partial [o][f] (stride FP): the 32 warps are summed in a fixed order, four feature columns at a time
-  float* part = p.part + (size_t)blockIdx.x * DTR * FP;
+  float* part = p.part + ((size_t)blockIdx.x * DT + og) * FP;
 #pragma unroll
   for (int q = 0; q < FC / 4; ++q) {
     __syncthreads();
@@ -792,7 +801,7 @@ input_proj_bwd_kernel(InputProjBwdArgs p) {
   }
   if (!last_cta_arrives(p.counter)) return;
   // only the F real feature columns; interleaved partial sums keep the loads of a thread independent; fixed order
-  for (int o2 = threadIdx.x; o2 < DTR * p.F; o2 += IPB_THREADS) {
+  for (int o2 = threadIdx.x; o2 < DT * p.F; o2 += IPB_THREADS) {
     const int oo = o2 / p.F, f = o2 % p.F;
     const float* src = p.part + oo * FP + f;
     double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
@@ -800,12 +809,12 @@ input_proj_bwd_kernel(InputProjBwdArgs p) {
     int b = 0;
 #pragma unroll 8
     for (; b + 3 < nb; b += 4) {
-      s0 += (double)__ldcg(src + (size_t)b * DTR * FP);
-      s1 += (double)__ldcg(src + (size_t)(b + 1) * DTR * FP);
-      s2 += (double)__ldcg(src + (size_t)(b + 2) * DTR * FP);
-      s3 += (double)__ldcg(src + (size_t)(b + 3) * DTR * FP);
+      s0 += (double)__ldcg(src + (size_t)b * DT * FP);
+      s1 += (double)__ldcg(src + (size_t)(b + 1) * DT * FP);
+      s2 += (double)__ldcg(src + (size_t)(b + 2) * DT * FP);
+      s3 += (double)__ldcg(src + (size_t)(b + 3) * DT * FP);
     }
-    for (; b < nb; ++b) s0 += (double)__ldcg(src + (size_t)b * DTR * FP);
+    for (; b < nb; ++b) s0 += (double)__ldcg(src + (size_t)b * DT * FP);
     p.d_Wt[oo * p.F + f] = (float)((s0 + s1) + (s2 + s3));
   }
 }
@@ -814,12 +823,18 @@ int input_proj_bwd_grid(int V0, int V1) {
   (void)V0; (void)V1;
   return num_sms();
 }
-size_t input_proj_bwd_part_floats(int V0, int V1, int F) { return (size_t)input_proj_bwd_grid(V0, V1) * DTR * ipb_fp(F); }
+size_t input_proj_bwd_part_floats(int V0, int V1, int F, int DT) { return (size_t)input_proj_bwd_grid(V0, V1) * DT * ipb_fp(F); }
+template <int FC, bool WIDE>
+static void launch_ipb(const InputProjBwdArgs& a, int grid, cudaStream_t s) {
+  if (a.DT == 32) launch_k((input_proj_bwd_kernel<FC, WIDE, 32>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+  else if (a.DT == 64) launch_k((input_proj_bwd_kernel<FC, WIDE, 64>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+  else launch_k((input_proj_bwd_kernel<FC, WIDE, 128>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+}
 void launch_input_proj_bwd(const InputProjBwdArgs& a, cudaStream_t s) {
   const int grid = input_proj_bwd_grid(a.V[0], a.V[1]);
-  if (a.F <= 12) launch_k((input_proj_bwd_kernel<12, false>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
-  else if (a.F <= 32) launch_k((input_proj_bwd_kernel<16, false>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
-  else launch_k((input_proj_bwd_kernel<16, true>), dim3(grid), dim3(IPB_THREADS), 0, s, a);
+  if (a.F <= 12) launch_ipb<12, false>(a, grid, s);
+  else if (a.F <= 32) launch_ipb<16, false>(a, grid, s);
+  else launch_ipb<16, true>(a, grid, s);
 }
 
 }  // namespace scgib

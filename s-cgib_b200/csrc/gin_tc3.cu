@@ -534,7 +534,7 @@ void launch_gin_fwd_tc3(const GinFwdArgs& a, int kin, cudaStream_t s) {
   pp.a[0] = a; pp.a[1] = a;
   const int grid = min((a.V + tc3::TM - 1) / tc3::TM, num_sms());
   pp.split = grid;                                   // single problem: every CTA works on a[0]
-  if (kin == DTR) launch_tc3<DTR>(pp, grid, s); else launch_tc3<HID>(pp, grid, s);
+  if (kin == 32) launch_tc3<32>(pp, grid, s); else launch_tc3<HID>(pp, grid, s);
 }
 
 // the same layer of both encoders in one launch (separate part / counter / bn_out buffers per problem)
@@ -545,7 +545,7 @@ void launch_gin_fwd_tc3_pair(const GinFwdArgs& a0, const GinFwdArgs& a1, int kin
   const int grid = min(t0 + t1, num_sms());
   pp.split = pair_split(grid, t0, t1);
   pp.a[0].dbg = pp.a[1].dbg = dbg_mask3();
-  if (kin == DTR) launch_tc3<DTR>(pp, grid, s); else launch_tc3<HID>(pp, grid, s);
+  if (kin == 32) launch_tc3<32>(pp, grid, s); else launch_tc3<HID>(pp, grid, s);
 }
 
 }  // namespace scgib

@@ -14,14 +14,14 @@ void launch_transposes(const TransposeJobs& jobs, cudaStream_t s);
 // eval mode (model.eval()): bn = {running_mean, 1/sqrt(running_var + eps), gamma, beta} replaces the batch statistics a
 // GIN forward kernel has just written, before the next layer / the pooling kernels read them
 void launch_bn_from_running(const float* running, const float* gamma, const float* beta, float* bn, int hidden, cudaStream_t s);
-void launch_input_proj_fwd(const float* x, const float* Wt, int N, int F, int normalize, float* t, cudaStream_t s, bool out_bf16 = false);
+void launch_input_proj_fwd(const float* x, const float* Wt, int N, int F, int DT, int normalize, float* t, cudaStream_t s, bool out_bf16 = false);
 void launch_f32_to_bf16(const float* in, void* out, size_t n, cudaStream_t s);
 // input projection + weight transposes + head-backward operand preparation in one launch (any part optional:
 // x == nullptr, jobs.n == 0, headW1 == nullptr)
 struct FwdPrepArgs {
   TransposeJobs jobs;
   const float* headW1 = nullptr; float *W1a = nullptr, *W1b = nullptr, *bn = nullptr, *cvec = nullptr; int hid = 64;
-  const float* x = nullptr; const float* Wt = nullptr; int N = 0, F = 0, normalize = 0; float* t = nullptr;
+  const float* x = nullptr; const float* Wt = nullptr; int N = 0, F = 0, DT = 32, normalize = 0; float* t = nullptr;   // t [N][DT]
   // aggregated normalised features xagg_v = x_hat[p(v)] + sum_{u in N(v)} x_hat[p(u)] of the parent rows and the ego rows
   // (a constant of the batch: the transfer_d backward contracts the layer-0 input gradient with it, input_proj_bwd)
   const int32_t* xa_indptr[2] = {nullptr, nullptr}; const int32_t* xa_indices[2] = {nullptr, nullptr};
@@ -113,7 +113,7 @@ void launch_gin_bwd_main_tc2_pair(const GinBwdMainArgs& a0, const GinBwdMainArgs
 int gin_bwd_pre_bf16_grid(int V, int hidden);
 void launch_gin_bwd_pre_bf16(const GinBwdPreArgs& a0, const GinBwdPreArgs* a1, int hidden, cudaStream_t s);
 void launch_gin_bwd_main_bf16(const GinBwdMainArgs& a0, const GinBwdMainArgs* a1, int kin, int hidden, int grid, cudaStream_t s,
-                              bool ga_f32 = false);      // ga_f32: g_a is written as fp32 also for kin == hidden (head backward)
+                              bool ga_f32 = false);      // ga_f32: g_a is written as fp32 (layer 0: input_proj_bwd reads it; head backward)
 void launch_gin_bwd_main_h_pair(const GinBwdMainArgs& a0, const GinBwdMainArgs& a1, int kin, int grid, cudaStream_t s,
                                 bool weights_from_prev_kernel = false);     // tcgen05, two-term fp16 splits, 128-row tiles (gin_bwd_h.cu); kin 32 | 64
 void launch_gin_bwd_main_h(const GinBwdMainArgs& a, int kin, int grid, cudaStream_t s);   // single problem
@@ -124,17 +124,18 @@ int bwd_h_mode();                                                          // SC
 int bwd_tensor_core_mode();                                                                // SCGIB_TC_BWD: 1 gin_bwd_tc2.cu (default), 0 FFMA cross-check
 
 struct InputProjBwdArgs {
-  const float* ga[2];       // layer-0 input gradients of the two encoders, [V][DTR]
+  const float* ga[2];       // layer-0 input gradients of the two encoders, [V][DT]
   const float* xagg[2];     // aggregated normalised features of the rows, [V][xa_stride] (fwd_prep)
   int xa_stride;
   int V[2];
   int F;
-  float* part;              // [grid][DTR][FP], FP = 32 for F <= 32 (input_proj_bwd_part_floats)
+  int DT;                   // d_transfer: 32, 64 or 128
+  float* part;              // [grid][DT][FP], FP = 32 for F <= 32 (input_proj_bwd_part_floats)
   unsigned int* counter;
-  float* d_Wt;              // [DTR][F]
+  float* d_Wt;              // [DT][F]
 };
 int input_proj_bwd_grid(int V0, int V1);
-size_t input_proj_bwd_part_floats(int V0, int V1, int F);
+size_t input_proj_bwd_part_floats(int V0, int V1, int F, int DT);
 void launch_input_proj_bwd(const InputProjBwdArgs& a, cudaStream_t s);
 
 // ---------------------------------------------------------------- encoder_ops.cu

@@ -26,8 +26,6 @@ import torch.nn as nn
 from . import ops
 from .ops import NORM_MEAN, NORM_NONE, NORM_SQRT
 
-DTR = 32
-
 
 def _f32_out(x):
     """keyword of the operators that leave the encoders (h3, g_t): fp32 output when the encoder runs in bf16."""

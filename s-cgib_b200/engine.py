@@ -18,7 +18,7 @@ import torch
 from . import _lib
 from .graph import BatchedGraph, EgoBatch, EgoWorkspace, khop_ego_batch
 
-HID, DTR = 64, 32
+HID = 64
 _VALIDATE = __import__("os").environ.get("SCGIB_VALIDATE", "0") == "1"     # per-batch input validation (one extra host read)
 
 
@@ -36,13 +36,13 @@ def param_names(gin_layers: int):
     return names
 
 
-def param_shapes(in_dim: int, gin_layers: int, hidden: int = HID):
-    H = hidden
+def param_shapes(in_dim: int, gin_layers: int, hidden: int = HID, d_transfer: int = 32):
+    H, D = hidden, d_transfer
     shapes = [(H, 2 * H), (H,), (H, H), (H,), (H, H), (H,), (H,), (H,), (1, H), (1,),
-              (1, 2 * H), (1,), (DTR, in_dim)]
+              (1, 2 * H), (1,), (D, in_dim)]
     for _e in range(2):
         for l in range(gin_layers):
-            shapes += [(H, DTR if l == 0 else H), (H,), (H, H), (H,), (H,), (H,)]
+            shapes += [(H, D if l == 0 else H), (H,), (H, H), (H,), (H,), (H,)]
     return shapes
 
 
@@ -81,17 +81,17 @@ class DeviceBatch:
         b.eval_mode = int(bool(self.eval_mode))
         return b
 
-    def algorithmic_bytes(self, gin_layers=4, F=9, s=4, hidden=HID):   # s = bytes per activation element (2 in bf16 mode)
+    def algorithmic_bytes(self, gin_layers=4, F=9, s=4, hidden=HID, d_transfer=32):   # s = bytes per activation element (2 in bf16 mode)
         """SURVEY.md §8(d) 'algorithmic bytes per training step' evaluated on this batch's actual sizes."""
-        N, E, Ns, Es, d = self.N, self.E, self.Ns, self.Es, hidden
+        N, E, Ns, Es, d, dt = self.N, self.E, self.Ns, self.Es, hidden, d_transfer
 
         def enc(V, D):
             tot = 0
             for l in range(gin_layers):
-                din = DTR if l == 0 else d
+                din = dt if l == 0 else d
                 tot += V * (din + d) * s + 4 * (V + 1 + D)
             return tot
-        fwd = enc(N, E) + enc(Ns, Es) + N * F * 4 + Ns * 4 + N * DTR * s + (Ns + N) * d * s + 2 * N * d * s + \
+        fwd = enc(N, E) + enc(Ns, Es) + N * F * 4 + Ns * 4 + N * dt * s + (Ns + N) * d * s + 2 * N * d * s + \
             (N + 1) * d * s + 2 * N * d * s + N * d * s + 4 * (N + 1 + E) + 4 * d * s
         ego = 4 * (N + 1 + E) + 4 * (2 * Ns + 1 + Es + N + 1)
         return 3 * fwd + ego
@@ -120,7 +120,7 @@ class PretrainEngine:
         self.total = int(self.lib.scgib_param_layout(ctypes.byref(self.dims), off, sz))
         self.offsets, self.sizes = list(off), list(sz)
         self.names = param_names(gin_layers)
-        self.shapes = param_shapes(in_dim, gin_layers, self.hidden)
+        self.shapes = param_shapes(in_dim, gin_layers, self.hidden, int(d_transfer))
         assert len(self.names) == n == len(self.shapes)
         self.params = torch.zeros(self.total, dtype=torch.float32, device=self.device)
         self.grads = torch.zeros_like(self.params)

@@ -52,6 +52,7 @@ class GIN(nn.Module):
         super().__init__()
         if hidden_dim not in (64, 128):
             raise NotImplementedError("libscgib is built for hidden_dim 64 or 128 (--dims, exp_pretraining.py:390)")
+        _check_transfer_width("GIN", input_dim, hidden_dim)
         self.hidden_dim = hidden_dim
         self.ginlayers = nn.ModuleList()
         self.batch_norms = nn.ModuleList()
@@ -186,7 +187,8 @@ class _Bridge:
     def _sync_slow(self, device):
         if self.engine is None or self.engine.device != device:
             self.engine = PretrainEngine(self.in_dim, gin_layers=self.gin_layers, hidden=int(getattr(self.owner, "hidden_dim", HID)),
-                                         device=device, dtype=getattr(self.owner, "act_dtype", "fp32"))
+                                         d_transfer=self.owner.transfer_d.out_features, device=device,
+                                         dtype=getattr(self.owner, "act_dtype", "fp32"))
         views = self.engine.views()
         params = []
         for name in self.slot_names:
@@ -218,6 +220,32 @@ def _check_composed_width(encoder, hidden_dim):
 
 
 MAX_IN_DIM, MAX_CLASSES = 128, 1024     # raw node-feature width and fine-tuning head outputs the kernels take
+TRANSFER_WIDTHS = (32, 64, 128)         # --d_transfer: the layer-0 input width of the encoders, at most --dims
+
+
+def _check_transfer_width(cls, d_transfer, hidden_dim):
+    """Refuse a --d_transfer the kernels do not take before any device work: 32, 64 or 128 and at most hidden_dim (the
+    tensor-core tiles are built from 32-column lines; one rule for every encoder)."""
+    d, h = int(d_transfer), int(hidden_dim)
+    if d not in TRANSFER_WIDTHS or d > h:
+        allowed = ", ".join(str(w) for w in TRANSFER_WIDTHS if w <= h)
+        raise NotImplementedError("%s: d_transfer = %d is not supported on the B200 path at hidden_dim %d (allowed: %s; "
+                                  "d_transfer in {32, 64, 128} and d_transfer <= hidden_dim)" % (cls, d, h, allowed))
+
+
+def _encoder_in_width(enc):
+    """layer-0 input width of an encoder: the d_transfer of the model that built it."""
+    if hasattr(enc, "ginlayers"):
+        return enc.ginlayers[0].apply_func.mlp[0].in_features
+    return int(enc.in_feats)
+
+
+def _check_loaded_width(cls, loaded, d_transfer):
+    """The loaded module's encoders read the wrapper's transfer_d output: their input width must be args.d_transfer."""
+    w = _encoder_in_width(loaded.Encoder1)
+    if w != int(d_transfer):
+        raise ValueError("%s: the loaded checkpoint's encoders take d_transfer = %d inputs, but --d_transfer is %d; pass "
+                         "--d_transfer %d (the width the checkpoint was pre-trained with)" % (cls, w, int(d_transfer), w))
 
 
 def _check_io_widths(cls, in_dim, num_out=0):
@@ -371,6 +399,7 @@ class Mainmodel(_HotPathMixin, nn.Module):
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
         _check_io_widths("Mainmodel", in_dim)
+        _check_transfer_width("Mainmodel", args.d_transfer, hidden_dim)
         self.encoder_kind = encoder
         self.tau = 1.0
         self.recons_type = args.recons_type
@@ -425,6 +454,7 @@ class Mainmodel_continue(_HotPathMixin, nn.Module):
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
         _check_io_widths("Mainmodel_continue", in_dim)
+        _check_transfer_width("Mainmodel_continue", args.d_transfer, hidden_dim)
         self.encoder_kind = encoder
         self.tau = 1.0
         self.readout = args.readout_f
@@ -460,6 +490,7 @@ class Mainmodel_continue(_HotPathMixin, nn.Module):
             self.Encoder1 = make_encoder(encoder, self.in_dim, hidden_dim)
             self.Encoder2 = make_encoder(encoder, self.in_dim, hidden_dim)
         self.model = torch.load(cp_filename, map_location=args.device, weights_only=False)
+        _check_loaded_width("Mainmodel_continue", self.model, args.d_transfer)
         for p in self.model.parameters():
             p.requires_grad = True
         self.compressor = nn.Sequential(nn.Linear(self.hidden_dim, self.hidden_dim), nn.BatchNorm1d(self.hidden_dim),
@@ -510,6 +541,7 @@ class Mainmodel_finetuning(nn.Module):
         super().__init__()
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
+        _check_transfer_width("Mainmodel_finetuning", args.d_transfer, hidden_dim)
         self.tau = 1.0
         self.dataset = args.dataset
         self.readout = args.readout_f
@@ -543,6 +575,7 @@ class Mainmodel_finetuning(nn.Module):
         self.Encoder1, self.Encoder2 = _own_encoders(encoder, self.in_dim, hidden_dim, self.gin_layers)
         print("Loading pre-trained model .pt  ... ")
         self.model = torch.load(cp_filename, map_location=args.device, weights_only=False)
+        _check_loaded_width("Mainmodel_finetuning", self.model, args.d_transfer)
         for name, para in self.model.named_parameters():     # models.py:424-435: the last list entry decides
             para.requires_grad = "layers.2" in name          # (no GraphSAGE / GCN name contains it: all frozen)
         self.compressor = nn.Sequential(nn.Linear(self.hidden_dim, self.hidden_dim), nn.BatchNorm1d(self.hidden_dim),
@@ -680,6 +713,7 @@ class Mainmodel_domainadapt(nn.Module):
         _check_args(args, encoder, allowed=("GIN", "GraphSAGE", "GCN"))
         _check_composed_width(encoder, hidden_dim)
         _check_io_widths("Mainmodel_domainadapt", in_dim)
+        _check_transfer_width("Mainmodel_domainadapt", args.d_transfer, hidden_dim)
         self.tau = 1.0
         self.readout = args.readout_f
         self.gin_layers = int(getattr(args, "gin_layers", DEFAULT_GIN_LAYERS))
@@ -708,6 +742,7 @@ class Mainmodel_domainadapt(nn.Module):
         self.Encoder1, self.Encoder2 = _own_encoders(encoder, self.in_dim, hidden_dim, self.gin_layers)
         print("Loading pre-trained model .pt  ... ")
         self.model = torch.load(cp_filename, map_location=args.device, weights_only=False)
+        _check_loaded_width("Mainmodel_domainadapt", self.model, args.d_transfer)
         for p in self.model.parameters():
             p.requires_grad = True
         self.compressor = nn.Sequential(nn.Linear(self.hidden_dim, self.hidden_dim), nn.BatchNorm1d(self.hidden_dim),

@@ -8,7 +8,7 @@ import torch
 
 from . import _lib
 
-HID, DTR = 64, 32
+HID = 64
 
 
 def _stream(t):
@@ -22,11 +22,12 @@ def _cuda(*ts):
 
 
 def input_proj(x: torch.Tensor, Wt: torch.Tensor, out_dtype=torch.float32) -> torch.Tensor:
-    """transfer_d(F.normalize(x))  (exp_pretraining.py:312, models.py:668); ``out_dtype`` torch.bfloat16 rounds the output."""
+    """transfer_d(F.normalize(x))  (exp_pretraining.py:312, models.py:668): [N, d_transfer] with d_transfer = Wt.shape[0]
+    (32, 64 or 128); ``out_dtype`` torch.bfloat16 rounds the output."""
     _cuda(x, Wt)
     x, Wt = x.contiguous().float(), Wt.contiguous().float()
-    t = torch.empty(x.shape[0], DTR, device=x.device, dtype=out_dtype)
-    entry = _lib.load().scgib_input_proj_fwd_bf16 if out_dtype == torch.bfloat16 else _lib.load().scgib_input_proj_fwd_f32
+    t = torch.empty(x.shape[0], Wt.shape[0], device=x.device, dtype=out_dtype)
+    entry = _lib.load().scgib_input_proj_fwd_d_bf16 if out_dtype == torch.bfloat16 else _lib.load().scgib_input_proj_fwd_f32
     _lib.check(entry(_lib.ptr(x), _lib.ptr(Wt), x.shape[0], x.shape[1], Wt.shape[0], _lib.ptr(t), _stream(x)), "input_proj_fwd")
     return t
 
@@ -369,18 +370,21 @@ def linear_bwd_w(G, X, dW, db=None, M=None, map=None, kxo=False, accumulate=Fals
 
 
 def transfer_bwd(x, g0, g1, map1, normalize=True, csr0=None, csr1=None):
-    """d transfer_d.weight [32, F] from the input gradients of the two row sets (parent rows / ego rows through map1)."""
+    """d transfer_d.weight [d_transfer, F] from the input gradients [V, d_transfer] of the two row sets (parent rows / ego rows
+    through map1); d_transfer = g0.shape[1] (32, 64 or 128)."""
     _cuda(x, g0)
     x, g0, g1 = _c32(x), _c32(g0), None if g1 is None else _c32(g1)
     lib = _lib.load()
-    F, V0, V1 = x.shape[1], g0.shape[0], 0 if g1 is None else g1.shape[0]
-    dWt = torch.empty(DTR, F, device=x.device)
-    nbytes = lib.scgib_transfer_bwd_workspace_bytes(V0, V1, F)
+    F, DT, V0, V1 = x.shape[1], g0.shape[1], g0.shape[0], 0 if g1 is None else g1.shape[0]
+    if g1 is not None and g1.shape[1] != DT:
+        raise ValueError("transfer_bwd: g0 and g1 differ in width (%d, %d)" % (DT, g1.shape[1]))
+    dWt = torch.empty(DT, F, device=x.device)
+    nbytes = lib.scgib_transfer_bwd_workspace_bytes_d(V0, V1, F, DT)
     ws = torch.empty(int(nbytes) + 256, dtype=torch.uint8, device=x.device)
     off = (-ws.data_ptr()) % 256
     ip0, ix0 = csr0 if csr0 is not None else (None, None)
     ip1, ix1 = csr1 if csr1 is not None else (None, None)
-    _lib.check(lib.scgib_transfer_bwd_f32(_lib.ptr(x), F, int(normalize), _lib.ptr(g0), V0, _lib.ptr(ip0), _lib.ptr(ix0), _lib.ptr(g1), V1,
-                                          _lib.ptr(ip1), _lib.ptr(ix1), _lib.ptr(map1), _lib.ptr(dWt), ctypes.c_void_p(ws.data_ptr() + off),
-                                          int(nbytes), _stream(x)), "transfer_bwd")
+    _lib.check(lib.scgib_transfer_bwd_d_f32(_lib.ptr(x), F, DT, int(normalize), _lib.ptr(g0), V0, _lib.ptr(ip0), _lib.ptr(ix0), _lib.ptr(g1),
+                                            V1, _lib.ptr(ip1), _lib.ptr(ix1), _lib.ptr(map1), _lib.ptr(dWt),
+                                            ctypes.c_void_p(ws.data_ptr() + off), int(nbytes), _stream(x)), "transfer_bwd")
     return dWt
