@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libscgib.so")
 SOURCES = ["api.cu", "graph_kernels.cu", "gin_kernels.cu", "head_kernels.cu", "loss_kernels.cu", "finetune_kernels.cu",
-           "logm_kernels.cu", "peer_kernels.cu", "gin_tc3.cu", "gin_tc4.cu", "gin_bwd_tc2.cu", "gin_bwd_h.cu", "contrastive_tc.cu", "head_tc.cu", "gin_bf16.cu", "gin_bwd_bf16.cu", "encoder_ops.cu",
+           "logm_kernels.cu", "peer_kernels.cu", "gin_tc3.cu", "gin_tc4.cu", "gin_bwd_h.cu", "contrastive_tc.cu", "head_tc.cu", "gin_bf16.cu", "gin_bwd_bf16.cu", "encoder_ops.cu",
            "encoder_bf16.cu"]
 HEADERS = ["common.cuh", "kernels.cuh", "umma.cuh", "side_jobs.cuh", "scgib_private.h", os.path.join("..", "..", "include", "scgib.h")]
 # hardware probes of the tcgen05 operand formats: test infrastructure, NOT linked into the product library

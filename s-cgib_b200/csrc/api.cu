@@ -19,7 +19,7 @@ int num_sms() {
   return n;
 }
 
-// SCGIB_TC / SCGIB_TC_BWD: 1 (default) = the tcgen05 kernels (gin_tc3.cu / gin_bwd_tc2.cu), 0 = the FP32 FFMA
+// SCGIB_TC / SCGIB_TC_BWD: 1 (default) = the tcgen05 kernels (gin_tc3.cu / gin_bwd_h.cu), 0 = the FP32 FFMA
 // register-tile kernels of gin_kernels.cu (the cross-check implementation)
 static int g_use_tc = -1;
 int tensor_core_mode() {
@@ -31,20 +31,8 @@ int bwd_tensor_core_mode() {
   if (g_bwd_tc < 0) { const char* e = getenv("SCGIB_TC_BWD"); g_bwd_tc = (e && e[0] == '0') ? 0 : 1; }
   return g_bwd_tc;
 }
-// SCGIB_RECON_SIDE=1: the adjacency-reconstruction backward as side CTAs of the contrastive backward launch (measured: the
-// 20 SMs that launch leaves idle need longer for it than the separate 29 us launch on all SMs; default off)
-static bool recon_side_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SCGIB_RECON_SIDE"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v == 1;
-}
 // CTAs of recon_fwd (= its per-CTA partial Gram matrices): two resident CTAs per SM at hidden 64 overlap the copy / Gram / gather phases
 static int recon_fwd_grid() { return 2 * num_sms(); }
-static int g_bwd_h = -1;
-int bwd_h_mode() {
-  if (g_bwd_h < 0) { const char* e = getenv("SCGIB_BWD_H"); g_bwd_h = (e && e[0] == '0') ? 0 : 1; }
-  return g_bwd_h;
-}
 static int g_fwd4 = -1;
 int fwd_tc4_mode() {
   if (g_fwd4 < 0) { const char* e = getenv("SCGIB_FWD4"); g_fwd4 = (e && e[0] == '1') ? 1 : 0; }
@@ -496,13 +484,12 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
   const int GP = num_sms();
   const float s_kl = loss_scale[0], s_con = loss_scale[1], s_rec = loss_scale[2];
   const bool bf = d->act_dtype == SCGIB_ACT_BF16;
-  const bool tc_bwd = HID == 64 && bwd_tensor_core_mode() != 0;    // 3xTF32 tcgen05 backward (fp32 data): hidden 64; else FFMA tiles
+  const bool use_h = HID == 64 && bwd_tensor_core_mode() != 0;     // fp16-split tcgen05 backward (gin_bwd_h.cu): hidden 64; else FFMA tiles
   if (b->recon_logm_steps > 0 && HID != 64 && !gZ_ext) return SCGIB_E_SHAPE;
 
   cudaMemsetAsync(w.counters, 0, 64 * sizeof(float), s);
   // gin_bwd_h.cu (two-term fp16 splits) normalises the gradients of a launch by a power of two derived from max |g_o|: the kernel
   // that produces g_o leaves it in one of these slots (zeroed above) with an order-independent atomicMax
-  const bool use_h = tc_bwd && bwd_h_mode() != 0;
   unsigned int* gm_head = w.counters + 52;
   auto gm_layer = [&](int e, int l) { return w.counters + 40 + e * 6 + l; };
   const int js = contrastive_jsplit(b->B);
@@ -512,26 +499,18 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
     cudaMemsetAsync(w.g_core, 0, (size_t)b->B * HID * sizeof(float), s);
     cudaMemsetAsync(w.g_readout, 0, (size_t)b->B * HID * sizeof(float), s);
   } else {
-    // contrastive backward; its normalisation backward (contrastive_bwd_finalize) is fused into graph_gate_bwd below.  On the
-    // tcgen05 launch the adjacency-reconstruction backward rides along as side CTAs on the SMs the 128-row blocks leave idle.
+    // contrastive backward; its normalisation backward (contrastive_bwd_finalize) is fused into graph_gate_bwd below
     ContrastiveBwdArgs a{w.z1, w.z2, w.D, b->B, js, w.g1p, w.g2p};
     const bool con_tc = HID == 64 && use_tc_contrastive();
     const bool logm = b->recon_logm_steps > 0;
     ReconBwdArgs ra{w.Z, w.G, b->indptr, b->indices, b->N, s_rec, w.gZ};
     if (use_h && !logm) ra.gmax = gm_head;          // max |gZ| for the head backward's gradient normalisation (gin_bwd_h.cu)
-    if (con_tc) {
-      ConBwdSides sd;
-      const bool recon_side = !logm && recon_side_mode();
-      if (recon_side) { sd.recon = ra; sd.n_recon = max(1, num_sms() - ((b->B + 127) / 128) * js); }
-      PROF("contrastive_bwd_tc", launch_contrastive_bwd_tc_sides(a, w.zsplit, sd, s));
-      if (!logm && !recon_side) PROF("recon_bwd", launch_recon_bwd(ra, HID, s));
-    } else {
-      PROF("contrastive_bwd_ffma", launch_contrastive_bwd(a, HID, s));
-    }
+    if (con_tc) PROF("contrastive_bwd_tc", launch_contrastive_bwd_tc(a, w.zsplit, s));
+    else PROF("contrastive_bwd_ffma", launch_contrastive_bwd(a, HID, s));
     if (logm) {
       PROF("logm_bwd", launch_logm_bwd(w.Z, b->graph_ptr, b->indptr, b->indices, b->B, b->N, b->recon_logm_steps, w.logm_walks,
                                        s_rec, w.gZ, (int32_t*)(w.counters + 32), HID, s));
-    } else if (!con_tc) {
+    } else {
       PROF("recon_bwd", launch_recon_bwd(ra, HID, s));
     }
   }
@@ -539,8 +518,8 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
   // K = H inputs, so its backward is the GIN backward kernel run on both halves (problem 0: a = noisy, W1a -> gI[:, :H], dW1a,
   // dW2, db1, db2; problem 1: a = alpha C, W1b -> gI[:, H:], dW1b; its duplicate dW2 / bias partials are not reduced) with an
   // identity BatchNorm backward (g_y = gZ).  tcgen05 kernel: both problems in ONE launch (CTAs split); FFMA tiles: two launches.
-  const bool head_pair = tc_bwd || bf;         // one shared launch (CTAs split between the two K halves)
-  const int head_split = head_pair ? pair_split(GP, (b->N + 127) / 128, (b->N + 127) / 128) : GP;
+  const bool pair = use_h || bf;               // one shared launch (CTAs split between the two K halves / the two encoders)
+  const int head_split = pair ? pair_split(GP, (b->N + 127) / 128, (b->N + 127) / 128) : GP;
   {
     // (W1a / W1b / head_bn / head_cvec were prepared by the forward pass of this step: fwd_prep)
     if (bf) PROF("head_gz_bf16", launch_f32_to_bf16(w.gZ, w.gZ_bf, (size_t)b->N * HID, s));
@@ -565,8 +544,6 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
       PROF("head_bwd_bf16", launch_gin_bwd_main_bf16(m[0], &m[1], HID, HID, GP, s, true));
     } else if (use_h) {
       PROF("head_bwd_h", launch_gin_bwd_main_h_pair(m[0], m[1], HID, GP, s));
-    } else if (tc_bwd) {
-      PROF("head_bwd_tc", launch_gin_bwd_main_tc2_pair(m[0], m[1], HID, GP, s));
     } else {
       PROF("head_bwd_ffma.a", launch_gin_bwd_main(m[0], HID, HID, GP, s));
       PROF("head_bwd_ffma.b", launch_gin_bwd_main(m[1], HID, HID, GP, s));   // rewrites the (identical) dW2 / bias partials of .a
@@ -601,7 +578,6 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
     PROF("gate_lin_bwd", launch_gate_lin_bwd(a, HID, GP, s));
   }
   const int enc_split = pair_split(GP, (b->N + 127) / 128, (b->Ns + 127) / 128);   // CTAs of Encoder1 in a shared launch
-  const bool pair_main = bf || tc_bwd;
   for (int l = L - 1; l >= 0; --l) {
     const int kin = l == 0 ? DT : HID;
     GinBwdPreArgs pa[2];
@@ -635,8 +611,6 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
     PROF("gin_bwd_pre.enc1+2", launch_gin_bwd_pre_pair(pa[0], pa[1], HID, s));
     if (use_h) {
       PROF("gin_bwd_main_h.enc1+2", launch_gin_bwd_main_h_pair(ma[0], ma[1], kin, GP, s));
-    } else if (pair_main) {
-      PROF("gin_bwd_main_tc.enc1+2", launch_gin_bwd_main_tc2_pair(ma[0], ma[1], kin, GP, s));
     } else {
       PROF("gin_bwd_main_ffma.enc1", launch_gin_bwd_main(ma[0], kin, HID, GP, s));
       PROF("gin_bwd_main_ffma.enc2", launch_gin_bwd_main(ma[1], kin, HID, GP, s));
@@ -658,14 +632,14 @@ static int backward_impl(const ScgibDims* d, const float* params, const ScgibBat
     // reduction writes them interleaved as the parameter's [H][2H] layout.
     add(lo.off[SCGIB_P_HEAD_W1], (int64_t)HID * HID, 0, head_split);
     r.dst[r.n - 1] = lo.off[SCGIB_P_HEAD_W1]; r.ilv[r.n - 1] = HID;
-    add(lo.off[SCGIB_P_HEAD_W1] + (int64_t)HID * HID, (int64_t)HID * HID, head_pair ? head_split : 0, GP);
+    add(lo.off[SCGIB_P_HEAD_W1] + (int64_t)HID * HID, (int64_t)HID * HID, pair ? head_split : 0, GP);
     r.dst[r.n - 1] = lo.off[SCGIB_P_HEAD_W1] + HID; r.ilv[r.n - 1] = HID;
     add(lo.off[SCGIB_P_HEAD_B1], lo.off[SCGIB_P_HEAD_B2] + HID - lo.off[SCGIB_P_HEAD_B1], 0, head_split);
     add(lo.off[SCGIB_P_COMP_W1], lo.off[SCGIB_P_COMP_B1] + HID - lo.off[SCGIB_P_COMP_W1], 0, GP);
     for (int e = 0; e < 2; ++e)        // shared launches: partial rows [0, split) belong to Encoder1, [split, GP) to Encoder2
       for (int l = 0; l < L; ++l)
         add(lo.enc(e, l, L, SCGIB_ENC_W1), lo.enc(e, l, L, SCGIB_ENC_B2) + HID - lo.enc(e, l, L, SCGIB_ENC_W1),
-            pair_main ? (e == 0 ? 0 : enc_split) : 0, pair_main ? (e == 0 ? enc_split : GP) : GP);
+            pair ? (e == 0 ? 0 : enc_split) : 0, pair ? (e == 0 ? enc_split : GP) : GP);
     PROF("reduce_partials", launch_reduce_partials(w.ppart, lo.total, GP, r, grads, s));
   }
   return (int)cudaGetLastError();
@@ -950,7 +924,8 @@ extern "C" SCGIB_API int scgib_gin_layer_bwd_f32(const float* g_next, const int3
   q.src = g_next; q.indptr = indptr; q.indices = indptr ? indices : nullptr; q.map = nullptr;
   q.y = y; q.bn = bn; q.V = V; q.g_o = w.g_o; q.part = w.part2; q.counter = w.counter;
   q.d_gamma = dgamma; q.d_beta = dbeta; q.cvec = w.cvec;
-  const bool use_h = bwd_tensor_core_mode() != 0 && bwd_h_mode() != 0 && (((uintptr_t)y | (uintptr_t)r | (uintptr_t)a | (uintptr_t)g_a) & 31u) == 0;
+  // the tensor-core kernel reads and writes 32-byte row chunks: operands that are not 32-byte aligned go to the FFMA tiles
+  const bool use_h = bwd_tensor_core_mode() != 0 && (((uintptr_t)y | (uintptr_t)r | (uintptr_t)a | (uintptr_t)g_a) & 31u) == 0;
   q.gmax = use_h ? w.counter + 32 : nullptr;         // max |g_o| for the fp16-split kernel's gradient normalisation (zeroed above)
   launch_gin_bwd_pre(q, HID, s);
   GinBwdMainArgs m;
@@ -958,7 +933,6 @@ extern "C" SCGIB_API int scgib_gin_layer_bwd_f32(const float* g_next, const int3
   m.part = w.ppart; m.pstride = w.pstride; m.off_W1 = w.off[0]; m.off_b1 = w.off[1]; m.off_W2 = w.off[2]; m.off_b2 = w.off[3];
   m.gmax = w.counter + 32;
   if (use_h) launch_gin_bwd_main_h(m, kin, GP, s);
-  else if (bwd_tensor_core_mode() != 0) launch_gin_bwd_main_tc2(m, kin, GP, s);
   else launch_gin_bwd_main(m, kin, HID, GP, s);
   // per-CTA partials -> the four gradient tensors (fixed order)
   float* outs[4] = {dW1, db1, dW2, db2};
@@ -1304,7 +1278,7 @@ static HeadOpWs head_op_carve(int H, int N, void* base) {
   w.off[0] = 0; w.off[1] = (int64_t)2 * H * H; w.off[2] = w.off[1] + H; w.off[3] = w.off[2] + (int64_t)H * H;   // W1 b1 W2 b2
   w.pstride = w.off[3] + H;
   w.ppart = take((size_t)num_sms() * w.pstride);
-  w.xmax = (unsigned int*)take(4);
+  w.xmax = (unsigned int*)take(6);    // max |x| slots: noisy, C, alpha (forward); gZ, alpha C, r (backward)
   w.bytes = o;
   return w;
 }
@@ -1346,6 +1320,7 @@ extern "C" SCGIB_API int scgib_head_mlp_fwd_f32(const float* noisy, const float*
 }
 
 // gI [N, 2H] = d<gZ, Z>/d interaction_map (first half: noisy, second half: alpha C); call after the forward with the same workspace
+// and the same noisy
 extern "C" SCGIB_API int scgib_head_mlp_bwd_f32(const float* gZ, const float* noisy, int32_t N, int32_t hidden, const float* W1,
                                       const float* W2, float* gI, float* dW1, float* db1, float* dW2, float* db2, void* workspace,
                                       size_t workspace_bytes, void* stream_) {
@@ -1357,7 +1332,9 @@ extern "C" SCGIB_API int scgib_head_mlp_bwd_f32(const float* gZ, const float* no
   if (workspace_bytes < w.bytes) return SCGIB_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream_;
   const int H = hidden, GP = num_sms();
-  const bool tc = H == 64 && bwd_tensor_core_mode() != 0;
+  // the tensor-core kernel reads and writes 32-byte row chunks: operands that are not 32-byte aligned go to the FFMA tiles
+  const bool tc = H == 64 && bwd_tensor_core_mode() != 0 && (((uintptr_t)gZ | (uintptr_t)noisy | (uintptr_t)gI) & 31u) == 0;
+  if (tc) cudaMemsetAsync(w.xmax + 3, 0, 3 * sizeof(unsigned int), s);
   launch_head_bwd_prep(W1, w.w1a, w.w1b, w.bnid, w.cvec, H, s);
   // the GIN backward kernel on the two K = H halves of the first layer (identity BatchNorm backward: g_y = gZ; its `y` operand
   // only enters multiplied by zero).  gI is returned as two dense halves [2][N][H]: gradient wrt noisy, then wrt alpha C.
@@ -1371,7 +1348,13 @@ extern "C" SCGIB_API int scgib_head_mlp_bwd_f32(const float* gZ, const float* no
   }
   int split = GP;
   if (tc) {
-    launch_gin_bwd_main_tc2_pair(m[0], m[1], H, GP, s, true);
+    // any input magnitude (GraphSAGE / GCN features are unbounded): gZ, the a operands and r get power-of-two pre-scales from
+    // their maxima (max |noisy| is the forward's)
+    launch_absmax(gZ, (size_t)N * H, w.xmax + 3, s);
+    launch_absmax(w.aC, (size_t)N * H, w.xmax + 4, s);
+    launch_absmax(w.r, (size_t)N * H, w.xmax + 5, s);
+    for (int h = 0; h < 2; ++h) { m[h].gmax = w.xmax + 3; m[h].amax = h == 0 ? w.xmax : w.xmax + 4; m[h].rmax = w.xmax + 5; }
+    launch_gin_bwd_main_h_pair(m[0], m[1], H, GP, s);
     split = pair_split(GP, (N + 127) / 128, (N + 127) / 128);
   } else {
     launch_gin_bwd_main(m[0], H, H, GP, s);

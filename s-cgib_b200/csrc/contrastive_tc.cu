@@ -12,7 +12,7 @@
 // 2^k ~ B into fp16's normal range, un-scaled exactly at the end) are split the same way in registers and handed to the
 // P Z GEMMs through TENSOR MEMORY (16-bit A operand: two K values per column), double-buffered.
 // Roles: 8 worker warps (copies, exp / P epilogues, results) + ONE MMA-issuing warp; every hand-off is an mbarrier.
-// Side jobs of other kernels ride along as extra CTAs (ConFwdSides / ConBwdSides, kernels.cuh).
+// Side jobs of other kernels ride along the forward as extra CTAs (ConFwdSides, kernels.cuh).
 #include "kernels.cuh"
 #include "umma.cuh"
 #include "side_jobs.cuh"
@@ -229,23 +229,16 @@ struct ConBwdTcLayout {
   static constexpr int off_di = off_zj + 2 * kStage16;        // float [128]
   static constexpr int off_dj = off_di + CI * 4;              // float [2][64]
   static constexpr int off_bar = off_dj + 2 * CJ * 4;         // tile[2], sim[2], p[2], pv[2] + tmem slot
-  static constexpr int total_main = off_bar + 128;
-  static constexpr int total = total_main > (int)sizeof(ReconBwdSmem<HID>) ? total_main : (int)sizeof(ReconBwdSmem<HID>);
+  static constexpr int total = off_bar + 128;
 };
 enum { CB_TILE = 0, CB_SIM = 2, CB_P = 4, CB_PV = 6 };
 
 __global__ void __launch_bounds__(kConThreads, 1)
-contrastive_bwd_tc_kernel(ContrastiveBwdArgs p, const float* __restrict__ zsplit, ConBwdSides sd, int iblocks, float pscale) {
+contrastive_bwd_tc_kernel(ContrastiveBwdArgs p, const float* __restrict__ zsplit, int iblocks, float pscale) {
   pdl_sync();
   using L = ConBwdTcLayout;
   extern __shared__ __align__(1024) unsigned char smem[];
-  const int nmain = iblocks * p.jsplit;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if ((int)blockIdx.x >= nmain) {          // side CTAs: the adjacency-reconstruction backward (independent of this kernel's work)
-    if (warp >= kSideWarps) return;        // (its body is written for kThreads threads)
-    recon_bwd_body<HID>(sd.recon, smem, (int)blockIdx.x - nmain, sd.n_recon);
-    return;
-  }
   const int bx = (int)blockIdx.x % iblocks, by = (int)blockIdx.x / iblocks, gy = p.jsplit;
   unsigned char* zi = smem + L::off_zi;
   unsigned char* zj = smem + L::off_zj;
@@ -476,16 +469,13 @@ void launch_contrastive_fwd_tc_sides(const ContrastiveFwdArgs& a, const ConFwdSi
 }
 void launch_contrastive_fwd_tc(const ContrastiveFwdArgs& a, cudaStream_t s) { launch_contrastive_fwd_tc_sides(a, ConFwdSides{}, s); }
 
-void launch_contrastive_bwd_tc_sides(const ContrastiveBwdArgs& a, const float* zsplit, const ConBwdSides& sides, cudaStream_t s) {
+void launch_contrastive_bwd_tc(const ContrastiveBwdArgs& a, const float* zsplit, cudaStream_t s) {
   static bool once = (cudaFuncSetAttribute(contrastive_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            ConBwdTcLayout::total), true);
   (void)once;
   const int iblocks = (a.B + CI - 1) / CI;
-  const int grid = iblocks * a.jsplit + sides.n_recon;
-  launch_k((contrastive_bwd_tc_kernel), dim3(grid), dim3(kConThreads), ConBwdTcLayout::total, s, a, zsplit, sides, iblocks, con_pscale(a.B));
-}
-void launch_contrastive_bwd_tc(const ContrastiveBwdArgs& a, const float* zsplit, cudaStream_t s) {
-  launch_contrastive_bwd_tc_sides(a, zsplit, ConBwdSides{}, s);
+  launch_k((contrastive_bwd_tc_kernel), dim3(iblocks * a.jsplit), dim3(kConThreads), ConBwdTcLayout::total, s, a, zsplit, iblocks,
+           con_pscale(a.B));
 }
 
 }  // namespace scgib

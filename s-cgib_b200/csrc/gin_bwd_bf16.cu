@@ -1,6 +1,6 @@
 // gin_bwd_bf16.cu - GIN layer BACKWARD in bf16 mode (ScgibDims.act_dtype = SCGIB_ACT_BF16), hidden width H = 64 or 128.
 //
-// Same math as gin_bwd_pre_kernel + gin_bwd_tc2 (reference: autograd of models.py:66-72), on bf16 activations / layer
+// Same math as gin_bwd_pre_kernel + gin_bwd_h (reference: autograd of models.py:66-72), on bf16 activations / layer
 // gradients with fp32 accumulation everywhere:
 //   pre : G_v = Ga_v + sum_{u in N(v)} Ga_u (bf16x8 gathers through the symmetric CSR; top layer: fp32 rows through a map),
 //         g_o = G * [relu(BN(y)) > 0] -> bf16, d gamma / d beta (of the ROUNDED g_o, so that the BatchNorm backward

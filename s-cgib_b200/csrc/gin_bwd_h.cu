@@ -1,22 +1,23 @@
 // gin_bwd_h.cu - GIN layer backward (part 2) on tcgen05 with TWO-TERM FP16 operand splits: 128-row tiles, K = 16 MMAs.
 //
-// Same contract and math as gin_bwd_tc2.cu (reference: autograd of models.py:66-72), every GIN layer (the 32-wide layer 0 runs
-// zero-padded to 64 input channels) and the head MLP:
+// Reference: autograd of models.py:66-72.  Runs every fp32 GIN layer at hidden 64 (the 32-wide layer 0 runs zero-padded to
+// 64 input channels), the head MLP and, in half mode, the compressor's first linear layer:
 //   g_y = rstd * (gamma*g_o - c1 - yhat*c2);  G1: g_r = g_y W2;  G3: dW2 += g_y^T r;  g_u = g_r * [r > 0];
 //   G2: g_a = g_u W1;  G4: dW1 += g_u^T a;  db2 += sum g_y;  db1 += sum g_u.
-// gin_bwd_tc2 (3xTF32, K = 8 per MMA, 64-row tiles: 64 MMAs per 64 rows) is bound by the per-tile dependency chain and the
-// ~54-cycle cost of each small MMA.  Here every operand is a two-term fp16 split (22 significand bits, as the 3xTF32 products):
+// Every operand is a two-term fp16 split (22 significand bits, the precision of 3xTF32 products at twice the K per MMA):
 //   * forward activations r, a and the weights (x 2^4): v = hi + lo, lo = fp16(v - hi) UNSCALED (|v| = O(1): absolute error
-//     <= 2^-25), so their hi and lo products accumulate into the SAME columns;
+//     <= 2^-25), so their hi and lo products accumulate into the SAME columns.  Where a and r are not O(1) (the head MLP
+//     operator: GraphSAGE / GCN features are unbounded) the caller leaves max |a| and max |r| in device slots, and a, r are
+//     first normalised by powers of two Sa, Sr as the gradients below; dW1 / dW2 undo them where they leave tensor memory;
 //   * gradients g_y, g_u: first normalised by a power of two S (max |g| of the launch -> ~2^8: the producing kernel leaves
 //     max |g_o| in a device slot by an order-independent atomicMax, the BN-backward factors are known here), then
 //     v = hi + 2^-11 lo' with the residual SCALED into fp16's normal range: small gradient entries keep their relative
 //     precision; the lo' products land in separate accumulator columns / TMEM lanes and are folded in with 2^-11 by the epilogues.
-// A 128-row tile then needs 12 + 16 + 12 + 16 = 56 kind::f16 MMAs (K = 16) instead of 128, its fp16 tiles are half the bytes
-// (two 128-row stages in the shared memory the 64-row fp32 stages took), and UMMA M = 128 uses all 128 TMEM lanes (8 epilogue
-// warps: lane quarter x 32-column half).  All scalings are exact powers of
-// two, undone exactly.  Roles: 8 epilogue warps, 1 MMA warp, 16 loader warps (the role timeline showed the loaders' dependent
-// 32-byte row loads as the serial bottleneck of a tile: 6 us with 8 warps); hand-offs are mbarriers with one arrival per warp.
+// A 128-row tile needs 12 + 16 + 12 + 16 = 56 kind::f16 MMAs (K = 16), two 128-row stages of fp16 tiles fit in shared
+// memory, and UMMA M = 128 uses all 128 TMEM lanes (8 epilogue warps: lane quarter x 32-column half).  All scalings are exact
+// powers of two, undone exactly.  Roles: 8 epilogue warps, 1 MMA warp, 16 loader warps (the role timeline showed the loaders'
+// dependent 32-byte row loads as the serial bottleneck of a tile: 6 us with 8 warps); hand-offs are mbarriers with one arrival
+// per warp.
 #include <stdlib.h>
 #include "kernels.cuh"
 #include "umma.cuh"
@@ -68,6 +69,14 @@ __device__ __forceinline__ void ld8cs(const float* p, float* v) {
                "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]) : "l"(p));
 }
 __device__ __forceinline__ float clamp16(float v) { return fminf(fmaxf(v, -65504.f), 65504.f); }
+// the power of two 2^(8 - e) for bound = m * 2^e (m in [0.5, 1)): it takes the bound into [2^7, 2^8); 1 for a bound of 0 or inf
+__device__ __forceinline__ float pow2_norm(float bound) {
+  if (!(bound > 0.f && bound < 3.0e38f)) return 1.f;
+  int e;
+  (void)frexpf(bound, &e);
+  return exp2f((float)max(-100, min(100, 8 - e)));
+}
+__device__ __forceinline__ float slot_norm(const unsigned int* slot) { return slot ? pow2_norm(__uint_as_float(__ldcg(slot))) : 1.f; }
 
 // transposed weight tile for the input-gradient GEMMs: B[n = input channel][k = output channel] = 16 W[out][in], fp16 hi / lo
 // (`in` < 64 input channels: the missing rows of the tile are zero)
@@ -107,7 +116,10 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_tiles = (p.V + TM - 1) / TM;
   const int my_tiles = max(0, (n_tiles - bid + nblk - 1) / nblk);
-  const bool rev = pp.reverse != 0;                           // descending row order: see gin_bwd_tc2.cu
+  // descending row order: gin_bwd_pre (the previous launch) walks ascending, so the rows it touched last (g_o just written,
+  // y just read) are still in L2 when this kernel starts, and the g_a rows written last here (the lowest) are the ones the
+  // next layer's gin_bwd_pre gathers first
+  const bool rev = pp.reverse != 0;
   const bool trace_on = pp.trace != 0;
   auto tile_base = [&](int i) { return (bid + (rev ? my_tiles - 1 - i : i) * nblk) * TM; };
   auto Xs = [&](int s) { return smem + L::off_stage + s * kStage; };
@@ -142,19 +154,12 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
   const uint32_t tmem = *s_tmem;
   // gradient normalisation: S = 2^e with S * max|g_o| * max|ka| in [2^7, 2^8): the other BN-backward terms are of the same order
   // and g_u = g_r * mask sums 64 weighted terms, so fp16's 2^16 keeps 2^8 of headroom (values are clamped to the fp16 range
-  // before conversion), while entries down to 2^-22 of the largest one keep the full 22-bit two-term precision
-  float S = 1.f;
-  {
-    float kamax = 0.f;
-    for (int c = 0; c < HID; ++c) kamax = fmaxf(kamax, fabsf(s_k[c]));
-    const float gmax = p.gmax ? __uint_as_float(__ldcg(p.gmax)) : 0.f;
-    const float bound = gmax * kamax;
-    if (bound > 0.f && bound < 3.0e38f) {
-      int e;
-      (void)frexpf(bound, &e);                               // bound = m * 2^e, m in [0.5, 1)
-      S = exp2f((float)max(-100, min(100, 8 - e)));
-    }
-  }
+  // before conversion), while entries down to 2^-22 of the largest one keep the full 22-bit two-term precision.  Sa, Sr: the
+  // same rule for a and r (1 without a slot); g_a, db1, db2 and the r > 0 mask do not depend on them.
+  float kamax = 0.f;
+  for (int c = 0; c < HID; ++c) kamax = fmaxf(kamax, fabsf(s_k[c]));
+  const float S = pow2_norm((p.gmax ? __uint_as_float(__ldcg(p.gmax)) : 0.f) * kamax);
+  const float Sa = slot_norm(p.amax), Sr = slot_norm(p.rmax);
   const float invS = 1.f / S;
 
   float* s_db1 = reinterpret_cast<float*>(smem + L::off_db1);
@@ -219,7 +224,7 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
           split_f16x2_s11(gy[2], gy[3], hi[2 * h + 1], lo[2 * h + 1]);
         }
 #pragma unroll
-        for (int q = 0; q < 4; ++q) split_f16x2_plain(fminf(rr[0][2 * q], 65504.f), fminf(rr[0][2 * q + 1], 65504.f), rh[q], rl[q]);
+        for (int q = 0; q < 4; ++q) split_f16x2_plain(fminf(rr[0][2 * q] * Sr, 65504.f), fminf(rr[0][2 * q + 1] * Sr, 65504.f), rh[q], rl[q]);
         const int off = tile_b_off(row, c8);
         *reinterpret_cast<uint4*>(X + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
         *reinterpret_cast<uint4*>(X + kTile + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
@@ -261,7 +266,7 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
       for (int j = 0; j < UPT; ++j) {
         uint32_t hi[4], lo[4];
 #pragma unroll
-        for (int q = 0; q < 4; ++q) split_f16x2_plain(clamp16(aa[j][2 * q]), clamp16(aa[j][2 * q + 1]), hi[q], lo[q]);
+        for (int q = 0; q < 4; ++q) split_f16x2_plain(clamp16(aa[j][2 * q] * Sa), clamp16(aa[j][2 * q + 1] * Sa), hi[q], lo[q]);
         const int off = tile_b_off(r0 + RPP * j, c8);
         *reinterpret_cast<uint4*>(Y + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
         *reinterpret_cast<uint4*>(Y + kTile + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
@@ -441,11 +446,12 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
   fence_after_sync();
   float* part = p.part + (size_t)blockIdx.x * p.pstride;
   // dW2 / dW1 from tensor memory: accumulator row L (TMEM lane L): L < 64 = hi part of out-channel L, L >= 64 = lo' part of
-  // out-channel L - 64 (both summed over B_hi + B_lo).  dW[o][i] = (row o + 2^-11 row 64 + o) / S.
+  // out-channel L - 64 (both summed over B_hi + B_lo).  dW2[o][i] = (row o + 2^-11 row 64 + o) / (S Sr), dW1: / (S Sa).
   float* s_x = reinterpret_cast<float*>(smem);          // [64][HID + 1] exchange buffer (the stages are dead)
   for (int pass = 0; pass < (half_mode ? 1 : 2); ++pass) {   // pass 0: dW2, pass 1: dW1
     const uint32_t col = pass == 0 ? kColD3 : kColD4;
     const int64_t offW = pass == 0 ? p.off_W2 : p.off_W1;
+    const float kW = invS * (1.f / (pass == 0 ? Sr : Sa));
     float t[64];
     if (warp < 4) {
       const uint32_t tl = (uint32_t)(warp * 32) << 16;
@@ -468,8 +474,8 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
       const int o = warp * 32 + lane;
       for (int j = 0; j < C; j += 4) {
         float4 v;
-        v.x = fmaf(s_x[o * (HID + 1) + j], kLo, t[j]) * invS;         v.y = fmaf(s_x[o * (HID + 1) + j + 1], kLo, t[j + 1]) * invS;
-        v.z = fmaf(s_x[o * (HID + 1) + j + 2], kLo, t[j + 2]) * invS; v.w = fmaf(s_x[o * (HID + 1) + j + 3], kLo, t[j + 3]) * invS;
+        v.x = fmaf(s_x[o * (HID + 1) + j], kLo, t[j]) * kW;         v.y = fmaf(s_x[o * (HID + 1) + j + 1], kLo, t[j + 1]) * kW;
+        v.z = fmaf(s_x[o * (HID + 1) + j + 2], kLo, t[j + 2]) * kW; v.w = fmaf(s_x[o * (HID + 1) + j + 3], kLo, t[j + 3]) * kW;
         st4(part + offW + (size_t)o * C + j, v);
       }
     }
@@ -496,7 +502,8 @@ gin_bwd_h_kernel(GinBwdMainPair pp) {
 }  // namespace bwdh
 
 // the same layer of both encoders (or the two K halves of the head MLP) in one launch: CTAs [0, split) write the partial
-// gradients of a0, [split, grid) of a1 (split as computed by pair_split on 128-row tile counts, as gin_bwd_tc2)
+// gradients of a0, [split, grid) of a1 (split = pair_split on the 128-row tile counts: the callers' partial-sum reduction
+// ranges use the same rule)
 void launch_gin_bwd_main_h_pair(const GinBwdMainArgs& a0, const GinBwdMainArgs& a1, int kin, int grid, cudaStream_t s, bool weights_from_prev_kernel) {
   static bool once = (cudaFuncSetAttribute(bwdh::gin_bwd_h_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bwdh::Smem::total), true);
   (void)once;

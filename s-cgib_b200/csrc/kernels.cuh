@@ -98,6 +98,8 @@ struct GinBwdMainArgs {
   int64_t pstride;
   int64_t off_W1, off_b1, off_W2, off_b2;
   const unsigned int* gmax = nullptr;   // gin_bwd_h: bits of max |g_o| (left by the kernel that produced g_o)
+  const unsigned int* amax = nullptr;   // gin_bwd_h: bits of max |a| and max |r| (same encoding); null: |a|, |r| = O(1), no
+  const unsigned int* rmax = nullptr;   //  pre-scale (inputs after a BatchNorm)
 };
 void launch_gin_bwd_main(const GinBwdMainArgs& a, int kin, int hidden, int grid, cudaStream_t s);      // FP32 FFMA tiles, hidden 64 / 128
 struct GinBwdMainPair {
@@ -107,9 +109,6 @@ struct GinBwdMainPair {
   int wait_first = 0;       // PDL: W1 / W2 are written by the kernel launched right before this one (the head backward's de-interleaved
                             //  W1 halves): wait for it before staging the weights instead of after
 };
-void launch_gin_bwd_main_tc2(const GinBwdMainArgs& a, int kin, int grid, cudaStream_t s);  // tcgen05 3xTF32, 64-row double-buffered tiles (gin_bwd_tc2.cu)
-void launch_gin_bwd_main_tc2_pair(const GinBwdMainArgs& a0, const GinBwdMainArgs& a1, int kin, int grid, cudaStream_t s,
-                                  bool weights_from_prev_kernel = false);
 int gin_bwd_pre_bf16_grid(int V, int hidden);
 void launch_gin_bwd_pre_bf16(const GinBwdPreArgs& a0, const GinBwdPreArgs* a1, int hidden, cudaStream_t s);
 void launch_gin_bwd_main_bf16(const GinBwdMainArgs& a0, const GinBwdMainArgs* a1, int kin, int hidden, int grid, cudaStream_t s,
@@ -120,8 +119,7 @@ void launch_gin_bwd_main_h(const GinBwdMainArgs& a, int kin, int grid, cudaStrea
 void launch_linear_bwd_h(const float* g, const float* x, const float* W, int V, float* g_in, const float* bn_identity, const float* cvec_zero,
                          const unsigned int* gmax, float* part, int64_t pstride, int64_t off_W, int64_t off_b, int grid, cudaStream_t s);
 void launch_absmax(const float* x, size_t n, unsigned int* slot, cudaStream_t s);   // atomicMax(slot, bits of max |x|)
-int bwd_h_mode();                                                          // SCGIB_BWD_H: 1 (default) gin_bwd_h.cu for the KIN = 64 layers and the head
-int bwd_tensor_core_mode();                                                                // SCGIB_TC_BWD: 1 gin_bwd_tc2.cu (default), 0 FFMA cross-check
+int bwd_tensor_core_mode();                                                                // SCGIB_TC_BWD: 1 gin_bwd_h.cu (default), 0 FFMA cross-check
 
 struct InputProjBwdArgs {
   const float* ga[2];       // layer-0 input gradients of the two encoders, [V][DT]
@@ -314,21 +312,18 @@ struct LossFinalizeArgs {
 };
 void launch_loss_finalize(const LossFinalizeArgs& a, cudaStream_t s);
 
-// Horizontal fusion of the step's small serial jobs: the tcgen05 contrastive kernels run one CTA per SM on 128-row blocks
-// and leave SMs idle (128 of 148 CTAs at B = 4096), so independent latency-bound jobs of the same phase ride along as
-// EXTRA CTAs of those launches (side_jobs.cuh) instead of paying a launch + drain each:
-//   forward : recon_reduce (n_reduce CTAs), compressor_ema (n_ema = 0 | 1 CTA), and loss_finalize run by whichever CTA
-//             of the launch finishes last (`counter`, self-resetting);
-//   backward: recon_bwd (n_recon CTAs walking all row tiles).
+// Horizontal fusion of the step's small serial jobs: the tcgen05 contrastive forward runs one CTA per SM on 128-row blocks
+// and leaves SMs idle (128 of 148 CTAs at B = 4096), so independent latency-bound jobs of the same phase ride along as
+// EXTRA CTAs of that launch (side_jobs.cuh) instead of paying a launch + drain each: recon_reduce (n_reduce CTAs),
+// compressor_ema (n_ema = 0 | 1 CTA), and loss_finalize run by whichever CTA of the launch finishes last (`counter`,
+// self-resetting).
 constexpr int kConSideCtas = 12;          // SMs contrastive_jsplit() leaves to the side jobs
 struct ConFwdSides {
   const float* rpart = nullptr; int rgrid = 0; float* G = nullptr; float* edge = nullptr; int n_reduce = 0;
   const float* cstat = nullptr; float* running = nullptr; int n_ema = 0;
   int finalize = 0; LossFinalizeArgs fin; unsigned int* counter = nullptr;
 };
-struct ConBwdSides { int n_recon = 0; ReconBwdArgs recon; };
 void launch_contrastive_fwd_tc_sides(const ContrastiveFwdArgs& a, const ConFwdSides& sides, cudaStream_t s);
-void launch_contrastive_bwd_tc_sides(const ContrastiveBwdArgs& a, const float* zsplit, const ConBwdSides& sides, cudaStream_t s);
 
 // grads[off..off+len) = sum_c part[c*pstride + off + i] for each listed range
 // partial rows [c0, c1) hold the range; ilv > 0: element i of the range goes to dst + (i / ilv) * 2 * ilv + i % ilv instead of

@@ -12,14 +12,14 @@ extern "C" {
 /* GIN forward: 1 = tcgen05 kernels (gin_tc3.cu fp32 / gin_bf16.cu bf16; default), 0 = FP32 FFMA register tiles
  * (gin_kernels.cu).  Also the environment variable SCGIB_TC; mode < 0 restores the default. */
 SCGIB_API void scgib_set_tensor_cores(int mode);
-/* GIN backward: 1 = tcgen05 (gin_bwd_tc2.cu; default), 0 = FFMA; environment variable SCGIB_TC_BWD. */
+/* fp32 GIN, head MLP and compressor backward at hidden 64: 1 = tcgen05 two-term fp16 splits (gin_bwd_h.cu; default),
+ * 0 = FP32 FFMA register tiles (gin_kernels.cu).  Also the environment variable SCGIB_TC_BWD; mode < 0 restores the default. */
 SCGIB_API void scgib_set_tensor_cores_bwd(int mode);
 /* Per-tile role timestamps of the last gin_fwd_tc3 launch run with SCGIB_DBG bit 1024
- * ([cta < 160][tile < 16][event < 12] SM clocks) copied to host memory; bit 2048: the same for gin_bwd_tc2. */
+ * ([cta < 160][tile < 16][event < 12] SM clocks) copied to host memory. */
 SCGIB_API int scgib_debug_tc2_trace(long long* host_out, int n);
-SCGIB_API int scgib_debug_bwd_trace(long long* host_out, int n);
 SCGIB_API int scgib_debug_bf16_trace(long long* host_out, int n);     /* gin_fwd_bf16 (bf16 mode), same layout */
-SCGIB_API int scgib_debug_bwdh_trace(long long* host_out, int n);     /* gin_bwd_h (SCGIB_DBG bit 2048), layout of scgib_debug_bwd_trace */
+SCGIB_API int scgib_debug_bwdh_trace(long long* host_out, int n);     /* gin_bwd_h (SCGIB_DBG bit 2048), same layout */
 SCGIB_API int scgib_debug_tc4_trace(long long* host_out, int n);      /* gin_fwd_tc4: [cta < 160][tile < 16][event < 16] */
 #ifdef __cplusplus
 }

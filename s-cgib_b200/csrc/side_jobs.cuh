@@ -1,6 +1,6 @@
 // side_jobs.cuh - device bodies of the step's small serial jobs, shared by their stand-alone kernels (loss_kernels.cu,
-// head_kernels.cu: op-level C ABI, FFMA / hidden-128 paths) and by the tcgen05 contrastive launches, where they run as
-// EXTRA CTAs on the SMs those launches leave idle (ConFwdSides / ConBwdSides, kernels.cuh).
+// head_kernels.cu: op-level C ABI, FFMA / hidden-128 paths) and, for the forward jobs, by the tcgen05 contrastive forward
+// launch, where they run as EXTRA CTAs on the SMs that launch leaves idle (ConFwdSides, kernels.cuh).
 //
 // Reference call sites replaced: loss_recon_adj (models.py:762-768, Gram identity), the compressor BatchNorm's B sequential
 // running-statistics updates (models.py:642 per graph), KL + recon + contrastive (exp_pretraining.py:321).

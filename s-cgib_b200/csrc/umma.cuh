@@ -197,14 +197,9 @@ __device__ __forceinline__ void mma_tf32_ta(uint32_t d_tmem, uint32_t a_tmem, ui
 
 // Format-S tile ([halves of 32 columns][R rows][128 B], 32-byte chunks XOR-swizzled with row % 4) read as a K-MAJOR
 // operand (MN index = tile row, K index = column): layout type SWIZZLE_128B_BASE32B, SBO = 512, LBO = half stride;
-// K step s (8 columns = 32 B) starts at half s/4, byte 32*(s%4) of the row.  Measured on B200 (tests/gpu_umma_probe2.py):
-// the same physical tile therefore serves both contractions of a backward pass (over columns and over rows).
+// K step s (8 columns = 32 B) starts at half s/4, byte 32*(s%4) of the row (measured on B200: tests/gpu_umma_probe2.py).
 __device__ __forceinline__ uint64_t desc_s_kmajor(uint32_t tile, int R, int s) {
   return desc_base(tile + (uint32_t)(s >> 2) * (uint32_t)(R * 128) + (uint32_t)(s & 3) * 32u, (uint32_t)R * 128u, 512u) | ((uint64_t)1 << 61);
-}
-// ... and as an MN-MAJOR operand (MN index = column, K index = tile row): K step s covers rows 8s..8s+7
-__device__ __forceinline__ uint64_t desc_s_mnmajor(uint32_t tile, int R, int s) {
-  return desc_base(tile + (uint32_t)s * 1024u, (uint32_t)R * 128u, 512u) | ((uint64_t)1 << 61);
 }
 // dense format-G weight tile [n rows][C cols] (128-byte cores) as the K-major B operand, K step s
 __device__ __forceinline__ uint64_t desc_g_dense(uint32_t tile, int C, int s) {

@@ -3,7 +3,7 @@
 Operators: the input projection (fp32 and bf16 output) and the transfer_d weight gradient (parent and ego rows, with and
 without the CSR) at d in {64, 128}.  Whole steps: GIN pre-training at (hidden, d) in {(64, 64), (128, 64), (128, 128)} in
 fp32 and bf16, with the adjacency and logM losses and 5 GIN layers, bit-identical reruns, and the FFMA cross-check kernels
-(SCGIB_TC=0 SCGIB_TC_BWD=0, SCGIB_BWD_H=0) in a subprocess each, since the switches are read once per process.
+(SCGIB_TC=0 SCGIB_TC_BWD=0) in a subprocess, since the switches are read once per process.
 GraphSAGE / GCN pre-training, eval-mode features, fine-tuning and domain adaptation around checkpoints pre-trained at
 d = 64, and the two CLIs with --d_transfer 64.
 
@@ -207,7 +207,7 @@ def test_gin_pretrain_step_d_5_layers(H, d, dtype):
     _with_flip_retries(_pretrain_case, 620 + H + d, H, d, 1, dtype, layers=5)
 
 
-@pytest.mark.parametrize("env", [{"SCGIB_TC": "0", "SCGIB_TC_BWD": "0"}, {"SCGIB_BWD_H": "0"}], ids=["ffma", "bwd_tc2"])
+@pytest.mark.parametrize("env", [{"SCGIB_TC": "0", "SCGIB_TC_BWD": "0"}], ids=["ffma"])
 def test_gin_pretrain_step_d_cross_check_kernels(env):
     """The cross-check implementations at the new layer-0 widths: the fp32 whole-step cases of this file, in a process
     that reads the switches."""

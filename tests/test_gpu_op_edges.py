@@ -253,7 +253,8 @@ def test_core_cand_attention_edges(kind, logits, H):
 
 # ------------------------------------------------------------------------------------------------ head MLP
 def _offset_copy(t):
-    """The same values in a view whose data pointer is 16 (not 32) bytes past an allocation: the FFMA branch at hidden 64."""
+    """The same values in a view whose data pointer is 16 (not 32) bytes past an allocation: the FFMA branch at hidden 64
+    (the tensor-core kernels read 32-byte row chunks)."""
     buf = torch.empty(t.numel() + 4, device=DEV)
     v = buf[4:].view(t.shape)
     v.copy_(t)
@@ -297,7 +298,7 @@ def test_head_mlp_edges(scale, N, H):
     op = ops.HeadMLP(H, _f(mlp[0].weight), _f(mlp[0].bias), _f(mlp[2].weight), _f(mlp[2].bias))
     branches = [("aligned", lambda t: t)] + ([("offset16", _offset_copy)] if H == 64 else [])
     Zs = {}
-    for br, place in branches:                   # hidden 64: aligned operands run head_tc.cu, 16-byte offsets the FFMA tiles
+    for br, place in branches:                   # hidden 64: aligned operands run head_tc.cu / gin_bwd_h, 16-byte offsets the FFMA tiles
         Zg, ig = op.forward(place(_f(noisy)), place(_f(C)), _f(alpha))
         Zs[br] = Zg.clone()
         assert rel(Zg, Z) <= 1e-5 and rel(ig, imap) <= 1e-6, (br, rel(Zg, Z), rel(ig, imap))
@@ -316,7 +317,8 @@ def test_head_mlp_edges(scale, N, H):
 @pytest.mark.parametrize("g_scale", [1e-6, 1e4])
 def test_gin_layer_backward_magnitudes(kin, csr, act_scale, g_scale):
     """scgib_gin_layer_bwd_f32 with the forward activations a, r and the upstream gradient far from 1 (the fp16-split kernel
-    scales the gradients by a power of two and splits a, r as they are)."""
+    scales the gradients by a power of two and splits a, r as they are), on 32-byte aligned operands (gin_bwd_h) and on
+    operands 16 bytes off (the FFMA tiles)."""
     from scgib_b200 import ops
     from oracle.scgib_oracle import GINConvRef, MLP
     g = synth_batch(5, 400)
@@ -346,17 +348,18 @@ def test_gin_layer_backward_magnitudes(kin, csr, act_scale, g_scale):
     mean, var = y_in.detach().mean(0), y_in.detach().var(0, unbiased=False)
     bn = torch.stack([mean, 1.0 / torch.sqrt(var + BN_EPS), bnm.weight.detach(), bnm.bias.detach()]).float().to(DEV)
     pg = product_graph(g, DEV)
-    res = ops.gin_layer_bwd(_f(g_up), _f(y_in), _f(r_ref), _f(a_ref), bn, _f(lin1.weight), _f(lin2.weight),
-                            indptr=pg.indptr if csr else None, indices=pg.indices if csr else None)
-    torch.cuda.synchronize()
     want = (a_ref.grad, lin1.weight.grad, lin1.bias.grad, lin2.weight.grad, lin2.bias.grad, bnm.weight.grad, bnm.bias.grad)
     names = ("g_a", "dW1", "db1", "dW2", "db2", "dgamma", "dbeta")
     gmax = max(float(w.abs().max()) for w in want)
-    for name, got, w in zip(names, res, want):
-        if name == "db2":        # a bias in front of a BatchNorm: mathematically zero
-            assert float(got.abs().max()) <= 1e-5 * gmax, name
-            continue
-        assert rel(got, w) <= 5e-5, (name, rel(got, w))
+    for br, place in (("aligned", lambda t: t), ("offset16", _offset_copy)):
+        res = ops.gin_layer_bwd(_f(g_up), place(_f(y_in)), place(_f(r_ref)), place(_f(a_ref)), bn, _f(lin1.weight), _f(lin2.weight),
+                                indptr=pg.indptr if csr else None, indices=pg.indices if csr else None)
+        torch.cuda.synchronize()
+        for name, got, w in zip(names, res, want):
+            if name == "db2":        # a bias in front of a BatchNorm: mathematically zero
+                assert float(got.abs().max()) <= 1e-5 * gmax, (br, name)
+                continue
+            assert rel(got, w) <= 5e-5, (br, name, rel(got, w))
 
 
 # ------------------------------------------------------------------------------------------------ logM operator
