@@ -148,7 +148,6 @@ _PRIVATE_SIGNATURES = {
     "scgib_set_tensor_cores_bwd": (None, [c_int]),
     "scgib_debug_tc2_trace": (c_int, [c_void_p, c_int]),
     "scgib_debug_bf16_trace": (c_int, [c_void_p, c_int]),
-    "scgib_debug_tc4_trace": (c_int, [c_void_p, c_int]),
     "scgib_debug_bwdh_trace": (c_int, [c_void_p, c_int]),
 }
 

@@ -33,14 +33,8 @@ int bwd_tensor_core_mode() {
 }
 // CTAs of recon_fwd (= its per-CTA partial Gram matrices): two resident CTAs per SM at hidden 64 overlap the copy / Gram / gather phases
 static int recon_fwd_grid() { return 2 * num_sms(); }
-static int g_fwd4 = -1;
-int fwd_tc4_mode() {
-  if (g_fwd4 < 0) { const char* e = getenv("SCGIB_FWD4"); g_fwd4 = (e && e[0] == '1') ? 1 : 0; }
-  return g_fwd4;
-}
 static void launch_gin_fwd_any(const GinFwdArgs& a, int kin, cudaStream_t s) {      // op-level entry: hidden 64
   if (tensor_core_mode() == 0) launch_gin_fwd(a, kin, HID, s);
-  else if (kin == HID && !a.row_map && fwd_tc4_mode()) launch_gin_fwd_tc4(a, s);
   else launch_gin_fwd_tc3(a, kin, s);
 }
 
@@ -49,14 +43,6 @@ static int g_con_tc = -1;
 static bool use_tc_contrastive() {
   if (g_con_tc < 0) { const char* e = getenv("SCGIB_CON_FFMA"); g_con_tc = (e && e[0] == '1') ? 0 : 1; }
   return g_con_tc == 1;
-}
-
-// layers alternate the direction in which they walk the row tiles (SCGIB_FWD_ALT=0 disables): layer l+1 starts with the
-// rows layer l wrote last, which are still in L2
-static bool fwd_alternate() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SCGIB_FWD_ALT"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
 }
 
 bool pdl_enabled() {
@@ -367,15 +353,15 @@ static int forward_impl(const ScgibDims* d, const float* params, float* bn_runni
       a.part = e == 0 ? w.small_part : w.small_part2; a.counter = w.counters + (e == 0 ? 0 : 8);
       a.bn_out = w.bn[e][l];
       a.running = (bn_running && !eval) ? bn_running + (size_t)(e * L + l) * 2 * HID : nullptr;
-      a.reverse = (l & 1) && fwd_alternate();
+      // layers alternate the direction in which they walk the row tiles: layer l+1 starts with the rows layer l wrote
+      // last, which are still in L2
+      a.reverse = l & 1;
     }
     const int kin = l == 0 ? DT : HID;
     if (bf) {
       PROF("gin_fwd_bf16.enc1+2", launch_gin_fwd_bf16(ga[0], &ga[1], kin, HID, s));
     } else if (tc64 && tensor_core_mode() != 0) {
-      // gin_tc4 has no ego row map: layer 0 stays on gin_fwd_tc3 also when d_transfer = hidden
-      if (l > 0 && fwd_tc4_mode()) PROF("gin_fwd_tc4.enc1+2", launch_gin_fwd_tc4_pair(ga[0], ga[1], s));
-      else PROF("gin_fwd_tc.enc1+2", launch_gin_fwd_tc3_pair(ga[0], ga[1], kin, s));
+      PROF("gin_fwd_tc.enc1+2", launch_gin_fwd_tc3_pair(ga[0], ga[1], kin, s));
     } else {
       for (int e = 0; e < 2; ++e) PROF(e == 0 ? "gin_fwd_ffma.enc1" : "gin_fwd_ffma.enc2", launch_gin_fwd(ga[e], kin, HID, s));
     }

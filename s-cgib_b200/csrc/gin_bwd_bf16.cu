@@ -33,8 +33,8 @@ __device__ __forceinline__ uint4 pack8(const float (&v)[8]) {
 // ------------------------------------------------------------------------------------------------
 // part 1: upstream gradient of h' = relu(BN(y)), ReLU mask, d gamma / d beta
 // ------------------------------------------------------------------------------------------------
-template <int H, int MINB>
-__global__ void __launch_bounds__(kThreads, MINB)
+template <int H>
+__global__ void __launch_bounds__(kThreads, kBwdPreOcc)
 gin_bwd_pre_bf16_kernel(GinBwdPrePair pp) {
   pdl_sync();
   const bool second = (int)blockIdx.x >= pp.split;
@@ -539,10 +539,7 @@ gin_bwd_bf16_kernel(GinBwdMainPair pp) {
 int gin_bwd_pre_bf16_grid(int V, int hidden) { return gin_bwd_pre_grid(V); }
 template <int H>
 static void launch_pre_bf16_t(const GinBwdPrePair& pp, int grid, cudaStream_t s) {
-  const int occ = gin_bwd_pre_occ();
-  if (occ == 2) launch_k((bfb::gin_bwd_pre_bf16_kernel<H, 2>), dim3(grid), dim3(kThreads), 0, s, pp);
-  else if (occ == 3) launch_k((bfb::gin_bwd_pre_bf16_kernel<H, 3>), dim3(grid), dim3(kThreads), 0, s, pp);
-  else launch_k((bfb::gin_bwd_pre_bf16_kernel<H, 4>), dim3(grid), dim3(kThreads), 0, s, pp);
+  launch_k((bfb::gin_bwd_pre_bf16_kernel<H>), dim3(grid), dim3(kThreads), 0, s, pp);
 }
 
 void launch_gin_bwd_pre_bf16(const GinBwdPreArgs& a0, const GinBwdPreArgs* a1, int hidden, cudaStream_t s) {

@@ -516,9 +516,7 @@ void launch_gin_bwd_main_h_pair(const GinBwdMainArgs& a0, const GinBwdMainArgs& 
   static int tr = -1;
   if (tr < 0) { const char* e = getenv("SCGIB_DBG"); tr = (e && (atoi(e) & 2048)) ? 1 : 0; }
   pp.trace = tr;
-  static int rev = -1;
-  if (rev < 0) { const char* e = getenv("SCGIB_BWD_REV"); rev = (e && e[0] == '0') ? 0 : 1; }
-  pp.reverse = rev;
+  pp.reverse = 1;
   launch_k((bwdh::gin_bwd_h_kernel<false>), dim3(grid), dim3(bwdh::kThreadsB), bwdh::Smem::total, s, pp);
 }
 

@@ -456,8 +456,8 @@ void launch_gin_fwd(const GinFwdArgs& a, int kin, int hidden, cudaStream_t s) {
 //   g_o = G * [gamma*yhat+beta > 0] ; dbeta = sum g_o ; dgamma = sum g_o*yhat
 // Last CTA: dgamma/dbeta -> grads, and the BN-backward constants c1 = gamma*dbeta/V, c2 = gamma*dgamma/V.
 // ------------------------------------------------------------------------------------------------
-template <int HID, int MINB>
-__global__ void __launch_bounds__(kThreads, MINB)
+template <int HID>
+__global__ void __launch_bounds__(kThreads, kBwdPreOcc)
 gin_bwd_pre_kernel(GinBwdPrePair pp) {
   pdl_sync();
   const bool second = (int)blockIdx.x >= pp.split;
@@ -537,23 +537,15 @@ gin_bwd_pre_kernel(GinBwdPrePair pp) {
   }
 }
 
-// resident CTAs per SM of the gather kernels: SCGIB_PRE_OCC = 2 (default) | 3 | 4.  Measured on B200 (B = 4096): 52 / 58 / 59 us
+// resident CTAs per SM of the gather kernels, kBwdPreOcc = 2 against 3 / 4.  Measured on B200 (B = 4096): 52 / 58 / 59 us
 // per launch in fp32 and 42 / 63 / 68 us in bf16 - the register cap of the higher occupancies spills the rows in flight.
 // Also measured and NOT kept: the CSR index chain software-pipelined one row group ahead (offsets and the first four
 // neighbour ids of the next group requested while this group's rows are in flight): 63 instead of 52.6 us per launch at
 // 128 registers - the kernel is bound by its L2 / DRAM traffic, not by the dependent index loads.
-int gin_bwd_pre_occ() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SCGIB_PRE_OCC"); v = (e && e[0] >= '2' && e[0] <= '4') ? e[0] - '0' : 2; }
-  return v;
-}
-int gin_bwd_pre_grid(int V) { return min((V + 63) / 64, gin_bwd_pre_occ() * num_sms()); }
+int gin_bwd_pre_grid(int V) { return min((V + 63) / 64, kBwdPreOcc * num_sms()); }
 template <int H>
 static void launch_pre_t(const GinBwdPrePair& pp, int grid, cudaStream_t s) {
-  const int occ = gin_bwd_pre_occ();
-  if (occ == 2) launch_k((gin_bwd_pre_kernel<H, 2>), dim3(grid), dim3(kThreads), 0, s, pp);
-  else if (occ == 3) launch_k((gin_bwd_pre_kernel<H, 3>), dim3(grid), dim3(kThreads), 0, s, pp);
-  else launch_k((gin_bwd_pre_kernel<H, 4>), dim3(grid), dim3(kThreads), 0, s, pp);
+  launch_k((gin_bwd_pre_kernel<H>), dim3(grid), dim3(kThreads), 0, s, pp);
 }
 
 void launch_gin_bwd_pre(const GinBwdPreArgs& a, int hidden, cudaStream_t s) {

@@ -13,7 +13,7 @@
 //   * the CSR gather reads neighbour rows from that window (LDS, ~30 cycles); only neighbours further than the halo
 //     (graphs larger than 64 nodes) fall back to a global load;
 //   * after a producer barrier the aggregated rows overwrite the same buffer as tf32 hi/lo operand tiles.
-// Roles: 8 epilogue warps (TMEM lane quarter x column half), 1 MMA warp, 8 producer warps; one CTA per SM,
+// Roles: 8 epilogue warps (TMEM lane quarter x column half), 1 MMA warp, 16 producer warps; one CTA per SM,
 // two stages; Encoder1 and Encoder2 rows share the launch (GinFwdPair).
 #include <stdlib.h>
 #include "kernels.cuh"
@@ -30,6 +30,7 @@ namespace tc3 {
 constexpr int TM = 128;                       // rows per tile = UMMA M
 constexpr int kEpiWarps = 8;
 constexpr int kMmaWarp = kEpiWarps;
+constexpr int PW = 16;                        // producer warps: 16 keep enough gather loads in flight to hide their latency (b03bb00)
 constexpr int kIdxCap = 1024;                 // staged neighbour indices per tile (more edges: read from global)
 constexpr int kStageBytes = 2 * TM * HID * 4; // hi + lo tile of one stage (format S); first holds the raw row window
 constexpr int HALO = 64, WIN = TM + 2 * HALO;  // window rows (WIN * 64 floats = the whole stage)
@@ -81,7 +82,7 @@ __device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity) {
   return ok != 0;
 }
 
-template <int KIN, int PW>
+template <int KIN>
 __global__ void __launch_bounds__((kEpiWarps + 1 + PW) * 32, 1)
 gin_fwd_tc3_kernel(GinFwdPair pp) {
   using L = Smem<KIN>;
@@ -500,21 +501,12 @@ gin_fwd_tc3_kernel(GinFwdPair pp) {
 
 }  // namespace tc3
 
-template <int KIN, int PW>
-static void launch_tc3_pw(const GinFwdPair& pp, int grid, cudaStream_t s) {
-  using L = tc3::Smem<KIN>;
-  static bool once = (cudaFuncSetAttribute(tc3::gin_fwd_tc3_kernel<KIN, PW>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::total), true);
-  (void)once;
-  launch_k((tc3::gin_fwd_tc3_kernel<KIN, PW>), dim3(grid), dim3((tc3::kEpiWarps + 1 + PW) * 32), L::total, s, pp);
-}
 template <int KIN>
 static void launch_tc3(const GinFwdPair& pp, int grid, cudaStream_t s) {
-  static int pw = -1;                     // producer warps: SCGIB_TC3_PW = 8 | 12 | 16 (default) | 20
-  if (pw < 0) { const char* e = getenv("SCGIB_TC3_PW"); pw = e ? atoi(e) : 16; }
-  if (pw == 20) launch_tc3_pw<KIN, 20>(pp, grid, s);
-  else if (pw == 16) launch_tc3_pw<KIN, 16>(pp, grid, s);
-  else if (pw == 12) launch_tc3_pw<KIN, 12>(pp, grid, s);
-  else launch_tc3_pw<KIN, 8>(pp, grid, s);
+  using L = tc3::Smem<KIN>;
+  static bool once = (cudaFuncSetAttribute(tc3::gin_fwd_tc3_kernel<KIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::total), true);
+  (void)once;
+  launch_k((tc3::gin_fwd_tc3_kernel<KIN>), dim3(grid), dim3((tc3::kEpiWarps + 1 + tc3::PW) * 32), L::total, s, pp);
 }
 
 }  // namespace scgib

@@ -45,40 +45,18 @@ void launch_segment_sum(const float* in, const int32_t* seg_ptr, int S, const fl
 }
 
 // C_v = sum over the ego-net of v of relu(BN(y)) ; logit_v = w_cand . C_v
-template <bool BF, int HID>
-__global__ void __launch_bounds__(kThreads)
-ego_pool_fwd_kernel(EgoPoolFwdArgs p) {
-  pdl_sync();
-  constexpr int LPR = HID / 4, SPC = kThreads / LPR;      // 16 lanes (half-warp) per seed at HID = 64, a full warp at 128
-  const int l = threadIdx.x % LPR;
-  Bn4 b;
-  b.load(p.bn, l * 4, HID);
-  const float4 w = ldg4(p.w_cand + l * 4);
-  for (int v = blockIdx.x * SPC + (threadIdx.x / LPR); v < p.N; v += gridDim.x * SPC) {
-    const int r0 = __ldg(p.ego_ptr + v), r1 = __ldg(p.ego_ptr + v + 1);
-    float4 acc = make4(0.f);
-#pragma unroll 4
-    for (int r = r0; r < r1; ++r) acc = add4(acc, b.act(ld4a<BF>(p.y, (size_t)r * HID + l * 4)));
-    st4(p.C + (size_t)v * HID + l * 4, acc);
-    float d = acc.x * w.x + acc.y * w.y + acc.z * w.z + acc.w * w.w;
-    const unsigned hmask = LPR == 32 ? 0xffffffffu : ((threadIdx.x & 16) ? 0xffff0000u : 0x0000ffffu);   // half-warps may diverge at the tail
-#pragma unroll
-    for (int o = LPR / 2; o > 0; o >>= 1) d += __shfl_xor_sync(hmask, d, o);
-    if (l == 0) p.logit[v] = d;
-  }
-}
-// the same with TWO consecutive seeds per lane group: their rows are contiguous, so one unrolled pass over [r0, r2) keeps up to 8
+// TWO consecutive seeds per lane group: their rows are contiguous, so one unrolled pass over [r0, r2) keeps up to 8
 // independent row loads in flight per lane (one seed's ~3 rows leave the memory pipeline idle behind the ego_ptr -> row chain)
 template <bool BF, int HID>
 __global__ void __launch_bounds__(kThreads)
-ego_pool_fwd2_kernel(EgoPoolFwdArgs p) {
+ego_pool_fwd_kernel(EgoPoolFwdArgs p) {
   pdl_sync();
   constexpr int LPR = HID / 4, SPC = kThreads / LPR;
   const int l = threadIdx.x % LPR;
   Bn4 b;
   b.load(p.bn, l * 4, HID);
   const float4 w = ldg4(p.w_cand + l * 4);
-  const unsigned hmask = LPR == 32 ? 0xffffffffu : ((threadIdx.x & 16) ? 0xffff0000u : 0x0000ffffu);
+  const unsigned hmask = LPR == 32 ? 0xffffffffu : ((threadIdx.x & 16) ? 0xffff0000u : 0x0000ffffu);   // half-warps may diverge at the tail
   // the segment offsets of the NEXT pair are requested before this pair's rows are consumed (persistent grid: the
   // ego_ptr -> rows dependency of one iteration overlaps the row loads of the previous one)
   const int stride = 2 * gridDim.x * SPC;
@@ -113,26 +91,8 @@ ego_pool_fwd2_kernel(EgoPoolFwdArgs p) {
 }
 
 void launch_ego_pool_fwd(const EgoPoolFwdArgs& a, int hidden, cudaStream_t s) {
-  static int var2 = -1;          // SCGIB_EGO_VAR=1: one seed per lane group (the round-1 kernel)
-  if (var2 < 0) { const char* e = getenv("SCGIB_EGO_VAR"); var2 = (e && e[0] == '1') ? 0 : 1; }
-  if (var2) {
-    const int spc2 = 2 * (kThreads / (hidden / 4));
-    static int per_sm = -1;        // SCGIB_EGO_CTAS: resident CTAs per SM of the persistent grid (0 = one pass per CTA)
-    if (per_sm < 0) { const char* e = getenv("SCGIB_EGO_CTAS"); per_sm = e ? atoi(e) : 3; }
-    const int grid2 = min((a.N + spc2 - 1) / spc2, (per_sm > 0 ? per_sm : 16) * num_sms());
-    if (hidden == 64) {
-      if (a.y_bf16) launch_k((ego_pool_fwd2_kernel<true, 64>), dim3(grid2), dim3(kThreads), 0, s, a);
-      else launch_k((ego_pool_fwd2_kernel<false, 64>), dim3(grid2), dim3(kThreads), 0, s, a);
-    } else {
-      if (a.y_bf16) launch_k((ego_pool_fwd2_kernel<true, 128>), dim3(grid2), dim3(kThreads), 0, s, a);
-      else launch_k((ego_pool_fwd2_kernel<false, 128>), dim3(grid2), dim3(kThreads), 0, s, a);
-    }
-    return;
-  }
-  const int spc = kThreads / (hidden / 4);
-  static int full = -1;          // SCGIB_EGO_GRID=full: one CTA pass per 16 seeds, no grid-stride tail (experiment)
-  if (full < 0) { const char* e = getenv("SCGIB_EGO_GRID"); full = (e && e[0] == 'f') ? 1 : 0; }
-  const int grid = full ? (a.N + spc - 1) / spc : min((a.N + spc - 1) / spc, 16 * num_sms());
+  const int spc = 2 * (kThreads / (hidden / 4));                 // seeds per CTA pass
+  const int grid = min((a.N + spc - 1) / spc, 3 * num_sms());    // persistent: 3 CTAs per SM
   if (hidden == 64) {
     if (a.y_bf16) launch_k((ego_pool_fwd_kernel<true, 64>), dim3(grid), dim3(kThreads), 0, s, a);
     else launch_k((ego_pool_fwd_kernel<false, 64>), dim3(grid), dim3(kThreads), 0, s, a);

@@ -47,7 +47,7 @@ struct GinFwdArgs {
   float* running;                     // optional {running_mean, running_var}[HID]
   int reverse = 0;                    // gin_tc3: walk the row tiles in descending order (alternate layers: the rows the
                                       //  previous layer wrote last are still in L2)
-  int dbg = 0;                        // gin_tc2 experiments (SCGIB_DBG bit mask): 1 no r/y stores, 2 no stats, 4 no gather loads, 8 no a store
+  int dbg = 0;                        // SCGIB_DBG: bit 1024 records the per-tile role timeline (gin_tc3 / gin_bf16)
 };
 // Two independent problems of the same shape class (the same layer of Encoder1 and Encoder2) in ONE launch: CTAs
 // [0, split) work on a[0], CTAs [split, grid) on a[1]; split is chosen proportional to the tile counts, so the 148
@@ -57,9 +57,6 @@ int gin_fwd_grid(int V);
 void launch_gin_fwd(const GinFwdArgs& a, int kin, int hidden, cudaStream_t s);        // FP32 FFMA tiles (gin_kernels.cu), hidden 64 / 128
 void launch_gin_fwd_tc3(const GinFwdArgs& a, int kin, cudaStream_t s);              // tcgen05 3xTF32, shared-memory window gather (gin_tc3.cu)
 void launch_gin_fwd_tc3_pair(const GinFwdArgs& a0, const GinFwdArgs& a1, int kin, cudaStream_t s);
-void launch_gin_fwd_tc4(const GinFwdArgs& a, cudaStream_t s);                       // tcgen05, aggregation on the tensor cores too (gin_tc4.cu); KIN = 64
-void launch_gin_fwd_tc4_pair(const GinFwdArgs& a0, const GinFwdArgs& a1, cudaStream_t s);
-int fwd_tc4_mode();                                                       // SCGIB_FWD4: 1 = gin_tc4.cu for the KIN = 64 layers
 // bf16 mode (gin_bf16.cu, gin_bwd_bf16.cu): the float* activation fields of the argument blocks point to bf16 data
 size_t gin_fwd_bf16_part_floats(int hidden);
 void launch_gin_fwd_bf16(const GinFwdArgs& a0, const GinFwdArgs* a1, int kin, int hidden, cudaStream_t s);
@@ -83,7 +80,7 @@ struct GinBwdPreArgs {
 };
 struct GinBwdPrePair { GinBwdPreArgs a[2]; int split; };
 int gin_bwd_pre_grid(int V);
-int gin_bwd_pre_occ();          // resident CTAs per SM of the gather kernels (SCGIB_PRE_OCC)
+constexpr int kBwdPreOcc = 2;   // resident CTAs per SM of the gather kernels (gin_bwd_pre, gin_bwd_pre_bf16; gin_kernels.cu)
 void launch_gin_bwd_pre(const GinBwdPreArgs& a, int hidden, cudaStream_t s);
 void launch_gin_bwd_pre_pair(const GinBwdPreArgs& a0, const GinBwdPreArgs& a1, int hidden, cudaStream_t s);   // grid = gin_bwd_pre_grid(V0 + V1)
 int pair_split(int grid, int work0, int work1);     // CTAs given to problem 0

@@ -20,7 +20,6 @@ SCGIB_API void scgib_set_tensor_cores_bwd(int mode);
 SCGIB_API int scgib_debug_tc2_trace(long long* host_out, int n);
 SCGIB_API int scgib_debug_bf16_trace(long long* host_out, int n);     /* gin_fwd_bf16 (bf16 mode), same layout */
 SCGIB_API int scgib_debug_bwdh_trace(long long* host_out, int n);     /* gin_bwd_h (SCGIB_DBG bit 2048), same layout */
-SCGIB_API int scgib_debug_tc4_trace(long long* host_out, int n);      /* gin_fwd_tc4: [cta < 160][tile < 16][event < 16] */
 #ifdef __cplusplus
 }
 #endif

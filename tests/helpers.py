@@ -67,7 +67,7 @@ def dump_parity(tag, report):
     """Measured errors of a parity case -> gpurun_out/parity_fp32/<tag>.json (kept in profiles/parity_r02.json)."""
     import json
     import os
-    if any(os.environ.get(k) for k in ("SCGIB_FWD4", "SCGIB_HEAD_FFMA", "SCGIB_CON_FFMA", "SCGIB_TC", "SCGIB_TC_BWD")):
+    if any(os.environ.get(k) for k in ("SCGIB_HEAD_FFMA", "SCGIB_CON_FFMA", "SCGIB_TC", "SCGIB_TC_BWD")):
         return      # a cross-check run (tests/test_gpu_round2.py): keep the default build's numbers
     out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out", "parity_fp32")
     os.makedirs(out, exist_ok=True)

@@ -213,12 +213,11 @@ def test_device_loader_reshuffles_every_pass():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [{"SCGIB_FWD4": "1"}, {"SCGIB_HEAD_FFMA": "1", "SCGIB_CON_FFMA": "1"}],
-                         ids=["tc4_forward", "ffma_head_contrastive"])
+@pytest.mark.parametrize("env", [{"SCGIB_HEAD_FFMA": "1", "SCGIB_CON_FFMA": "1"}], ids=["ffma_head_contrastive"])
 def test_implementation_switches_stay_parity_green(env):
-    """The experimental / cross-check kernels behind the environment switches (INTEGRATION.md) pass the same parity tests as
-    the defaults: the tensor-core-aggregation forward gin_tc4 and the FFMA head / contrastive kernels with the un-fused
-    forward tail.  The switches are read once per process, hence the subprocess."""
+    """The cross-check kernels behind the environment switches (INTEGRATION.md) pass the same parity tests as the
+    defaults: the FFMA head / contrastive kernels with the un-fused forward tail.  The switches are read once per
+    process, hence the subprocess."""
     import os
     import subprocess
     import sys
