@@ -60,7 +60,8 @@ def run_pretraining(model, pre_train_loader1, optimizer, batch_size, device):
             best_model, best_epoch, best_loss = model, epoch, epoch_train_loss
         if epoch - best_epoch > 50:
             break
-        print("Epoch:%d	|Best_epoch:%d	|Train_loss:%0.4f" % (epoch, best_epoch, epoch_train_loss))
+        if rank == 0:
+            print("Epoch:%d	|Best_epoch:%d	|Train_loss:%0.4f" % (epoch, best_epoch, epoch_train_loss))
     return best_model, best_epoch
 
 

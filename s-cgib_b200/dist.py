@@ -35,6 +35,57 @@ def shard_range(num_graphs: int, rank: int, world: int):
     return lo, lo + base + (1 if rank < rem else 0)
 
 
+def rank_world():
+    """(rank, world) of the initialised process group; (0, 1) without one."""
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_rank(), dist.get_world_size()
+    return 0, 1
+
+
+def round_robin_batches(num_items: int, batch_size: int, rank: int, world: int):
+    """Whole-batch shard for evaluation: the [lo, hi) item ranges of batches rank, rank + world, rank + 2 world, ... of
+    the single-process batch list (the last batch may be short).  The union over the ranks is that batch list, so every
+    item is evaluated exactly once whatever ``num_items`` is."""
+    starts = range(rank * batch_size, num_items, world * batch_size)
+    return [(lo, min(lo + batch_size, num_items)) for lo in starts]
+
+
+def mean_over_ranks(sums, count: int, device=None):
+    """Per-batch means over the union of every rank's batches: ``sums`` are this rank's sums of per-batch values,
+    ``count`` its number of batches.  One all-reduce (float64) of the sums and the count; every rank gets the same
+    floats back."""
+    _, world = rank_world()
+    if world == 1:
+        return [float(s) / max(count, 1) for s in sums]
+    t = torch.tensor([float(s) for s in sums] + [float(count)], dtype=torch.float64, device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    vals = t.tolist()
+    return [s / max(vals[-1], 1.0) for s in vals[:-1]]
+
+
+@torch.no_grad()
+def average_bn_buffers_(module: torch.nn.Module):
+    """All-reduce-average ``running_mean`` / ``running_var`` of every BatchNorm in ``module`` across the ranks, in place:
+    the buffers of the GIN engine path are views into the engine's ``bn_running`` and must keep aliasing it.  BatchNorm
+    batch statistics stay per rank during training, so the running estimates drift apart; averaging them before an
+    evaluation or a checkpoint keeps the replicas identical.  ``num_batches_tracked`` is left alone (equal on every rank
+    when every rank runs the same number of batches)."""
+    _, world = rank_world()
+    if world == 1:
+        return
+    bufs = [b for m in module.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm) and m.track_running_stats
+            for b in (m.running_mean, m.running_var)]
+    if not bufs:
+        return
+    flat = torch.cat([b.reshape(-1) for b in bufs])
+    dist.all_reduce(flat, op=dist.ReduceOp.SUM)
+    flat /= world
+    off = 0
+    for b in bufs:
+        b.copy_(flat[off:off + b.numel()].view_as(b))
+        off += b.numel()
+
+
 def allreduce_grads_(flat_grads: torch.Tensor, world: int) -> float:
     """Sum-all-reduce the flat gradient buffer in place; returns the scale the optimiser applies (1/world)."""
     if world > 1:

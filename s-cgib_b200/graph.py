@@ -346,13 +346,17 @@ class DeviceLoader:
     """Drop-in for ``DataLoader(dataset, batch_size, shuffle=True, collate_fn=dataset.collate)`` (exp_pretraining.py:283) over
     a ``DeviceDataset``: iterating yields the reference's 4-tuples ``(batched_graph, labels, subgraphs, logMs)`` with the
     batch assembled on the GPU from B molecule ids (no Python object per molecule, no collate, no H2D of graph data).
-    ``rank`` / ``world`` shard every epoch's permutation like a ``DistributedSampler(drop_last=True)``."""
+    ``rank`` / ``world`` shard every epoch's permutation like a ``DistributedSampler(drop_last=True)``.  With
+    ``shard_batches=True`` they shard whole batches instead: rank r takes batches r, r + world, r + 2 world, ... of the
+    single-process batch list, so the ranks together see every molecule exactly once (evaluation splits)."""
 
     def __init__(self, dataset: DeviceDataset, batch_size: int, shuffle: bool = True, drop_last: bool = False,
-                 labels: Optional[torch.Tensor] = None, rank: int = 0, world: int = 1, seed: int = 0):
+                 labels: Optional[torch.Tensor] = None, rank: int = 0, world: int = 1, seed: int = 0,
+                 shard_batches: bool = False):
         self.dataset, self.batch_size, self.shuffle, self.drop_last = dataset, int(batch_size), shuffle, drop_last
         self.labels = None if labels is None else labels.to(dataset.device)
         self.rank, self.world, self.seed, self.epoch = rank, world, seed, 0
+        self.shard_batches = shard_batches
         self.sampler = self                      # ``loader.sampler.set_epoch(e)`` works as with a DistributedSampler
         self._bufs = [{}, {}]                    # two sets of reusable device buffers (consecutive batches never share one)
 
@@ -361,19 +365,26 @@ class DeviceLoader:
 
     def _per_rank(self):
         n = len(self.dataset)
-        return n // self.world if self.world > 1 else n
+        return n // self.world if self.world > 1 and not self.shard_batches else n
+
+    def _ranges(self):
+        """[lo, hi) positions in the pass's id list of this rank's batches."""
+        n, B = self._per_rank(), self.batch_size
+        if self.drop_last:
+            n -= n % B
+        if self.shard_batches:
+            from .dist import round_robin_batches
+            return round_robin_batches(n, B, self.rank, self.world)
+        return [(lo, min(lo + B, n)) for lo in range(0, n, B)]
 
     def __len__(self):
-        n = self._per_rank()
-        return n // self.batch_size if self.drop_last else (n + self.batch_size - 1) // self.batch_size
+        return len(self._ranges())
 
     def id_batches(self):
         """The epoch's mini-batches as device tensors of molecule ids (what ``__iter__`` assembles one by one)."""
         ids_dev = self._epoch_ids()
-        for i in range(len(self)):
-            ids = ids_dev[i * self.batch_size:(i + 1) * self.batch_size]
-            if ids.numel():
-                yield ids
+        for lo, hi in self._ranges():
+            yield ids_dev[lo:hi]
 
     def _epoch_ids(self):
         """Permutation of this pass, then advance the epoch: like ``DataLoader(shuffle=True)`` every pass reshuffles
@@ -384,17 +395,15 @@ class DeviceLoader:
             self.epoch += 1
         else:
             perm = torch.arange(n)
-        if self.world > 1:
+        if self.world > 1 and not self.shard_batches:
             per = n // self.world
             perm = perm[self.rank * per:(self.rank + 1) * per]
         return perm.to(torch.int32).to(self.dataset.device)
 
     def __iter__(self):
         ids_dev = self._epoch_ids()
-        for i in range(len(self)):
-            ids = ids_dev[i * self.batch_size:(i + 1) * self.batch_size]
-            if ids.numel() == 0:
-                break
+        for i, (lo, hi) in enumerate(self._ranges()):
+            ids = ids_dev[lo:hi]
             g = self.dataset.assemble(ids, out=self._bufs[i & 1])
             labels = self.labels[ids.long()] if self.labels is not None else torch.zeros(ids.numel(), 1, device=self.dataset.device)
             yield g, labels, None, None

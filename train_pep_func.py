@@ -1,10 +1,14 @@
 """Drop-in for the reference's ``train_pep_func.py`` training / evaluation loops (reference train_pep_func.py:91-230) on the
 B200 path: same function names, arguments and return values.  Differences: the ego-nets come from the GPU extraction
 kernel (``khop_ego_batch``) instead of pickled DGLGraph lists, and the NaN-masking of ``MetricWrapper`` (goli / ogb are not
-installable here) is restated in ``masked_loss``."""
+installable here) is restated in ``masked_loss``.
+
+Under torch.distributed (one process per GPU) every function returns the per-batch mean over the union of all ranks'
+batches (``scgib_b200.dist.mean_over_ranks``), identical on every rank; single process, the values are the reference's."""
 import torch
 import torch.nn.functional as F
 
+from scgib_b200.dist import mean_over_ranks, rank_world
 from scgib_b200.graph import khop_ego_batch
 
 
@@ -36,6 +40,9 @@ def train_epoch_domainadaptation(model, args, optimizer, device, data_loader, ep
         optimizer.step()
         epoch_loss += loss.detach().item()
         epoch_reconstruction_loss += reconstruction_loss.detach()
+    if rank_world()[1] > 1:
+        epoch_loss, rec = mean_over_ranks([epoch_loss, epoch_reconstruction_loss], count + 1, device)
+        return epoch_loss, torch.tensor(rec, dtype=torch.float32, device=device)
     epoch_loss /= (count + 1)
     epoch_reconstruction_loss /= (count + 1)
     return epoch_loss, epoch_reconstruction_loss
@@ -65,6 +72,9 @@ def train_epoch_graph_classification(args, model, optimizer, device, data_loader
             optimizer.zero_grad()
         epoch_loss += loss.detach().item()
         epoch_train_ap += model.BCEWithLogitsLoss(batch_scores.detach(), batch_targets)
+    if rank_world()[1] > 1:
+        epoch_loss, ap = mean_over_ranks([epoch_loss, epoch_train_ap], it + 1, device)
+        return epoch_loss, torch.tensor(ap, dtype=torch.float32), optimizer
     epoch_train_ap /= (it + 1)
     epoch_loss /= (it + 1)
     return epoch_loss, epoch_train_ap.detach().cpu(), optimizer
@@ -87,6 +97,9 @@ def evaluate_network(args, model, optimizer, device, data_loader, epoch, batch_s
             loss = masked_loss(model.loss, batch_scores, batch_targets)
             epoch_test_loss += loss.detach().item()
             epoch_test_ap += model.BCEWithLogitsLoss(batch_scores, batch_targets)
+    if rank_world()[1] > 1:         # whole-batch shards (round robin): a rank may hold fewer batches, or none
+        loss, ap = mean_over_ranks([epoch_test_loss, epoch_test_ap], it + 1, device)
+        return loss, torch.tensor(ap, dtype=torch.float32)
     epoch_test_ap /= (it + 1)
     epoch_test_loss /= (it + 1)
     return epoch_test_loss, epoch_test_ap.detach().cpu()
