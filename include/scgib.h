@@ -296,6 +296,26 @@ SCGIB_API int scgib_gin_layer_bwd_f32(const float* g_next, const int32_t* indptr
                                       float* db2, float* dgamma, float* dbeta, void* workspace, size_t workspace_bytes,
                                       void* stream);
 
+/* The same layer in bf16 mode (the kernels of the fused step with SCGIB_ACT_BF16), hidden H = 64 (kin 32 or 64) or 128
+ * (kin 32, 64 or 128); other shapes return SCGIB_E_SHAPE.  Activations are bf16 (16-byte aligned rows), weights, biases,
+ * BatchNorm constants and weight gradients fp32.
+ *  forward : in, a_out, r_out, y_out bf16; y is rounded once and bn_out holds the statistics of the rounded y.
+ *            workspace >= scgib_gin_layer_fwd_bf16_workspace_bytes(V, H), 256-byte aligned.
+ *  backward: g_next bf16 [V,H] with indptr (CSR mode), fp32 [V,H] without (gradient wrt the layer output); y, r, a bf16;
+ *            g_a fp32 when ga_f32 != 0 or kin < H, else bf16.  workspace >= scgib_gin_layer_bwd_bf16_workspace_bytes. */
+SCGIB_API size_t scgib_gin_layer_fwd_bf16_workspace_bytes(int32_t V, int32_t hidden);
+SCGIB_API int scgib_gin_layer_fwd_bf16(const void* in, int32_t kin, int32_t hidden, const int32_t* row_map, const float* bn_in,
+                                       const int32_t* indptr, const int32_t* indices, int32_t V,
+                                       const float* W1, const float* b1, const float* W2, const float* b2,
+                                       void* a_out, void* r_out, void* y_out, float* bn_out, float* running,
+                                       void* workspace, size_t workspace_bytes, void* stream);
+SCGIB_API size_t scgib_gin_layer_bwd_bf16_workspace_bytes(int32_t V, int32_t kin, int32_t hidden);
+SCGIB_API int scgib_gin_layer_bwd_bf16(const void* g_next, const int32_t* indptr, const int32_t* indices, int32_t V,
+                                       int32_t kin, int32_t hidden, int32_t ga_f32, const void* y, const void* r, const void* a,
+                                       const float* bn, const float* W1, const float* W2, void* g_a, float* dW1, float* db1,
+                                       float* dW2, float* db2, float* dgamma, float* dbeta, void* workspace,
+                                       size_t workspace_bytes, void* stream);
+
 /* Loss operators: value and gradient in one call (the units of the whole-step functions).  workspace >=
  * scgib_loss_workspace_bytes(B) (B = 1 for the reconstruction loss), 256-byte aligned; loss = device float[1].
  *  scgib_recon_adj_f32  : loss_recon_adj (models.py:762-768) = sum_{ij} (z_i . z_j - A_ij)^2 / N over the WHOLE batch

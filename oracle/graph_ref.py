@@ -212,17 +212,44 @@ def _synth_bonds(rng: np.random.Generator, n: int, window: int, p_chain: float, 
     return bonds, deg
 
 
+def _macrocycle_bonds(rng: np.random.Generator, n: int):
+    """Peptides-shape chain with a head-to-tail closure (atom 0 - atom n-1) and 3 closures 65 .. 200 atoms apart: the bonds
+    of a macrocyclic peptide, whose neighbours lie further apart in atom order than the local ring closures of ``peptides``."""
+    bonds, deg = _synth_bonds(rng, n, window=6, p_chain=0.5, n_rings=3)
+    have = {(min(a, b), max(a, b)) for a, b in bonds}
+    extra = [(0, n - 1)]
+    while len(extra) < 4:
+        a = int(rng.integers(n))
+        b = a + int(rng.integers(65, 201)) * (1 if rng.random() < 0.5 else -1)
+        if 0 <= b < n and (min(a, b), max(a, b)) not in have and (min(a, b), max(a, b)) not in extra:
+            extra.append((min(a, b), max(a, b)))
+    for a, b in extra:
+        if (a, b) not in have:
+            bonds.append((a, b))
+            deg[a] += 1
+            deg[b] += 1
+    return bonds, deg
+
+
 def synth_molecule(rng: np.random.Generator, shape: str = "pcqm") -> RefGraph:
     """One synthetic molecule.  ``pcqm``: n~U[8,22], tree + 2 ring closures (bonds ~ n+1).
-    ``peptides``: n~U[120,180], chain-biased tree + 3 ring closures."""
+    ``peptides``: n~U[120,180], chain-biased tree + 3 ring closures.  ``macrocycle``: a ``peptides`` chain with a head-to-tail
+    closure and 3 closures 65 .. 200 atoms apart (_macrocycle_bonds)."""
     if shape == "pcqm":
         n = int(rng.integers(8, 23))
         bonds, deg = _synth_bonds(rng, n, window=6, p_chain=0.0, n_rings=2)
     elif shape == "peptides":
         n = int(rng.integers(120, 181))
         bonds, deg = _synth_bonds(rng, n, window=6, p_chain=0.5, n_rings=3)
+    elif shape == "macrocycle":
+        n = int(rng.integers(120, 181))
+        bonds, deg = _macrocycle_bonds(rng, n)
     else:
         raise ValueError(shape)
+    return _molecule(rng, n, bonds, deg)
+
+
+def _molecule(rng: np.random.Generator, n: int, bonds, deg) -> RefGraph:
     b = np.asarray(bonds, dtype=np.int64)
     nn_, s, d = to_bidirected_ref(b[:, 0], b[:, 1], n)
     indptr, indices = csr_from_edges(n, s, d)
@@ -261,3 +288,79 @@ def graph_from_bonds(n: int, bonds, F: int = 9, seed: int = 0) -> RefGraph:
     indptr, indices = csr_from_edges(n, ss, dd)
     x = np.random.default_rng(seed).random((n, F), dtype=np.float32) + 0.1
     return RefGraph(np.asarray([0, n], dtype=np.int32), indptr, indices, x)
+
+
+# --------------------------------------------------------------------------------------
+# Non-local and dense graphs: the gather paths of the GIN forward kernels (csrc/gin_tc3.cu, gin_bf16.cu) beyond the
+# 256-row window (a 128-row tile + a 64-row halo on each side) and beyond the 1024 staged neighbour indices of a tile
+# --------------------------------------------------------------------------------------
+GIN_TILE, GIN_HALO, GIN_IDX_CAP = 128, 64, 1024
+
+
+def macrocycle_batch(seed: int, num_graphs: int, big: int = 420) -> RefGraph:
+    """``num_graphs`` macrocyclic peptides (synth_molecule "macrocycle") and, with ``big`` > 0, one macrocycle of ``big``
+    atoms: neighbours up to 200 rows apart, beyond the gather window."""
+    rng = np.random.default_rng(seed)
+    mols = [synth_molecule(rng, "macrocycle") for _ in range(num_graphs)]
+    if big:
+        mols.append(_molecule(rng, big, *_macrocycle_bonds(rng, big)))
+    return batch_ref(mols)
+
+
+def shuffle_nodes(g: RefGraph, seed: int) -> RefGraph:
+    """The same graphs with the node ids randomly permuted inside each graph (arbitrary atom order: neighbours anywhere in
+    the graph's row range)."""
+    rng = np.random.default_rng(seed)
+    N = g.num_nodes
+    perm = np.concatenate([lo + rng.permutation(hi - lo) for lo, hi in zip(g.graph_ptr[:-1], g.graph_ptr[1:])]).astype(np.int64)
+    src, dst = g.edges()
+    indptr, indices = csr_from_edges(N, perm[src], perm[dst])
+    x = np.empty_like(g.x)
+    x[perm] = g.x
+    return RefGraph(g.graph_ptr.copy(), indptr, indices, x)
+
+
+def halo_graph(V: int, F: int = 9) -> RefGraph:
+    """One graph of V rows: a path, plus edges from rows 0 and 127 of every tile to the rows just inside and just outside
+    its window [ws, ws + 256), ws = max(0, base - 64): u = ws (inside), ws - 1 (outside), ws + 255 (inside), ws + 256
+    (outside), where those rows exist.  Tile 0 has its window clipped at row 0, the last tile at V."""
+    bonds = [(i, i + 1) for i in range(V - 1)]
+    for base in range(0, V, GIN_TILE):
+        ws = max(0, base - GIN_HALO)
+        for v in (base, base + GIN_TILE - 1):
+            for u in (ws - 1, ws, ws + 2 * GIN_HALO + GIN_TILE - 1, ws + 2 * GIN_HALO + GIN_TILE):
+                if v < V and 0 <= u < V and u != v:
+                    bonds.append((v, u))
+    return graph_from_bonds(V, bonds, F)
+
+
+def circulant_bonds(V: int, half_degree: int = 4):
+    """Bonds of the circulant graph with offsets 1 .. half_degree (wrapping): every row has 2 * half_degree neighbours."""
+    return [(i, (i + k) % V) for i in range(V) for k in range(1, half_degree + 1)]
+
+
+def dense_tiles_graph(F: int = 9) -> RefGraph:
+    """Three tiles of a degree-8 circulant (1024 edges each) with one bond removed between tiles 0 and 1 and one added
+    between tiles 1 and 2: tiles of exactly 1023, 1024 and 1025 edges."""
+    V = 3 * GIN_TILE
+    bonds = [b for b in circulant_bonds(V) if b != (127, 128)] + [(200, 300)]
+    return graph_from_bonds(V, bonds, F)
+
+
+def dense_walk_graph(ctas: int = 148, walk: int = 4, F: int = 9) -> RefGraph:
+    """``walk`` tiles per CTA of a ``ctas``-CTA persistent grid (tile t is the (t // ctas)-th tile its CTA walks): a degree-8
+    circulant (1024 edges per tile) where every odd step of the walk gets 64 more bonds inside the tile (1152 edges, over
+    the staged-index capacity), so that overflowing and fitting tiles alternate through the three index buffers."""
+    V = ctas * walk * GIN_TILE
+    bonds = circulant_bonds(V)
+    for t in range(V // GIN_TILE):
+        if (t // ctas) % 2 == 1:
+            base = t * GIN_TILE
+            bonds += [(base + r, base + r + GIN_HALO) for r in range(GIN_HALO)]
+    return graph_from_bonds(V, bonds, F)
+
+
+def star_graph(leaves: int, F: int = 9) -> RefGraph:
+    """A hub (row 0) bonded to ``leaves`` leaves: the hub row alone exceeds the staged indices of its tile, and most leaves,
+    and the hub for every leaf past row 255, lie outside the window."""
+    return graph_from_bonds(leaves + 1, [(0, i) for i in range(1, leaves + 1)], F)

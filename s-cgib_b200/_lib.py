@@ -84,6 +84,14 @@ _SIGNATURES = {
     "scgib_gin_layer_bwd_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_size_t, c_void_p]),
+    "scgib_gin_layer_fwd_bf16_workspace_bytes": (c_size_t, [c_int32, c_int32]),
+    "scgib_gin_layer_fwd_bf16": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "scgib_gin_layer_bwd_bf16_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "scgib_gin_layer_bwd_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "scgib_loss_workspace_bytes": (c_size_t, [c_int32]),
     "scgib_recon_adj_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_float, c_void_p, c_void_p, c_void_p,
                                     c_size_t, c_void_p]),

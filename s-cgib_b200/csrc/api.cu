@@ -931,6 +931,100 @@ extern "C" SCGIB_API int scgib_gin_layer_bwd_f32(const float* g_next, const int3
   return (int)cudaGetLastError();
 }
 
+// The same layer in bf16 mode: the kernels and launch configuration of the fused step (gin_bf16.cu, gin_bwd_bf16.cu), one problem
+static bool gin_bf16_shape_ok(int kin, int H) { return (H == 64 && (kin == 32 || kin == 64)) || (H == 128 && (kin == 32 || kin == 64 || kin == 128)); }
+static bool al16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
+
+extern "C" SCGIB_API size_t scgib_gin_layer_fwd_bf16_workspace_bytes(int32_t V, int32_t hidden) {
+  if (V < 1 || (hidden != 64 && hidden != 128)) return 0;
+  return 256 + al(gin_fwd_bf16_part_floats(hidden) * sizeof(float));
+}
+
+extern "C" SCGIB_API int scgib_gin_layer_fwd_bf16(const void* in, int32_t kin, int32_t hidden, const int32_t* row_map, const float* bn_in,
+                                        const int32_t* indptr, const int32_t* indices, int32_t V, const float* W1,
+                                        const float* b1, const float* W2, const float* b2, void* a_out, void* r_out,
+                                        void* y_out, float* bn_out, float* running, void* workspace,
+                                        size_t workspace_bytes, void* stream_) {
+  if (!in || !indptr || !W1 || !b1 || !W2 || !b2 || !y_out || !bn_out || !workspace) return SCGIB_E_NULL;
+  if (!gin_bf16_shape_ok(kin, hidden)) return SCGIB_E_SHAPE;
+  if (bn_in && kin != hidden) return SCGIB_E_SHAPE;
+  if (V < 1) return SCGIB_E_RANGE;
+  if (!al16(in) || !al16(a_out) || !al16(r_out) || !al16(y_out) || !al16(W1) || !al16(W2) || ((uintptr_t)workspace & 255u) != 0)
+    return SCGIB_E_ALIGN;
+  if (workspace_bytes < scgib_gin_layer_fwd_bf16_workspace_bytes(V, hidden)) return SCGIB_E_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream_;
+  char* p = (char*)workspace;
+  unsigned int* counter = (unsigned int*)p;
+  cudaMemsetAsync(counter, 0, 256, s);
+  GinFwdArgs a;
+  a.in = (const float*)in; a.row_map = row_map; a.bn_in = bn_in; a.indptr = indptr; a.indices = indices; a.V = V;
+  a.W1t = nullptr; a.b1 = b1; a.W2t = nullptr; a.b2 = b2; a.W1 = W1; a.W2 = W2;
+  a.gamma = nullptr; a.beta = nullptr;
+  a.a_out = (float*)a_out; a.r_out = (float*)r_out; a.y_out = (float*)y_out; a.part = (float*)(p + 256); a.counter = counter;
+  a.bn_out = bn_out; a.running = running;
+  launch_gin_fwd_bf16(a, nullptr, kin, hidden, s);
+  return (int)cudaGetLastError();
+}
+
+namespace scgib {
+static GinBwdOpWs gin_bwd_bf16_op_carve(int V, int kin, int H, void* base) {
+  GinBwdOpWs w;
+  char* p = (char*)base;
+  size_t o = 0;
+  auto take = [&](size_t nfloats) { float* r = (float*)(p + o); o += al(nfloats * sizeof(float)); return r; };
+  w.g_o = take((size_t)V * H / 2); w.cvec = take(2 * H);      // g_o: bf16 [V][H]
+  w.part2 = take((size_t)(gin_bwd_pre_bf16_grid(V, H) + 2) * 2 * H);
+  w.counter = (unsigned int*)take(64);
+  w.off[0] = 0; w.off[1] = (int64_t)H * kin; w.off[2] = w.off[1] + H; w.off[3] = w.off[2] + (int64_t)H * H;   // W1 b1 W2 b2
+  w.pstride = w.off[3] + H;
+  w.ppart = take((size_t)num_sms() * w.pstride);
+  w.bytes = o;
+  return w;
+}
+}  // namespace scgib
+
+extern "C" SCGIB_API size_t scgib_gin_layer_bwd_bf16_workspace_bytes(int32_t V, int32_t kin, int32_t hidden) {
+  if (V < 1 || !gin_bf16_shape_ok(kin, hidden)) return 0;
+  return gin_bwd_bf16_op_carve(V, kin, hidden, nullptr).bytes;
+}
+
+extern "C" SCGIB_API int scgib_gin_layer_bwd_bf16(const void* g_next, const int32_t* indptr, const int32_t* indices, int32_t V,
+                                        int32_t kin, int32_t hidden, int32_t ga_f32, const void* y, const void* r, const void* a,
+                                        const float* bn, const float* W1, const float* W2, void* g_a, float* dW1, float* db1,
+                                        float* dW2, float* db2, float* dgamma, float* dbeta, void* workspace,
+                                        size_t workspace_bytes, void* stream_) {
+  if (!g_next || !y || !r || !a || !bn || !W1 || !W2 || !g_a || !dW1 || !db1 || !dW2 || !db2 || !dgamma || !dbeta || !workspace)
+    return SCGIB_E_NULL;
+  if (indptr && !indices) return SCGIB_E_NULL;
+  if (!gin_bf16_shape_ok(kin, hidden)) return SCGIB_E_SHAPE;
+  if (V < 1) return SCGIB_E_RANGE;
+  if (!al16(g_next) || !al16(y) || !al16(r) || !al16(a) || !al16(g_a) || !al16(W1) || !al16(W2) || ((uintptr_t)workspace & 255u) != 0)
+    return SCGIB_E_ALIGN;
+  const GinBwdOpWs w = gin_bwd_bf16_op_carve(V, kin, hidden, workspace);
+  if (workspace_bytes < w.bytes) return SCGIB_E_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream_;
+  const int GP = num_sms();
+  cudaMemsetAsync(w.counter, 0, 256, s);
+  GinBwdPreArgs q;
+  q.src = (const float*)g_next; q.indptr = indptr; q.indices = indptr ? indices : nullptr; q.map = nullptr;
+  q.y = (const float*)y; q.bn = bn; q.V = V; q.g_o = w.g_o; q.part = w.part2; q.counter = w.counter;
+  q.d_gamma = dgamma; q.d_beta = dbeta; q.cvec = w.cvec;
+  launch_gin_bwd_pre_bf16(q, nullptr, hidden, s);
+  GinBwdMainArgs m;
+  m.g_o = w.g_o; m.y = (const float*)y; m.r = (const float*)r; m.a = (const float*)a; m.bn = bn; m.cvec = w.cvec;
+  m.W1 = W1; m.W2 = W2; m.V = V; m.g_a = (float*)g_a;
+  m.part = w.ppart; m.pstride = w.pstride; m.off_W1 = w.off[0]; m.off_b1 = w.off[1]; m.off_W2 = w.off[2]; m.off_b2 = w.off[3];
+  launch_gin_bwd_main_bf16(m, nullptr, kin, hidden, GP, s, ga_f32 != 0 || kin < hidden);
+  float* outs[4] = {dW1, db1, dW2, db2};
+  const int64_t lens[4] = {(int64_t)hidden * kin, hidden, (int64_t)hidden * hidden, hidden};
+  for (int i = 0; i < 4; ++i) {
+    ReduceRanges rr;
+    rr.n = 1; rr.off[0] = w.off[i]; rr.len[0] = lens[i]; rr.c0[0] = 0; rr.c1[0] = GP;
+    launch_reduce_partials(w.ppart, w.pstride, GP, rr, outs[i] - w.off[i], s);
+  }
+  return (int)cudaGetLastError();
+}
+
 // ---- loss operators (forward + gradient in one call; the units of the whole-step functions)
 namespace scgib {
 struct LossOpWs { float *rpart, *G, *edge, *z1, *z2, *zsplit, *n1, *n2, *diag, *D, *rowsum, *g1p, *g2p, *kl, *losses; size_t bytes; };

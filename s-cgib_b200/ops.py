@@ -42,11 +42,29 @@ def to_bf16(t: torch.Tensor) -> torch.Tensor:
 
 
 def gin_layer_fwd(h, indptr, indices, W1, b1, W2, b2, row_map=None, bn_in=None, running=None, save=False):
-    """One GINConv + batch statistics (models.py:66-72).  Returns (y, bn{mean,rstd}[2,64], a, r)."""
+    """One GINConv + batch statistics (models.py:66-72).  Returns (y, bn{mean,rstd}[2,H], a, r), H = W1.shape[0].
+    A torch.bfloat16 ``h`` runs the bf16-mode kernel (H 64 or 128): y, a, r bf16, bn the statistics of the rounded y."""
     _cuda(h, indptr, W1)
     lib = _lib.load()
     V = indptr.numel() - 1
-    kin = h.shape[1]
+    kin, H = h.shape[1], W1.shape[0]
+    if h.dtype == torch.bfloat16:
+        h = _b16(h)
+        W1, b1, W2, b2 = _c32(W1), _c32(b1), _c32(W2), _c32(b2)
+        y = torch.empty(V, H, device=h.device, dtype=torch.bfloat16)
+        a = torch.empty(V, kin, device=h.device, dtype=torch.bfloat16) if save else None
+        r = torch.empty(V, H, device=h.device, dtype=torch.bfloat16) if save else None
+        bn_out = torch.zeros(4, H, device=h.device)
+        ws = _ws(lib.scgib_gin_layer_fwd_bf16_workspace_bytes(V, H), h.device)
+        off = (-ws.data_ptr()) % 256
+        _lib.check(lib.scgib_gin_layer_fwd_bf16(_lib.ptr(h), kin, H, _lib.ptr(row_map), _lib.ptr(bn_in), _lib.ptr(indptr),
+                                                _lib.ptr(indices), V, _lib.ptr(W1), _lib.ptr(b1), _lib.ptr(W2), _lib.ptr(b2),
+                                                _lib.ptr(a), _lib.ptr(r), _lib.ptr(y), _lib.ptr(bn_out),
+                                                _lib.ptr(running), ctypes.c_void_p(ws.data_ptr() + off), ws.numel() - off,
+                                                _stream(h)), "gin_layer_fwd_bf16")
+        return y, bn_out[:2], a, r
+    if H != HID:
+        raise ValueError("gin_layer_fwd: the fp32 layer entry is hidden %d (got %d)" % (HID, H))
     y = torch.empty(V, HID, device=h.device)
     a = torch.empty(V, kin, device=h.device) if save else None
     r = torch.empty(V, HID, device=h.device) if save else None
@@ -70,13 +88,34 @@ def segment_sum(h, seg_ptr, bn=None):
     return out
 
 
-def gin_layer_bwd(g_next, y, r, a, bn, W1, W2, indptr=None, indices=None):
+def gin_layer_bwd(g_next, y, r, a, bn, W1, W2, indptr=None, indices=None, ga_f32=False):
     """Backward of one GINConv + BatchNorm(train) + ReLU layer.  ``g_next``: gradient wrt the layer output (``indptr`` None)
-    or wrt the next layer's aggregated input (gathered through the CSR).  ``bn`` = [4,64] {mean, rstd, gamma, beta}.
-    Returns (g_a, dW1, db1, dW2, db2, dgamma, dbeta)."""
+    or wrt the next layer's aggregated input (gathered through the CSR).  ``bn`` = [4,H] {mean, rstd, gamma, beta}, H = W1.shape[0].
+    Returns (g_a, dW1, db1, dW2, db2, dgamma, dbeta).
+    A torch.bfloat16 ``y`` runs the bf16-mode kernels: y, r, a bf16, g_next bf16 with ``indptr`` and fp32 without; g_a is fp32
+    with ``ga_f32`` or a.shape[1] < H, else bf16."""
     _cuda(g_next, y, r, a, bn, W1, W2)
     lib = _lib.load()
     V, kin, dev = y.shape[0], a.shape[1], y.device
+    H = W1.shape[0]
+    if y.dtype == torch.bfloat16:
+        y, r, a = _b16(y), _b16(r), _b16(a)
+        g_next = _b16(g_next) if indptr is not None else _c32(g_next)
+        bn, W1, W2 = _c32(bn), _c32(W1), _c32(W2)
+        f32 = bool(ga_f32) or kin < H
+        g_a = torch.empty(V, kin, device=dev, dtype=torch.float32 if f32 else torch.bfloat16)
+        dW1, db1 = torch.empty(H, kin, device=dev), torch.empty(H, device=dev)
+        dW2, db2 = torch.empty(H, H, device=dev), torch.empty(H, device=dev)
+        dgamma, dbeta = torch.empty(H, device=dev), torch.empty(H, device=dev)
+        ws = _ws(lib.scgib_gin_layer_bwd_bf16_workspace_bytes(V, kin, H), dev)
+        off = (-ws.data_ptr()) % 256
+        _lib.check(lib.scgib_gin_layer_bwd_bf16(_lib.ptr(g_next), _lib.ptr(indptr), _lib.ptr(indices), V, kin, H, int(f32),
+                                                _lib.ptr(y), _lib.ptr(r), _lib.ptr(a), _lib.ptr(bn), _lib.ptr(W1), _lib.ptr(W2),
+                                                _lib.ptr(g_a), _lib.ptr(dW1), _lib.ptr(db1), _lib.ptr(dW2),
+                                                _lib.ptr(db2), _lib.ptr(dgamma), _lib.ptr(dbeta),
+                                                ctypes.c_void_p(ws.data_ptr() + off), ws.numel() - off, _stream(y)),
+                   "gin_layer_bwd_bf16")
+        return g_a, dW1, db1, dW2, db2, dgamma, dbeta
     g_a = torch.empty(V, kin, device=dev)
     dW1, db1 = torch.empty(HID, kin, device=dev), torch.empty(HID, device=dev)
     dW2, db2 = torch.empty(HID, HID, device=dev), torch.empty(HID, device=dev)

@@ -132,11 +132,20 @@ def test_bf16_parity_full_size(k):
     _check(20 + k, 4096, k)
 
 
-@pytest.mark.parametrize("seed,B,k,shape", [(31, 128, 1, "pcqm"), (32, 300, 2, "pcqm"), (33, 64, 1, "peptides"), (34, 1024, 1, "pcqm")])
+@pytest.mark.parametrize("seed,B,k,shape", [(31, 128, 1, "pcqm"), (32, 300, 2, "pcqm"), (33, 64, 1, "peptides"), (34, 1024, 1, "pcqm"),
+                                            (35, 8, 2, "macrocycle")])
 def test_bf16_parity_hidden128(seed, B, k, shape):
     """--dims 128 (BASELINE configs[4] GIN-5x128) in bf16 mode: the same kernels instantiated at H = 128 (K = 128 GEMMs over two
     64-column operand blocks, 128-column accumulators)."""
     _check(seed, B, k, hidden=128, shape=shape)
+
+
+@pytest.mark.parametrize("seed,B,k", [(17, 130, 1)])
+def test_bf16_parity_macrocycles(seed, B, k):
+    """Macrocyclic peptides (neighbours up to 200 rows apart, beyond the forward kernels' gather window).  B = 130 (~20k rows,
+    ~64k ego rows) gives every CTA of the shared encoder launches several row tiles, so the layers that walk their tiles in
+    reverse order walk more than one."""
+    _check(seed, B, k, shape="macrocycle")
 
 
 def test_bf16_deterministic_and_trains():

@@ -20,7 +20,8 @@ pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 
 
-@pytest.mark.parametrize("seed,B,k,shape", [(51, 100, 1, "pcqm"), (52, 60, 2, "pcqm"), (53, 24, 1, "peptides"), (54, 2, 1, "pcqm")])
+@pytest.mark.parametrize("seed,B,k,shape", [(51, 100, 1, "pcqm"), (52, 60, 2, "pcqm"), (53, 24, 1, "peptides"), (54, 2, 1, "pcqm"),
+                                            (55, 8, 2, "macrocycle")])
 def test_fp32_parity_hidden128(seed, B, k, shape):
     """Forward 1e-5 and the gradient policy of tests/helpers.py.  A hidden unit within rounding distance of the ReLU kink
     takes different sides in two correct fp32 implementations and moves EVERY gradient below it by O(1/rows) (measured

@@ -15,8 +15,8 @@ import numpy as np
 import pytest
 import torch
 
-from oracle.graph_ref import (RefEgoBatch, RefGraph, batch_ref, ego_batch_ref, graph_from_bonds, path_graph,
-                              synth_batch)
+from oracle.graph_ref import (RefEgoBatch, RefGraph, batch_ref, ego_batch_ref, graph_from_bonds, macrocycle_batch, path_graph,
+                              shuffle_nodes, synth_batch)
 from oracle.scgib_oracle import (OracleMainmodel, draw_noise_like_reference, normalize_rows, tgraph_from_ego,
                                  tgraph_from_ref)
 from tests.helpers import (GRAD_TOL_MAX, GRAD_TOL_MEDIAN, check_against_truth, engine_from_oracle, fp64_truth,
@@ -302,10 +302,14 @@ def _edge_case_batch(kind):
         mols = [path_graph(2, seed=1), synth_batch(23, 1, "peptides"), star, path_graph(3, seed=2), ring,
                 synth_batch(24, 1, "peptides"), path_graph(2, seed=5)]
         return batch_ref(mols)
+    if kind == "macrocycles":      # head-to-tail and 65 .. 200-atom ring closures, one 420-atom ring: neighbours beyond the gather window
+        return macrocycle_batch(25, 5)
+    if kind == "shuffled":         # Peptides-shape molecules with the atom order permuted inside each graph
+        return shuffle_nodes(synth_batch(26, 5, "peptides"), 27)
     raise ValueError(kind)
 
 
-@pytest.mark.parametrize("kind,k", [("pairs", 1), ("peptides", 1), ("peptides", 3), ("ragged", 2)])
+@pytest.mark.parametrize("kind,k", [("pairs", 1), ("peptides", 1), ("peptides", 3), ("ragged", 2), ("macrocycles", 2), ("shuffled", 1)])
 def test_parity_edge_shapes(kind, k):
     """Ragged / extreme batches against the faithful oracle (same policy as test_parity_vs_faithful_oracle)."""
     g = _edge_case_batch(kind)
